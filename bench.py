@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the CryoVIT feature-extraction hot path on B200 (contract: see the task's bench.py section).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one synthetic tomogram: 128 slices of 512x512 uint8 -> DINOv2
 ViT-g/14-reg4 features, fp16 (1536, 128, 32, 32) (BASELINE.json configs[1]; slice batch 128 as in the reference's
@@ -41,6 +41,23 @@ DTYPES = {"mixed-attn": "fp16 (norm1 out, attention out, qkv/proj weights) + bf1
           "mixed": "fp16 (LayerNorm out, attention out, qkv/proj/w12 weights) + bf16 (q/k/v, probabilities, FFN hidden, w3) operands, fp32 accumulate",
           "fp16": "fp16 (LayerNorm out, q/k/v, probabilities, attention out, qkv/proj/w12 weights) + bf16 (FFN hidden, w3) operands, fp32 accumulate",
           "bf16": "bf16 operands, fp32 accumulate"}
+
+
+DUMP_POSITIONS = 4096  # --dump-outputs keeps 4096 of the 131072 feature vectors: 4096 x 1536 float32 = 25 MB
+
+
+def dump_features(torch, feats, out_dir: str) -> None:
+    """--dump-outputs: the (C, D, 32, 32) features of the last timed step, as whole C-channel feature vectors at a fixed
+    seeded sample of (slice, row, column) positions, in flat position order: DIR/features_sample.npy, float32 (C, n).
+    Two builds run with the same arguments see the same inputs, so their files compare element for element."""
+    import numpy as np
+
+    n = feats.shape[1] * feats.shape[2] * feats.shape[3]
+    pos = np.sort(np.random.default_rng(0).choice(n, size=min(DUMP_POSITIONS, n), replace=False))
+    sample = feats.reshape(feats.shape[0], n)[:, torch.from_numpy(pos).to(feats.device)]
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "features_sample.npy", sample.float().cpu().numpy())
 
 
 def measured_peaks() -> tuple[dict, str]:
@@ -424,8 +441,9 @@ def head_train_voxels_per_s(torch, dist, world: int, steps: int = 3) -> dict:
     return line
 
 
-def cpu_oracle_slices_per_s(n_slices: int, sd=None, threads: int | None = None) -> tuple[float, int, float]:
-    """fp32 oracle (pre-processing + ViT-g forward + layout/cast) on the host cores over n_slices slices."""
+def cpu_oracle_slices_per_s(n_slices: int, sd=None, threads: int | None = None):
+    """fp32 oracle (pre-processing + ViT-g forward + layout/cast) on the host cores over n_slices slices:
+    (slices/s, cores, seconds, fp16 features)."""
     import numpy as np
     import torch
 
@@ -445,7 +463,7 @@ def cpu_oracle_slices_per_s(n_slices: int, sd=None, threads: int | None = None) 
     feats = oextract.dino_features(opre.dino_transform(opre.load_tomogram(tomo)), model, BATCH)
     dt = time.perf_counter() - t0
     assert feats.shape == (C, n_slices, 32, 32)
-    return n_slices / dt, cores, dt
+    return n_slices / dt, cores, dt, feats
 
 
 def gpu_eager_baseline(torch, sd_cpu) -> dict:
@@ -770,14 +788,18 @@ def run_reference(args) -> None:
 
     sd = random_state_dict(CONFIGS[MODEL], seed=0)
     rates, cores = [], os.cpu_count()
-    for i in range(args.warmup_ref + args.steps_ref):
-        r, cores, _ = cpu_oracle_slices_per_s(sample, sd)
+    for i in range(args.warmup_ref + args.steps):
+        r, cores, _, feats = cpu_oracle_slices_per_s(sample, sd)
         if i >= args.warmup_ref:
             rates.append(r)
+    if args.dump_outputs:
+        import torch
+
+        dump_features(torch, torch.from_numpy(feats), args.dump_outputs)
     v = statistics.median(rates)
     line = {
         "impl": "reference", "metric": METRIC, "value": round(v, 4), "unit": "slices/s", "n_gpus": args.gpus,
-        "steps": args.steps_ref, "warmup": args.warmup_ref, "ms_per_step": round(1e3 * sample / v, 1),
+        "steps": args.steps, "warmup": args.warmup_ref, "ms_per_step": round(1e3 * sample / v, 1),
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": config_dict(args.gpus),
         "cpu_baseline": {"value": round(v, 4), "unit": "slices/s", "cores": cores, "kind": "port",
@@ -956,6 +978,8 @@ def run_b200(args) -> None:
         sampler.start()
     ms, launches = timed(step_device, args.steps, args.warmup, timer)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_features(torch, feats, args.dump_outputs)
     ms_e2e, _ = timed(step_e2e, args.steps, max(2, args.warmup // 2), drain=drain_e2e)
 
     # head inference and data-parallel head training: every rank takes part (training all-reduces its gradients)
@@ -1030,7 +1054,7 @@ def run_b200(args) -> None:
     torch.cuda.empty_cache()
     if world == 1 and not args.no_cpu_baseline:
         line["gpu_eager_baseline"] = gpu_eager_baseline(torch, sd)
-        v, cores, dt = cpu_oracle_slices_per_s(2, sd)
+        v, cores, dt, _ = cpu_oracle_slices_per_s(2, sd)
         line["cpu_baseline"] = {"value": round(v, 4), "unit": "slices/s", "cores": cores, "kind": "port",
                                 "sample": f"2 slices of {H}x{W} through preproc + ViT-g fp32 oracle + layout/cast ({dt:.1f} s)"}
         del sd
@@ -1052,9 +1076,13 @@ def main() -> None:
     ap.add_argument("--operands", default="mixed-attn", choices=["mixed-attn", "mixed", "fp16", "bf16"],
                     help="16-bit formats of the ViT operands (cryovit_b200/vit.py): mixed-attn = fp16 norm1 / attention output and "
                          "the qkv / proj weights, everything else bf16 (default, the product path); mixed = the FFN input side fp16 too")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the features of the last one (a fixed "
+                    "seeded sample of whole feature vectors) to DIR/features_sample.npy as float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
-    args.steps_ref, args.warmup_ref = min(args.steps, 3), min(args.warmup, 1)
+    args.warmup_ref = min(args.warmup, 1)
     if args.impl == "reference":
         run_reference(args)
     else:

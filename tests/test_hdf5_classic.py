@@ -13,12 +13,9 @@ from cryovit_b200.host import hdf, hdf5_classic as h5c
 
 
 def _libhdf5_file():
-    """A file written by libhdf5 itself (MATLAB 7.3 = HDF5 behind a 512-byte user block) that ships with scipy."""
-    import scipy.io
-    p = Path(scipy.io.__file__).parent / "matlab" / "tests" / "data" / "testhdf5_7.4_GLNX86.mat"
-    if not p.exists():
-        pytest.skip("scipy's HDF5 test file is not in this image")
-    return p
+    """A file written by libhdf5 itself (MATLAB 7.3 = HDF5 behind a 512-byte user block): scipy's test file
+    scipy/io/matlab/tests/data/testhdf5_7.4_GLNX86.mat (BSD-3-Clause), stored byte for byte."""
+    return Path(__file__).resolve().parent / "golden" / "testhdf5_7.4_GLNX86.mat"
 
 
 def test_reader_parses_a_libhdf5_written_file():

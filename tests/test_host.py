@@ -248,13 +248,16 @@ assert not dist.is_initialized()               # torn down again: it was created
 def test_entry_point_process_group_plumbing_two_ranks(tmp_path):
     """ADVICE r1 (high): under torchrun the train / eval entry points must join ONE process group (gradient all-reduce,
     csv row gather) and bind their own GPU; a loop that shards by RANK without a group must refuse to run. Launched
-    the way torchrun launches (RANK / LOCAL_RANK / WORLD_SIZE / MASTER_ADDR / MASTER_PORT), gloo on this CPU box."""
+    the way torchrun launches (RANK / LOCAL_RANK / WORLD_SIZE / MASTER_ADDR / MASTER_PORT): NCCL with one GPU per rank
+    where there are two, gloo otherwise (NCCL refuses two ranks on one GPU, so the ranks are then shown no GPU)."""
     script = tmp_path / "pg_worker.py"
     script.write_text(PG_WORKER)
     port = str(31500 + os.getpid() % 2000)
+    gpus = {} if torch.cuda.device_count() >= 2 else {"CUDA_VISIBLE_DEVICES": ""}
     procs = []
     for r in range(2):
-        env = dict(os.environ, RANK=str(r), LOCAL_RANK=str(r), WORLD_SIZE="2", MASTER_ADDR="127.0.0.1", MASTER_PORT=port, REPO=str(ROOT))
+        env = dict(os.environ, RANK=str(r), LOCAL_RANK=str(r), WORLD_SIZE="2", MASTER_ADDR="127.0.0.1", MASTER_PORT=port, REPO=str(ROOT),
+                   **gpus)
         procs.append(subprocess.Popen([sys.executable, str(script)], env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True))
     outs = [p.communicate(timeout=240)[0] for p in procs]
     assert all(p.returncode == 0 for p in procs), "\n".join(outs)
