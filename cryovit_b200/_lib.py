@@ -27,6 +27,10 @@ SIGNATURES: dict[str, list] = {
     "cvit_preproc_resize_f32_3ch": [P, I32, P, I64, I64, I64, P],
     "cvit_patchify_f32_3ch": [P, P, I64, I64, I64, I64, P],
     "cvit_patch_embed_gemm": [P, I64, P, P, P, I64, I64, I64, I64, I64, I64, I64, P],
+    "cvit_patch_embed_gemm_fmt": [P, I64, P, P, P, I64, I64, I64, I64, I64, I64, I64, I32, P],
+    "cvit_preproc_patchify_tf32": [P, I32, P, I64, I64, I64, I64, P],
+    "cvit_patchify_f32_3ch_tf32": [P, P, I64, I64, I64, I64, P],
+    "cvit_layernorm_f32_tf32": [P, I64, P, P, P, I64, I64, I64, F32, P],
     "cvit_assemble_special_tokens": [P, P, I64, I64, I64, I64, P],
     "cvit_layernorm_f32_bf16": [P, I64, P, P, P, I64, I64, I64, F32, P],
     "cvit_layernorm_f32_f16": [P, I64, P, P, P, I64, I64, I64, F32, P],

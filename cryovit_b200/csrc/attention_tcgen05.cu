@@ -91,7 +91,10 @@ __device__ __forceinline__ float fmax3(float a, float b, float c) {
 // F16: q/k/v and P are IEEE fp16 instead of bf16 (P <= 2^8 under the lazy rescale, far inside the fp16 range);
 // OUT16: the output is stored as IEEE fp16 instead of bf16 (independent of F16: the output only has to match the
 // operand type of the projection GEMM that reads it). Everything else is identical.
-template <bool F16, bool OUT16>
+// OUT32: the output is stored as TF32-rounded fp32 (the A operand of a kind::tf32 projection GEMM); the epilogue
+// stores straight from registers (no shared-memory staging), 16 columns per TMEM load so its live registers stay
+// within the 16-bit path's under the epilogue's setmaxnreg budget.
+template <bool F16, bool OUT16, bool OUT32 = false>
 __global__ void __launch_bounds__(FA_THREADS, 1)
 attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const FaArgs args) {
   extern __shared__ uint8_t smem_raw[];
@@ -337,6 +340,7 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const FaArgs
     for (int item = blockIdx.x; item < total_items; item += gridDim.x) {
       const int pair = item % n_pairs, bh = item / n_pairs, kind = item_kind(item);
       __nv_bfloat16* out_bh = args.out + ((size_t)(bh / args.heads) * T) * args.C + (bh % args.heads) * FA_D;
+      float* outf_bh = reinterpret_cast<float*>(args.out) + ((size_t)(bh / args.heads) * T) * args.C + (bh % args.heads) * FA_D;
       if (kind == SPLIT) {
         // two partial softmaxes of the same query tile (even / odd K/V tiles): merge, then normalise
         const int qt = 2 * pair;
@@ -356,7 +360,24 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const FaArgs
         mbar_wait(bar_grp + 64 + B_OFULL, pb);
         tcgen05_fence_after();
         const bool warp_active = qt * FA_BQ + q * 32 < T;  // warp-uniform
-        if (warp_active) {
+        if (OUT32 && warp_active) {
+          const int tok = qt * FA_BQ + row;
+          uint4* dst = reinterpret_cast<uint4*>(outf_bh + (size_t)tok * args.C);
+#pragma unroll 1
+          for (int hh = 0; hh < 4; ++hh) {
+            uint32_t oa[16], o2[16];
+            tmem_ld_32x16(t_row + FA_COL_O + hh * 16, oa);
+            tmem_ld_32x16(t_row + FA_COL_O + 64 + hh * 16, o2);
+            tmem_ld_wait();
+#pragma unroll
+            for (int i = 0; i < 16; ++i)
+              oa[i] = __float_as_uint(round_tf32(__uint_as_float(oa[i]) * wa + __uint_as_float(o2[i]) * wb));
+            if (tok < T) {
+#pragma unroll
+              for (int i = 0; i < 4; ++i) dst[4 * hh + i] = make_uint4(oa[4 * i], oa[4 * i + 1], oa[4 * i + 2], oa[4 * i + 3]);
+            }
+          }
+        } else if (warp_active) {
           const int tok = qt * FA_BQ + row;
           uint4* dst = reinterpret_cast<uint4*>(out_bh + (size_t)tok * args.C);
 #pragma unroll 1
@@ -395,7 +416,23 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const FaArgs
         mbar_wait(bg + B_OFULL, par);
         tcgen05_fence_after();
         const bool warp_active = qt * FA_BQ + q * 32 < T;  // warp-uniform
-        if (warp_active) {
+        if (OUT32 && warp_active) {
+          const float inv = 1.0f / l;
+          const int tok = qt * FA_BQ + row;
+          uint4* dst = reinterpret_cast<uint4*>(outf_bh + (size_t)tok * args.C);
+#pragma unroll 1
+          for (int hh = 0; hh < 4; ++hh) {
+            uint32_t o[16];
+            tmem_ld_32x16(t_row + FA_COL_O + g * 64 + hh * 16, o);
+            tmem_ld_wait();
+#pragma unroll
+            for (int i = 0; i < 16; ++i) o[i] = __float_as_uint(round_tf32(__uint_as_float(o[i]) * inv));
+            if (tok < T) {
+#pragma unroll
+              for (int i = 0; i < 4; ++i) dst[4 * hh + i] = make_uint4(o[4 * i], o[4 * i + 1], o[4 * i + 2], o[4 * i + 3]);
+            }
+          }
+        } else if (warp_active) {
           const float inv = 1.0f / l;
           const int tok = qt * FA_BQ + row;
           uint4* dst = reinterpret_cast<uint4*>(out_bh + (size_t)tok * args.C);
@@ -655,7 +692,7 @@ static long long* g_fa_trace = nullptr;
 extern "C" void cvit_fa_set_trace(long long* p) { g_fa_trace = p; }
 #endif
 
-template <bool F16, bool OUT16>
+template <bool F16, bool OUT16, bool OUT32 = false>
 static int attention_fwd(const void* qkv, void* out, int64_t n_slices, int64_t tokens, int64_t heads, int64_t head_dim,
                          void* stream) {
   if (!qkv || !out || n_slices <= 0 || tokens <= 0 || heads <= 0) {
@@ -679,7 +716,7 @@ static int attention_fwd(const void* qkv, void* out, int64_t n_slices, int64_t t
   if (rc) return rc;
   static bool configured = false;
   if (!configured) {
-    cudaError_t e = cudaFuncSetAttribute(attention_tcgen05_kernel<F16, OUT16>, cudaFuncAttributeMaxDynamicSharedMemorySize, FA_SMEM);
+    cudaError_t e = cudaFuncSetAttribute(attention_tcgen05_kernel<F16, OUT16, OUT32>, cudaFuncAttributeMaxDynamicSharedMemorySize, FA_SMEM);
     if (e != cudaSuccess) {
       set_error("attention: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
       return CVIT_ERR_CUDA;
@@ -702,7 +739,7 @@ static int attention_fwd(const void* qkv, void* out, int64_t n_slices, int64_t t
   const int64_t items = (int64_t)((n_qt + 1) / 2) * heads * n_slices;
   int grid = num_sms();
   if (grid > items) grid = (int)items;
-  attention_tcgen05_kernel<F16, OUT16><<<grid, FA_THREADS, FA_SMEM, (cudaStream_t)stream>>>(tm, a);
+  attention_tcgen05_kernel<F16, OUT16, OUT32><<<grid, FA_THREADS, FA_SMEM, (cudaStream_t)stream>>>(tm, a);
   return check_launch("attention_tcgen05_kernel");
 }
 
@@ -717,15 +754,17 @@ extern "C" int cvit_attention_fwd_f16(const void* qkv, void* out, int64_t n_slic
   return attention_fwd<true, true>(qkv, out, n_slices, tokens, heads, head_dim, stream);
 }
 
-// fmt: CVIT_FMT_OPERANDS_F16 (q/k/v and the probabilities are fp16) | CVIT_FMT_OUT_F16 (the output is stored as fp16).
+// fmt: CVIT_FMT_OPERANDS_F16 (q/k/v and the probabilities are fp16) | CVIT_FMT_OUT_F16 (the output is stored as fp16)
+// | CVIT_FMT_OUT_F32 (bf16 q/k/v and probabilities, TF32-rounded fp32 output).
 extern "C" int cvit_attention_fwd_fmt(const void* qkv, void* out, int64_t n_slices, int64_t tokens, int64_t heads,
                                       int64_t head_dim, int fmt, void* stream) {
   switch (fmt) {
     case 0: return attention_fwd<false, false>(qkv, out, n_slices, tokens, heads, head_dim, stream);
     case 2: return attention_fwd<false, true>(qkv, out, n_slices, tokens, heads, head_dim, stream);
     case 3: return attention_fwd<true, true>(qkv, out, n_slices, tokens, heads, head_dim, stream);
+    case 8: return attention_fwd<false, false, true>(qkv, out, n_slices, tokens, heads, head_dim, stream);
     default:
-      set_error("attention: unsupported format flags 0x%x (0, OUT_F16, OPERANDS_F16|OUT_F16)", fmt);
+      set_error("attention: unsupported format flags 0x%x (0, OUT_F16, OPERANDS_F16|OUT_F16, OUT_F32)", fmt);
       return CVIT_ERR_UNSUPPORTED;
   }
 }

@@ -11,11 +11,11 @@ namespace cvit {
 // everywhere. Process-wide switch for A/B measurements (tools/kernel_probe.py); the default is pairs.
 static int g_gemm_pair = 1;
 
-template <int BN, int EPI, int AMODE, int KSPAN, bool PAIR = false, int SUB = 1>
+template <int BN, int EPI, int AMODE, int KSPAN, bool PAIR = false, int SUB = 1, int OPK = OPK_F16>
 static int launch_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, const GemmArgs& args, int num_tiles,
                        cudaStream_t stream) {
   using Cfg = GemmCfg<BN, KSPAN, PAIR, SUB>;
-  auto kern = gemm_tcgen05_kernel<BN, EPI, AMODE, KSPAN, PAIR, SUB>;
+  auto kern = gemm_tcgen05_kernel<BN, EPI, AMODE, KSPAN, PAIR, SUB, OPK>;
   static bool configured = false;  // per instantiation; attribute is per function, setting twice is harmless
   if (!configured) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
@@ -58,11 +58,12 @@ static int launch_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, const Gem
 }
 
 static int make_tmap_rows(CUtensorMap* tm, const void* base, int64_t rows, int64_t K, int64_t ld, int box_rows,
-                          int kspan, bool f16 = false) {
+                          int kspan, TmapDtype dt = TmapDtype::BF16) {
+  const int esz = dt == TmapDtype::F32 ? 4 : 2;
   uint64_t dims[2] = {(uint64_t)K, (uint64_t)rows};
-  uint64_t strides[2] = {0, (uint64_t)ld * 2};
-  uint32_t box[2] = {(uint32_t)(kspan / 2), (uint32_t)box_rows};
-  return encode_tmap(tm, f16 ? TmapDtype::F16 : TmapDtype::BF16, 2, base, dims, strides, box, kspan);
+  uint64_t strides[2] = {0, (uint64_t)ld * esz};
+  uint32_t box[2] = {(uint32_t)(kspan / esz), (uint32_t)box_rows};
+  return encode_tmap(tm, dt, 2, base, dims, strides, box, kspan);
 }
 
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
@@ -77,6 +78,50 @@ static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 
 #define CVIT_GEMM_PAIR_CASE(EPI_)                                                     \
   if (pair && epi == EPI_)                                                            \
     return launch_gemm<256, EPI_, AMODE_ROWS, 128, true>(tmA, tmB, args, num_tiles, stream);
+// TF32 operands (fp32 containers, 32 values per 128-byte swizzle span): the ViT linears and the patch embedding
+#define CVIT_GEMM_TF32_CASE(BN_, EPI_)                                                \
+  if (bn == BN_ && epi == EPI_)                                                       \
+    return launch_gemm<BN_, EPI_, AMODE_ROWS, 128, false, 1, OPK_TF32>(tmA, tmB, args, num_tiles, stream);
+#define CVIT_GEMM_TF32_PAIR_CASE(EPI_)                                                \
+  if (pair && epi == EPI_)                                                            \
+    return launch_gemm<256, EPI_, AMODE_ROWS, 128, true, 1, OPK_TF32>(tmA, tmB, args, num_tiles, stream);
+
+// [M,K] x [N,K]^T with TF32 operands: K and lda in fp32 elements (multiples of 4, K >= 32: one 128-byte span per stage).
+static int gemm_rows_tf32(const void* A, int64_t lda, const void* B, GemmArgs args, int epi, cudaStream_t stream) {
+  const int64_t M = args.M, N = args.N, K = args.K;
+  if (!A || !B || !args.out || !aligned16(A) || !aligned16(B) || !aligned16(args.out) || (lda % 4) != 0 || (K % 4) != 0 || K < 32) {
+    set_error("gemm tf32: null/unaligned operand (A,B,out need 16B alignment; lda and K multiples of 4, K >= 32)");
+    return CVIT_ERR_INVALID;
+  }
+  const int bn = (epi == EPI_BIAS_SWIGLU) ? ((N % 256 == 0) ? 256 : 0) : (N % 256 == 0) ? 256 : (N % 128 == 0) ? 128 : 0;
+  if (bn == 0) {
+    set_error("gemm tf32: N=%lld not tileable for epilogue %d (multiple of 128; 256 for SwiGLU)", (long long)N, epi);
+    return CVIT_ERR_UNSUPPORTED;
+  }
+  CUtensorMap tmA, tmB;
+  int rc = make_tmap_rows(&tmA, A, M, K, lda, GEMM_BM, 128, TmapDtype::F32);
+  if (rc) return rc;
+  const bool pair = g_gemm_pair && bn == 256 && M > GEMM_BM && epi != EPI_PATCH_EMBED;
+  rc = make_tmap_rows(&tmB, B, N, K, K, pair ? bn / 2 : bn, 128, TmapDtype::F32);
+  if (rc) return rc;
+  const int bm = pair ? 2 * GEMM_BM : GEMM_BM;
+  const int num_tiles = (int)(((M + bm - 1) / bm) * (N / bn));
+  CVIT_GEMM_TF32_PAIR_CASE(EPI_BIAS)
+  CVIT_GEMM_TF32_PAIR_CASE(EPI_BIAS_GELU)
+  CVIT_GEMM_TF32_PAIR_CASE(EPI_BIAS_SWIGLU)
+  CVIT_GEMM_TF32_PAIR_CASE(EPI_SCALE_RESIDUAL)
+  CVIT_GEMM_TF32_CASE(256, EPI_BIAS)
+  CVIT_GEMM_TF32_CASE(128, EPI_BIAS)
+  CVIT_GEMM_TF32_CASE(256, EPI_BIAS_GELU)
+  CVIT_GEMM_TF32_CASE(128, EPI_BIAS_GELU)
+  CVIT_GEMM_TF32_CASE(256, EPI_BIAS_SWIGLU)
+  CVIT_GEMM_TF32_CASE(256, EPI_SCALE_RESIDUAL)
+  CVIT_GEMM_TF32_CASE(128, EPI_SCALE_RESIDUAL)
+  CVIT_GEMM_TF32_CASE(256, EPI_PATCH_EMBED)
+  CVIT_GEMM_TF32_CASE(128, EPI_PATCH_EMBED)
+  set_error("gemm tf32: no kernel instantiated for BN=%d epilogue=%d", bn, epi);
+  return CVIT_ERR_UNSUPPORTED;
+}
 
 // Plain [M,K] x [N,K]^T GEMM with a fused epilogue.
 static int gemm_rows(const void* A, int64_t lda, const void* B, GemmArgs args, int epi, cudaStream_t stream) {
@@ -85,6 +130,7 @@ static int gemm_rows(const void* A, int64_t lda, const void* B, GemmArgs args, i
     set_error("gemm: non-positive dimension M=%lld N=%lld K=%lld", (long long)M, (long long)N, (long long)K);
     return CVIT_ERR_INVALID;
   }
+  if (args.fmt & GEMM_FMT_OPERANDS_TF32) return gemm_rows_tf32(A, lda, B, args, epi, stream);
   if (!A || !B || !args.out || !aligned16(A) || !aligned16(B) || !aligned16(args.out) || (lda % 8) != 0 || (K % 8) != 0) {
     set_error("gemm: null/unaligned operand (A,B,out need 16B alignment; lda and K multiples of 8)");
     return CVIT_ERR_INVALID;
@@ -103,13 +149,13 @@ static int gemm_rows(const void* A, int64_t lda, const void* B, GemmArgs args, i
   }
   if (kspan != 128 && bn > 128) bn = 128;
   CUtensorMap tmA, tmB;
-  const bool f16 = (args.fmt & GEMM_FMT_OPERANDS_F16) != 0;
-  int rc = make_tmap_rows(&tmA, A, M, K, lda, GEMM_BM, kspan, f16);
+  const TmapDtype dt = (args.fmt & GEMM_FMT_OPERANDS_F16) ? TmapDtype::F16 : TmapDtype::BF16;
+  int rc = make_tmap_rows(&tmA, A, M, K, lda, GEMM_BM, kspan, dt);
   if (rc) return rc;
   // CTA pairs (256 x 256 output tile per TPC) whenever there is more than one 128-row tile to share a B tile over
   const bool pair = g_gemm_pair && bn == 256 && kspan == 128 && M > GEMM_BM &&
                     (epi == EPI_BIAS || epi == EPI_BIAS_GELU || epi == EPI_BIAS_SWIGLU || epi == EPI_SCALE_RESIDUAL);
-  rc = make_tmap_rows(&tmB, B, N, K, K, pair ? bn / 2 : bn, kspan, f16);
+  rc = make_tmap_rows(&tmB, B, N, K, K, pair ? bn / 2 : bn, kspan, dt);
   if (rc) return rc;
   const int bm = pair ? 2 * GEMM_BM : GEMM_BM;
   const int num_tiles = (int)(((M + bm - 1) / bm) * (N / bn));
@@ -167,7 +213,7 @@ static int gemm_rows_mn(const void* At, int64_t ldat, const void* B, GemmArgs ar
     if (rc) return rc;
   }
   const bool pair = g_gemm_pair && bn == 256 && M > GEMM_BM;
-  int rc = make_tmap_rows(&tmB, B, N, K, K, pair ? bn / 2 : bn, kspan, true);
+  int rc = make_tmap_rows(&tmB, B, N, K, K, pair ? bn / 2 : bn, kspan, TmapDtype::F16);
   if (rc) return rc;
   const int bm = pair ? 2 * GEMM_BM : GEMM_BM;
   const int num_tiles = (int)(((M + bm - 1) / bm) * (N / bn));
@@ -271,10 +317,21 @@ int cvit_set_gemm_pair(int enable) {
   return prev;
 }
 
-static int check_fmt(int fmt) {
-  if (fmt & ~(GEMM_FMT_OPERANDS_F16 | GEMM_FMT_OUT_F16)) {
-    set_error("linear: unknown format flags 0x%x", fmt);
+// tf32_out_f32: with TF32 operands this entry point's epilogue stores TF32-rounded fp32 (GELU / SwiGLU), so
+// CVIT_FMT_OUT_F32 is required; otherwise (EPI_BIAS: 16-bit qkv output; the fp32 residual stream) it is refused.
+static int check_fmt(int fmt, const char* who, bool tf32_out_f32) {
+  if (fmt & ~(GEMM_FMT_OPERANDS_F16 | GEMM_FMT_OUT_F16 | GEMM_FMT_OPERANDS_TF32 | GEMM_FMT_OUT_F32)) {
+    set_error("%s: unknown format flags 0x%x", who, fmt);
     return CVIT_ERR_INVALID;
+  }
+  const bool tf32 = (fmt & GEMM_FMT_OPERANDS_TF32) != 0, f32 = (fmt & GEMM_FMT_OUT_F32) != 0;
+  // instantiated: 16-bit operands with 16-bit outputs; TF32 operands with fp32 GELU / SwiGLU output or 16-bit EPI_BIAS
+  // output. Everything else is refused rather than run in some other format.
+  if ((tf32 && (fmt & GEMM_FMT_OPERANDS_F16)) || (f32 && !tf32) || (tf32 && f32 != tf32_out_f32) ||
+      (f32 && (fmt & GEMM_FMT_OUT_F16))) {
+    set_error("%s: format flags 0x%x are not instantiated (TF32 operands need %s)", who, fmt,
+              tf32_out_f32 ? "CVIT_FMT_OUT_F32 and no fp16 flag" : "no CVIT_FMT_OUT_F32 and no fp16 operands");
+    return CVIT_ERR_UNSUPPORTED;
   }
   return CVIT_OK;
 }
@@ -282,7 +339,7 @@ static int check_fmt(int fmt) {
 int cvit_linear_bias_fmt(const void* A, int64_t lda, const void* W, const float* bias, void* out, int64_t ldo,
                          int64_t M, int64_t N, int64_t K, int gelu, int fmt, void* stream) {
   if (!bias) { set_error("linear_bias: bias is required"); return CVIT_ERR_INVALID; }
-  if (int rc = check_fmt(fmt)) return rc;
+  if (int rc = check_fmt(fmt, "linear_bias", gelu != 0)) return rc;
   GemmArgs a = base_args(M, N, K, out, ldo);
   a.bias = bias;
   a.fmt = fmt;
@@ -381,7 +438,7 @@ int cvit_linear_bias_gelu_bf16_gn(const void* A, int64_t lda, const void* W, con
 int cvit_linear_swiglu_fmt(const void* A, int64_t lda, const void* W12i, const float* bias12i, void* out,
                            int64_t ldo, int64_t M, int64_t N2, int64_t K, int fmt, void* stream) {
   if (!bias12i) { set_error("linear_swiglu: bias is required"); return CVIT_ERR_INVALID; }
-  if (int rc = check_fmt(fmt)) return rc;
+  if (int rc = check_fmt(fmt, "linear_swiglu", true)) return rc;
   GemmArgs a = base_args(M, N2, K, out, ldo);
   a.bias = bias12i;
   a.fmt = fmt;
@@ -396,11 +453,11 @@ int cvit_linear_swiglu_bf16(const void* A, int64_t lda, const void* W12i, const 
 int cvit_linear_scale_residual_fmt(const void* A, int64_t lda, const void* W, const float* bias, const float* gamma,
                                    float* x, int64_t ldx, int64_t M, int64_t N, int64_t K, int fmt, void* stream) {
   if (!bias || !gamma) { set_error("linear_scale_residual: bias and gamma are required"); return CVIT_ERR_INVALID; }
-  if (int rc = check_fmt(fmt)) return rc;
+  if (int rc = check_fmt(fmt & ~GEMM_FMT_OUT_F16, "linear_scale_residual", false)) return rc;
   GemmArgs a = base_args(M, N, K, x, ldx);
   a.bias = bias;
   a.gamma = gamma;
-  a.fmt = fmt & GEMM_FMT_OPERANDS_F16;
+  a.fmt = fmt & (GEMM_FMT_OPERANDS_F16 | GEMM_FMT_OPERANDS_TF32);
   return gemm_rows(A, lda, W, a, EPI_SCALE_RESIDUAL, (cudaStream_t)stream);
 }
 
@@ -409,11 +466,27 @@ int cvit_linear_scale_residual_f32(const void* A, int64_t lda, const void* W, co
   return cvit_linear_scale_residual_fmt(A, lda, W, bias, gamma, x, ldx, M, N, K, 0, stream);
 }
 
+int cvit_patch_embed_gemm_fmt(const void* patches, int64_t lda, const void* W, const float* pos_bias_table, float* x,
+                              int64_t ldx, int64_t n_slices, int64_t n_patches, int64_t tokens_per_slice,
+                              int64_t first_patch_token, int64_t N, int64_t K, int fmt, void* stream);
+
 int cvit_patch_embed_gemm(const void* patches, int64_t lda, const void* W, const float* pos_bias_table, float* x,
                           int64_t ldx, int64_t n_slices, int64_t n_patches, int64_t tokens_per_slice,
                           int64_t first_patch_token, int64_t N, int64_t K, void* stream) {
+  return cvit_patch_embed_gemm_fmt(patches, lda, W, pos_bias_table, x, ldx, n_slices, n_patches, tokens_per_slice,
+                                   first_patch_token, N, K, 0, stream);
+}
+
+int cvit_patch_embed_gemm_fmt(const void* patches, int64_t lda, const void* W, const float* pos_bias_table, float* x,
+                              int64_t ldx, int64_t n_slices, int64_t n_patches, int64_t tokens_per_slice,
+                              int64_t first_patch_token, int64_t N, int64_t K, int fmt, void* stream) {
   if (!pos_bias_table) { set_error("patch_embed: table is required"); return CVIT_ERR_INVALID; }
+  if (fmt != 0 && fmt != GEMM_FMT_OPERANDS_TF32) {
+    set_error("patch_embed: format flags 0x%x are not instantiated (0: bf16 patches and weight, CVIT_FMT_OPERANDS_TF32)", fmt);
+    return CVIT_ERR_UNSUPPORTED;
+  }
   GemmArgs a = base_args(n_slices * n_patches, N, K, x, ldx);
+  a.fmt = fmt;
   a.table = pos_bias_table;
   a.pe_np = (int)n_patches;
   a.pe_tokens = (int)tokens_per_slice;

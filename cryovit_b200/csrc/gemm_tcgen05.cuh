@@ -2,6 +2,8 @@
 //
 //   D[M,N] = A[M,K] (bf16, K-major) x B[N,K]^T (bf16, K-major, i.e. torch Linear weight layout)
 //   (GemmArgs::fmt: both operands IEEE fp16 instead, and/or the 16-bit output stored as fp16)
+//   OPK = OPK_TF32: A and B are fp32 holding TF32 values, tcgen05.mma kind::tf32 (half the kind::f16 rate); the
+//   bias(+GELU / SwiGLU) epilogues then store TF32-rounded fp32 for the next TF32 GEMM (EPI_BIAS stays 16-bit)
 //
 // One CTA per SM, 320 threads:
 //   warp 0      TMA producer  (one lane): cp.async.bulk.tensor -> 128B/64B/32B-swizzled smem ring
@@ -74,7 +76,12 @@ struct GemmArgs {
 // A and B hold IEEE fp16 instead of bf16 (same type on both sides: tcgen05 kind::f16 rule); EPI_BIAS / _GELU / _SWIGLU
 // store fp16 instead of bf16. fp16 keeps three more mantissa bits than bf16 for operands whose range is bounded
 // (LayerNorm output, q/k/v, attention output and the weights they meet).
-enum { GEMM_FMT_OPERANDS_F16 = 1, GEMM_FMT_OUT_F16 = 2 };
+// GEMM_FMT_OPERANDS_TF32: A and B are fp32 holding TF32 values (the OPK_TF32 kernels); GEMM_FMT_OUT_F32: EPI_BIAS_GELU /
+// EPI_BIAS_SWIGLU of those kernels store TF32-rounded fp32. The host picks kernels from these bits; the kernel body reads
+// only GEMM_FMT_OUT_F16 at run time.
+enum { GEMM_FMT_OPERANDS_F16 = 1, GEMM_FMT_OUT_F16 = 2, GEMM_FMT_OPERANDS_TF32 = 4, GEMM_FMT_OUT_F32 = 8 };
+// Operand kind of a kernel instantiation: kind::f16 (bf16 or fp16 by GemmArgs::fmt) or kind::tf32 (fp32 containers).
+enum { OPK_F16 = 0, OPK_TF32 = 1 };
 
 constexpr int GEMM_BM = 128;
 constexpr int GEMM_THREADS = 320;
@@ -152,7 +159,7 @@ __device__ __forceinline__ int tile_row_to_global(const TileCoord& t, int r, con
 // memory traffic (TMA writes and MMA reads) against the single-CTA kernel. Barriers: the "full" barriers that count
 // TMA bytes live in the leader (both producers signal them), "empty"/"accumulator full" are multicast commits to both
 // CTAs, "accumulator empty" collects the epilogue warps of both CTAs in the leader.
-template <int BN, int EPI, int AMODE, int KSPAN, bool PAIR = false, int SUB = 1>
+template <int BN, int EPI, int AMODE, int KSPAN, bool PAIR = false, int SUB = 1, int OPK = OPK_F16>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                     const GemmArgs args) {
@@ -161,10 +168,13 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   // leader's MMA schedule matches both producers'.
   static_assert(SUB == 1 || (AMODE == AMODE_ROWS && !PAIR), "tall tiles are implemented for the single-CTA plain-rows GEMM only");
   static_assert(AMODE != AMODE_ROWS_MN || KSPAN == 128, "the MN-major A operand is staged in 128-byte swizzled rows");
+  static_assert(OPK == OPK_F16 || (AMODE == AMODE_ROWS && SUB == 1 && (EPI <= EPI_PATCH_EMBED)),
+                "TF32 operands are implemented for the plain-rows ViT GEMMs only");
   using Cfg = GemmCfg<BN, KSPAN, PAIR, SUB>;
+  constexpr bool TF32 = OPK == OPK_TF32;
   constexpr int TILE_M = (PAIR ? 2 : SUB) * GEMM_BM;  // output rows per tile (per CTA pair with PAIR)
-  constexpr int KC = KSPAN / 2;        // bf16 elements of K per stage
-  constexpr int MMAS_PER_STAGE = KC / 16;
+  constexpr int KC = KSPAN / (TF32 ? 4 : 2);  // elements of K per stage (16-bit, or fp32 for TF32)
+  constexpr int MMAS_PER_STAGE = KC / (TF32 ? 8 : 16);  // 32 bytes of K per MMA either way
   constexpr int STAGES = Cfg::STAGES;
 
   extern __shared__ uint8_t smem_raw[];
@@ -286,9 +296,10 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     // in uniform registers; one elected lane issues the MMAs and commits. (Issuing from a divergent `lane == 0`
     // region cost ~90 cycles per tcgen05.mma: every operand went through R2UR and a per-lane ELECT loop.)
     {
-      const uint32_t idesc = umma_idesc_f16_f32(PAIR ? 2 * GEMM_BM : GEMM_BM, BN) |
-                             ((args.fmt & GEMM_FMT_OPERANDS_F16) ? 0u : UMMA_IDESC_BF16_BITS) |
-                             (AMODE == AMODE_ROWS_MN ? (1u << 15) : 0u);  // bit 15: A is MN-major
+      const uint32_t idesc = TF32 ? umma_idesc_tf32_f32(PAIR ? 2 * GEMM_BM : GEMM_BM, BN)
+                                  : umma_idesc_f16_f32(PAIR ? 2 * GEMM_BM : GEMM_BM, BN) |
+                                        ((args.fmt & GEMM_FMT_OPERANDS_F16) ? 0u : UMMA_IDESC_BF16_BITS) |
+                                        (AMODE == AMODE_ROWS_MN ? (1u << 15) : 0u);  // bit 15: A is MN-major
       int s = 0;
       uint32_t ph = 0;
       int acc = 0;
@@ -321,8 +332,10 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                 constexpr int ASTEP = AMODE == AMODE_ROWS_MN ? 128 : 2;
 #pragma unroll
                 for (int k = 0; k < MMAS_PER_STAGE; ++k) {
-                  // B: advance 16 bf16 = 32 bytes along K inside the swizzle span: +2 in 16-byte units
-                  if (PAIR) umma_bf16_pair(d_tmem, adesc + ASTEP * k, bdesc + 2 * k, idesc, accumulate | (k > 0));
+                  // B: advance 16 bf16 (8 TF32) = 32 bytes along K inside the swizzle span: +2 in 16-byte units
+                  if (TF32 && PAIR) umma_tf32_pair(d_tmem, adesc + ASTEP * k, bdesc + 2 * k, idesc, accumulate | (k > 0));
+                  else if (TF32) umma_tf32(d_tmem, adesc + ASTEP * k, bdesc + 2 * k, idesc, accumulate | (k > 0));
+                  else if (PAIR) umma_bf16_pair(d_tmem, adesc + ASTEP * k, bdesc + 2 * k, idesc, accumulate | (k > 0));
                   else umma_bf16(d_tmem + sub * Cfg::ACC_STRIDE, adesc + ASTEP * k, bdesc + 2 * k, idesc, accumulate | (k > 0));
                 }
               }
@@ -535,7 +548,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
               xs[it].w = silu(xs[it].w) * (ys[it].w + b4b.w);
             }
           }
-          if ((EPI == EPI_BIAS_GELU || EPI == EPI_BIAS) && args.act == ACT_GELU_GRAD) {
+          if (!TF32 && (EPI == EPI_BIAS_GELU || EPI == EPI_BIAS) && args.act == ACT_GELU_GRAD) {
             // input-gradient GEMM / convolution: times gelu'(z) of the layer below, z read where the result is stored
             const __nv_bfloat16* zbase = static_cast<const __nv_bfloat16*>(args.aux) + ocol;
             uint2 z2[8];
@@ -552,7 +565,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
               xs[it].w *= gelu_grad(__uint_as_float(z2[it].y & 0xffff0000u));
             }
           }
-          if (EPI == EPI_BIAS_GELU && args.act == ACT_DUAL) {
+          if (!TF32 && EPI == EPI_BIAS_GELU && args.act == ACT_DUAL) {
             // training forward: the pre-activation stays in `out` for the backward pass, the activation goes to `aux`
 #pragma unroll
             for (int it = 0; it < 8; ++it)
@@ -568,8 +581,18 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
               gelu_erf2(xs[it].z, xs[it].w);
             }
           }
-          if (EPI == EPI_BIAS_GELU && AMODE != AMODE_CONV3 && args.gn_partials)
+          if (!TF32 && EPI == EPI_BIAS_GELU && AMODE != AMODE_CONV3 && args.gn_partials)
             gn_stats(xs, grow_it, t.m0 + (SUB == 1 ? 0 : sub * GEMM_BM) + q * 32, ncol);
+          if (TF32 && EPI != EPI_BIAS) {
+            // the FFN hidden activations of the TF32 path: fp32, rounded to TF32 so the next GEMM reads them exactly
+            float* of = static_cast<float*>(args.out) + ocol;
+#pragma unroll
+            for (int it = 0; it < 8; ++it)
+              if (grow_it[it] >= 0)
+                *reinterpret_cast<float4*>(of + (size_t)grow_it[it] * args.ldo) =
+                    make_float4(round_tf32(xs[it].x), round_tf32(xs[it].y), round_tf32(xs[it].z), round_tf32(xs[it].w));
+            continue;
+          }
           uint2 pk[8];
           if (out_f16) {
 #pragma unroll

@@ -279,6 +279,18 @@ __device__ __forceinline__ void umma_bf16_pair(uint32_t d_tmem, uint64_t adesc, 
       "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// The CTA-pair form with TF32 operands (see umma_tf32).
+__device__ __forceinline__ void umma_tf32_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                               uint32_t accumulate) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n"
+      "}\n" ::"r"(d_tmem),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // Arrives (count 1) on the barrier at this shared-memory offset in BOTH CTAs once the leader's MMAs retired.
 __device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
   asm volatile(
@@ -321,6 +333,26 @@ __host__ __device__ constexpr uint32_t umma_idesc_f16_f32(int M, int N) {
 }
 // format bits that turn umma_idesc_f16_f32 into umma_idesc_bf16_f32
 constexpr uint32_t UMMA_IDESC_BF16_BITS = (1u << 7) | (1u << 10);
+// Instruction descriptor, kind::tf32, TF32 x TF32 -> FP32, both operands K-major: the same fields as kind::f16 with
+// a_format = b_format = 2 (TF32) (PTX ISA, instruction descriptor table for .kind::f16 / .kind::tf32; cute::UMMA::
+// UMMAFormat::TF32). Each MMA consumes K = 8 fp32 values = 32 bytes of a K-major row, the same bytes as K = 16 of a
+// 16-bit operand, so the shared-memory descriptors and their per-MMA advance do not change.
+__host__ __device__ constexpr uint32_t umma_idesc_tf32_f32(int M, int N) {
+  return (1u << 4) | (2u << 7) | (2u << 10) | (static_cast<uint32_t>(N >> 3) << 17) |
+         (static_cast<uint32_t>(M >> 4) << 24);
+}
+// D[tmem] (+)= A * B with TF32 operands (fp32 containers; the tensor core reads the upper 19 bits); ONE thread.
+__device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                          uint32_t accumulate) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n"
+      "}\n" ::"r"(d_tmem),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 
 // ----------------------------------------------------------------------------- misc
 __device__ __forceinline__ float gelu_erf_exact(float x) { return 0.5f * x * (1.0f + erff(x * 0.70710678118654752f)); }
@@ -438,6 +470,14 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
 __device__ __forceinline__ uint32_t pack_f16x2(float lo, float hi) {
   __half2 v = __floats2half2_rn(lo, hi);
   return *reinterpret_cast<uint32_t*>(&v);
+}
+// fp32 -> the nearest TF32 value, ties away from zero (cvt.rna), in an fp32 container with the 13 low mantissa bits
+// zero: what a producer stores for a kind::tf32 GEMM, so the tensor core consumes exactly the stored value. The mask
+// makes the container's low bits zero whatever the conversion leaves in them.
+__device__ __forceinline__ float round_tf32(float x) {
+  uint32_t r;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
+  return __uint_as_float(r & 0xffffe000u);
 }
 // two fp32 -> one packed pair of the 16-bit operand type (F16: IEEE fp16, else bf16)
 template <bool F16>

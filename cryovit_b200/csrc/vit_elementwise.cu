@@ -19,8 +19,13 @@ __device__ __forceinline__ float cubic2(float x, float A) { return ((A * x - 5.f
 __device__ __forceinline__ float load_px(const uint8_t* p) { return static_cast<float>(*p) / 255.0f; }
 __device__ __forceinline__ float load_px(const float* p) { return *p; }
 
-template <typename T>
-__global__ void preproc_patchify_kernel(const T* __restrict__ src, __nv_bfloat16* __restrict__ dst, int D, int H,
+// Patch rows are stored as bf16 (the 16-bit operand paths) or, for the TF32 GEMMs, as TF32-rounded fp32: bf16 keeps 8
+// significant bits of the 10-bit-exact pixels the reference embeds, TF32 keeps 11.
+__device__ __forceinline__ void store_patch(__nv_bfloat16* p, float v) { *p = __float2bfloat16(v); }
+__device__ __forceinline__ void store_patch(float* p, float v) { *p = round_tf32(v); }
+
+template <typename T, typename OutT>
+__global__ void preproc_patchify_kernel(const T* __restrict__ src, OutT* __restrict__ dst, int D, int H,
                                         int W, int OH, int OW, int Kp, float inv_scale) {
   const int pw = OW / 14, ph = OH / 14;
   const int64_t total = (int64_t)D * ph * pw * Kp;
@@ -29,7 +34,7 @@ __global__ void preproc_patchify_kernel(const T* __restrict__ src, __nv_bfloat16
     const int col = (int)(idx % Kp);
     const int64_t row = idx / Kp;
     if (col >= 196) {
-      dst[idx] = __float2bfloat16(0.f);
+      store_patch(dst + idx, 0.f);
       continue;
     }
     const int p = (int)(row % (ph * pw));
@@ -59,7 +64,7 @@ __global__ void preproc_patchify_kernel(const T* __restrict__ src, __nv_bfloat16
       }
       acc += wy[i] * r;
     }
-    dst[idx] = __float2bfloat16(acc);
+    store_patch(dst + idx, acc);
   }
 }
 
@@ -98,7 +103,8 @@ __global__ void preproc_resize3_kernel(const T* __restrict__ src, float* __restr
 
 // General patchify for the reference-facing forward_features(x: f32[B,3,H',W']) entry (seam B2):
 // rows [b*Np + patch], cols c*196 + i*14 + j, zero-padded to Kp.
-__global__ void patchify3_kernel(const float* __restrict__ src, __nv_bfloat16* __restrict__ dst, int B, int OH, int OW,
+template <typename OutT>
+__global__ void patchify3_kernel(const float* __restrict__ src, OutT* __restrict__ dst, int B, int OH, int OW,
                                  int Kp) {
   const int pw = OW / 14, ph = OH / 14;
   const int64_t total = (int64_t)B * ph * pw * Kp;
@@ -107,7 +113,7 @@ __global__ void patchify3_kernel(const float* __restrict__ src, __nv_bfloat16* _
     const int col = (int)(idx % Kp);
     const int64_t row = idx / Kp;
     if (col >= 588) {
-      dst[idx] = __float2bfloat16(0.f);
+      store_patch(dst + idx, 0.f);
       continue;
     }
     const int c = col / 196, ij = col % 196;
@@ -115,7 +121,7 @@ __global__ void patchify3_kernel(const float* __restrict__ src, __nv_bfloat16* _
     const int b = (int)(row / (ph * pw));
     const int oy = (p / pw) * 14 + ij / 14;
     const int ox = (p % pw) * 14 + ij % 14;
-    dst[idx] = __float2bfloat16(src[(((int64_t)b * 3 + c) * OH + oy) * OW + ox]);
+    store_patch(dst + idx, src[(((int64_t)b * 3 + c) * OH + oy) * OW + ox]);
   }
 }
 
@@ -144,6 +150,13 @@ __device__ __forceinline__ void ln_store4(__half* row, int i4, float o0, float o
 }
 __device__ __forceinline__ void ln_store4(float* row, int i4, float o0, float o1, float o2, float o3) {
   reinterpret_cast<float4*>(row)[i4] = make_float4(o0, o1, o2, o3);
+}
+// fp32 output rounded to TF32: the A operand of the TF32 linears (cvit_layernorm_f32_tf32)
+struct Tf32Out {
+  float v;
+};
+__device__ __forceinline__ void ln_store4(Tf32Out* row, int i4, float o0, float o1, float o2, float o3) {
+  reinterpret_cast<float4*>(row)[i4] = make_float4(round_tf32(o0), round_tf32(o1), round_tf32(o2), round_tf32(o3));
 }
 
 template <int NV, typename OutT>  // float4 per lane: C == NV * 128
@@ -274,11 +287,10 @@ static int grid_for(int64_t total, int threads) {
 
 using namespace cvit;
 
-extern "C" {
-
-int cvit_preproc_patchify(const void* src, int src_is_u8, void* patches_bf16, int64_t D, int64_t H, int64_t W,
-                          int64_t Kp, void* stream) {
-  if (!src || !patches_bf16 || D <= 0 || H <= 0 || W <= 0 || Kp < 196 || (Kp % 64) != 0) {
+template <typename OutT>
+static int preproc_patchify(const void* src, int src_is_u8, OutT* patches, int64_t D, int64_t H, int64_t W, int64_t Kp,
+                            void* stream) {
+  if (!src || !patches || D <= 0 || H <= 0 || W <= 0 || Kp < 196 || (Kp % 64) != 0) {
     set_error("preproc_patchify: bad arguments (D=%lld H=%lld W=%lld Kp=%lld)", (long long)D, (long long)H,
               (long long)W, (long long)Kp);
     return CVIT_ERR_INVALID;
@@ -289,14 +301,36 @@ int cvit_preproc_patchify(const void* src, int src_is_u8, void* patches_bf16, in
   const int64_t total = D * (OH / 14) * (OW / 14) * Kp;
   const int grid = grid_for(total, 256);
   if (src_is_u8)
-    preproc_patchify_kernel<uint8_t><<<grid, 256, 0, (cudaStream_t)stream>>>(
-        static_cast<const uint8_t*>(src), static_cast<__nv_bfloat16*>(patches_bf16), (int)D, (int)H, (int)W, OH, OW,
-        (int)Kp, inv_scale);
+    preproc_patchify_kernel<uint8_t, OutT><<<grid, 256, 0, (cudaStream_t)stream>>>(
+        static_cast<const uint8_t*>(src), patches, (int)D, (int)H, (int)W, OH, OW, (int)Kp, inv_scale);
   else
-    preproc_patchify_kernel<float><<<grid, 256, 0, (cudaStream_t)stream>>>(
-        static_cast<const float*>(src), static_cast<__nv_bfloat16*>(patches_bf16), (int)D, (int)H, (int)W, OH, OW,
-        (int)Kp, inv_scale);
+    preproc_patchify_kernel<float, OutT><<<grid, 256, 0, (cudaStream_t)stream>>>(
+        static_cast<const float*>(src), patches, (int)D, (int)H, (int)W, OH, OW, (int)Kp, inv_scale);
   return check_launch("preproc_patchify_kernel");
+}
+
+template <typename OutT>
+static int patchify_f32_3ch(const float* src, OutT* patches, int64_t B, int64_t OH, int64_t OW, int64_t Kp, void* stream) {
+  if (!src || !patches || B <= 0 || OH <= 0 || OW <= 0 || (OH % 14) || (OW % 14) || Kp < 588 || (Kp % 64)) {
+    set_error("patchify_f32_3ch: bad arguments (B=%lld OH=%lld OW=%lld Kp=%lld)", (long long)B, (long long)OH,
+              (long long)OW, (long long)Kp);
+    return CVIT_ERR_INVALID;
+  }
+  const int64_t total = B * (OH / 14) * (OW / 14) * Kp;
+  patchify3_kernel<OutT><<<grid_for(total, 256), 256, 0, (cudaStream_t)stream>>>(src, patches, (int)B, (int)OH, (int)OW, (int)Kp);
+  return check_launch("patchify3_kernel");
+}
+
+extern "C" {
+
+int cvit_preproc_patchify(const void* src, int src_is_u8, void* patches_bf16, int64_t D, int64_t H, int64_t W,
+                          int64_t Kp, void* stream) {
+  return preproc_patchify(src, src_is_u8, static_cast<__nv_bfloat16*>(patches_bf16), D, H, W, Kp, stream);
+}
+
+int cvit_preproc_patchify_tf32(const void* src, int src_is_u8, float* patches, int64_t D, int64_t H, int64_t W,
+                               int64_t Kp, void* stream) {
+  return preproc_patchify(src, src_is_u8, patches, D, H, W, Kp, stream);
 }
 
 int cvit_preproc_resize_f32_3ch(const void* src, int src_is_u8, float* out, int64_t D, int64_t H, int64_t W,
@@ -319,15 +353,12 @@ int cvit_preproc_resize_f32_3ch(const void* src, int src_is_u8, float* out, int6
 
 int cvit_patchify_f32_3ch(const float* src, void* patches_bf16, int64_t B, int64_t OH, int64_t OW, int64_t Kp,
                           void* stream) {
-  if (!src || !patches_bf16 || B <= 0 || OH <= 0 || OW <= 0 || (OH % 14) || (OW % 14) || Kp < 588 || (Kp % 64)) {
-    set_error("patchify_f32_3ch: bad arguments (B=%lld OH=%lld OW=%lld Kp=%lld)", (long long)B, (long long)OH,
-              (long long)OW, (long long)Kp);
-    return CVIT_ERR_INVALID;
-  }
-  const int64_t total = B * (OH / 14) * (OW / 14) * Kp;
-  patchify3_kernel<<<grid_for(total, 256), 256, 0, (cudaStream_t)stream>>>(
-      src, static_cast<__nv_bfloat16*>(patches_bf16), (int)B, (int)OH, (int)OW, (int)Kp);
-  return check_launch("patchify3_kernel");
+  return patchify_f32_3ch(src, static_cast<__nv_bfloat16*>(patches_bf16), B, OH, OW, Kp, stream);
+}
+
+int cvit_patchify_f32_3ch_tf32(const float* src, float* patches, int64_t B, int64_t OH, int64_t OW, int64_t Kp,
+                               void* stream) {
+  return patchify_f32_3ch(src, patches, B, OH, OW, Kp, stream);
 }
 
 int cvit_assemble_special_tokens(float* x, const float* special, int64_t B, int64_t T, int64_t C, int64_t S,
@@ -367,6 +398,15 @@ int cvit_layernorm_f32_f32(const float* x, int64_t ldx, const float* gamma, cons
     return CVIT_ERR_INVALID;
   }
   return launch_layernorm(x, ldx, gamma, beta, out, ldo, M, C, eps, (cudaStream_t)stream);
+}
+
+int cvit_layernorm_f32_tf32(const float* x, int64_t ldx, const float* gamma, const float* beta, float* out,
+                            int64_t ldo, int64_t M, int64_t C, float eps, void* stream) {
+  if (!x || !gamma || !beta || !out || M <= 0 || (ldx % 4) || (ldo % 4)) {
+    set_error("layernorm_tf32: bad arguments");
+    return CVIT_ERR_INVALID;
+  }
+  return launch_layernorm(x, ldx, gamma, beta, reinterpret_cast<Tf32Out*>(out), ldo, M, C, eps, (cudaStream_t)stream);
 }
 
 int cvit_final_norm_writeout_f16(const float* x, const float* gamma, const float* beta, void* features_f16,

@@ -32,10 +32,12 @@ def patch_grid(H: int, W: int) -> tuple[int, int, int, int]:
 
 
 def preproc_patchify(src: torch.Tensor, out: torch.Tensor) -> None:
-    """src u8|f32 [D,H,W] -> out bf16 [D*Np, Kp] (one channel, Kp >= 196)."""
+    """src u8|f32 [D,H,W] -> out [D*Np, Kp] (one channel, Kp >= 196): bf16, or fp32 rounded to TF32 (the TF32 patch
+    embedding's operand) when ``out`` is fp32."""
     D, H, W = src.shape
     is_u8 = src.dtype == U8
-    _lib.call("cvit_preproc_patchify", _chk(src, U8 if is_u8 else F32, "src"), int(is_u8), _chk(out, BF16, "out"),
+    name = "cvit_preproc_patchify_tf32" if out.dtype == F32 else "cvit_preproc_patchify"
+    _lib.call(name, _chk(src, U8 if is_u8 else F32, "src"), int(is_u8), _chk(out, F32 if out.dtype == F32 else BF16, "out"),
               D, H, W, out.shape[1], _stream())
 
 
@@ -54,14 +56,20 @@ def patchify_f32_3ch(src: torch.Tensor, out: torch.Tensor) -> None:
     B, C, OH, OW = src.shape
     if C != 3:
         raise _lib.CryovitB200Error("patchify_f32_3ch: expected [B,3,H,W]")
-    _lib.call("cvit_patchify_f32_3ch", _chk(src, F32, "src"), _chk(out, BF16, "out"), B, OH, OW, out.shape[1], _stream())
+    # fp32 out: TF32-rounded patch rows for the TF32 patch embedding
+    name = "cvit_patchify_f32_3ch_tf32" if out.dtype == F32 else "cvit_patchify_f32_3ch"
+    _lib.call(name, _chk(src, F32, "src"), _chk(out, F32 if out.dtype == F32 else BF16, "out"), B, OH, OW, out.shape[1],
+              _stream())
 
 
 def patch_embed_gemm(patches, w, table, x, n_slices, n_patches, tokens, first_patch_token) -> None:
+    """bf16 patches x bf16 weight, or (both fp32 holding TF32 values) a TF32 GEMM."""
     N, K = w.shape
-    _lib.call("cvit_patch_embed_gemm", _chk(patches, BF16, "patches"), patches.shape[1], _chk(w, BF16, "w"),
+    if patches.dtype not in (BF16, F32) or w.dtype != patches.dtype:
+        raise _lib.CryovitB200Error(f"patch_embed: patches and weight must both be bf16 or both fp32, got {patches.dtype} x {w.dtype}")
+    _lib.call("cvit_patch_embed_gemm_fmt", _chk(patches, patches.dtype, "patches"), patches.shape[1], _chk(w, w.dtype, "w"),
               _chk(table, F32, "table"), _chk(x, F32, "x"), x.shape[-1], n_slices, n_patches, tokens,
-              first_patch_token, N, K, _stream())
+              first_patch_token, N, K, FMT_OPERANDS_TF32 if w.dtype == F32 else 0, _stream())
 
 
 def assemble_special_tokens(x: torch.Tensor, special: torch.Tensor, B: int, T: int) -> None:
@@ -69,10 +77,13 @@ def assemble_special_tokens(x: torch.Tensor, special: torch.Tensor, B: int, T: i
     _lib.call("cvit_assemble_special_tokens", _chk(x, F32, "x"), _chk(special, F32, "special"), B, T, C, S, _stream())
 
 
-def layernorm(x: torch.Tensor, gamma, beta, out: torch.Tensor, eps: float) -> None:
+def layernorm(x: torch.Tensor, gamma, beta, out: torch.Tensor, eps: float, tf32: bool = False) -> None:
+    """x fp32 -> out bf16 | fp16 | fp32; ``tf32`` (fp32 out only) rounds the result to TF32 for a TF32 linear."""
     M, C = x.shape
+    if tf32 and out.dtype != F32:
+        raise _lib.CryovitB200Error(f"layernorm: TF32 rounding needs an fp32 output, got {out.dtype}")
     if out.dtype == F32:
-        _lib.call("cvit_layernorm_f32_f32", _chk(x, F32, "x"), x.stride(0), _chk(gamma, F32, "gamma"),
+        _lib.call("cvit_layernorm_f32_tf32" if tf32 else "cvit_layernorm_f32_f32", _chk(x, F32, "x"), x.stride(0), _chk(gamma, F32, "gamma"),
                   _chk(beta, F32, "beta"), _chk(out, F32, "out"), out.stride(0), M, C, float(eps), _stream())
         return
     name = "cvit_layernorm_f32_f16" if out.dtype == F16 else "cvit_layernorm_f32_bf16"
@@ -80,23 +91,27 @@ def layernorm(x: torch.Tensor, gamma, beta, out: torch.Tensor, eps: float) -> No
               _chk(beta, F32, "beta"), _chk(out, out.dtype if out.dtype == F16 else BF16, "out"), out.stride(0), M, C, float(eps), _stream())
 
 
-FMT_OPERANDS_F16, FMT_OUT_F16 = 1, 2  # include/cryovit_b200.h CVIT_FMT_*
+FMT_OPERANDS_F16, FMT_OUT_F16, FMT_OPERANDS_TF32, FMT_OUT_F32 = 1, 2, 4, 8  # include/cryovit_b200.h CVIT_FMT_*
 
 
-def _fmt16(a, w, out=None) -> int:
-    """Format flags of a linear from the tensors' own dtypes: A and W must share one 16-bit type (bf16 or fp16: a
-    tcgen05 kind::f16 MMA takes one type for both operands); a 16-bit output may be either."""
-    if a.dtype not in (BF16, F16) or w.dtype != a.dtype:
-        raise _lib.CryovitB200Error(f"linear: operands must both be bf16 or both fp16, got {a.dtype} x {w.dtype}")
-    if out is not None and out.dtype not in (BF16, F16):
-        raise _lib.CryovitB200Error(f"linear: output must be bf16 or fp16, got {out.dtype}")
-    return (FMT_OPERANDS_F16 if a.dtype == F16 else 0) | (FMT_OUT_F16 if out is not None and out.dtype == F16 else 0)
+def _fmt(a, w, out=None) -> int:
+    """Format flags of a linear from the tensors' own dtypes: A and W share one type -- bf16 or fp16 (a tcgen05
+    kind::f16 MMA takes one type for both operands), or fp32 holding TF32 values (kind::tf32). The output may be bf16,
+    fp16 or, with fp32 operands, fp32; the library refuses a combination it has no kernel for."""
+    if a.dtype not in (BF16, F16, F32) or w.dtype != a.dtype:
+        raise _lib.CryovitB200Error(f"linear: operands must both be bf16, both fp16 or both fp32 (TF32), got {a.dtype} x {w.dtype}")
+    if out is not None and (out.dtype not in (BF16, F16, F32) or (out.dtype == F32 and a.dtype != F32)):
+        raise _lib.CryovitB200Error(f"linear: output must be bf16 or fp16 (or fp32 with fp32 operands), got {out.dtype}")
+    fmt = {F16: FMT_OPERANDS_F16, F32: FMT_OPERANDS_TF32}.get(a.dtype, 0)
+    if out is not None:
+        fmt |= {F16: FMT_OUT_F16, F32: FMT_OUT_F32}.get(out.dtype, 0)
+    return fmt
 
 
 def linear_bias(a, w, bias, out, gelu: bool = False) -> None:
     M, K = a.shape
     N = w.shape[0]
-    fmt = _fmt16(a, w, out)
+    fmt = _fmt(a, w, out)
     _lib.call("cvit_linear_bias_fmt", _chk(a, a.dtype, "a"), a.stride(0), _chk(w, w.dtype, "w"), _chk(bias, F32, "bias"),
               _chk(out, out.dtype, "out"), out.stride(0), M, N, K, int(gelu), fmt, _stream())
 
@@ -214,7 +229,7 @@ def conv3d_wpackn(x, w_img, table, out, dil: int, cout_pad: int, act=True, aux=N
 def linear_swiglu(a, w12i, bias12i, out) -> None:
     M, K = a.shape
     N2 = w12i.shape[0]
-    fmt = _fmt16(a, w12i, out)
+    fmt = _fmt(a, w12i, out)
     _lib.call("cvit_linear_swiglu_fmt", _chk(a, a.dtype, "a"), a.stride(0), _chk(w12i, w12i.dtype, "w12i"),
               _chk(bias12i, F32, "bias12i"), _chk(out, out.dtype, "out"), out.stride(0), M, N2, K, fmt, _stream())
 
@@ -222,16 +237,17 @@ def linear_swiglu(a, w12i, bias12i, out) -> None:
 def linear_scale_residual(a, w, bias, gamma, x) -> None:
     M, K = a.shape
     N = w.shape[0]
-    fmt = _fmt16(a, w)
+    fmt = _fmt(a, w)
     _lib.call("cvit_linear_scale_residual_fmt", _chk(a, a.dtype, "a"), a.stride(0), _chk(w, w.dtype, "w"),
               _chk(bias, F32, "bias"), _chk(gamma, F32, "gamma"), _chk(x, F32, "x"), x.stride(0), M, N, K, fmt, _stream())
 
 
 def attention(qkv, out, n_slices: int, tokens: int, heads: int, legacy_mma_sync: bool = False) -> None:
+    """out bf16 | fp16 | fp32 (TF32-rounded, from bf16 q/k/v only)."""
     if not legacy_mma_sync:
-        if qkv.dtype not in (BF16, F16) or out.dtype not in (BF16, F16) or (qkv.dtype == F16 and out.dtype != F16):
+        if qkv.dtype not in (BF16, F16) or out.dtype not in (BF16, F16, F32) or (qkv.dtype == F16 and out.dtype != F16):
             raise _lib.CryovitB200Error(f"attention: unsupported formats qkv {qkv.dtype} -> out {out.dtype}")
-        fmt = (FMT_OPERANDS_F16 if qkv.dtype == F16 else 0) | (FMT_OUT_F16 if out.dtype == F16 else 0)
+        fmt = (FMT_OPERANDS_F16 if qkv.dtype == F16 else 0) | {F16: FMT_OUT_F16, F32: FMT_OUT_F32}.get(out.dtype, 0)
         _lib.call("cvit_attention_fwd_fmt", _chk(qkv, qkv.dtype, "qkv"), _chk(out, out.dtype, "out"), n_slices, tokens, heads, 64,
                   fmt, _stream())
         return

@@ -16,7 +16,15 @@ Layout in HBM for a batch of B slices (T tokens per slice, C channels, F hidden)
     hidden   bf16 [B*T, F]        post-activation FFN hidden
     features fp16 [C, D, Np]      the reference's on-disk layout (C, D, h, w)
 
-op16 = the operand format, chosen by ``operands`` (``"mixed-attn"`` default | ``"mixed"`` | ``"fp16"`` | ``"bf16"``). The reference runs
+``operands="tf32"`` runs every linear (patch embedding, qkv, proj, w12 / fc1, w3 / fc2) as a tcgen05 kind::tf32 MMA,
+the reference's own matmul precision (run/dino_features.py:24 ``set_float32_matmul_precision("high")``): patches, ln,
+attn and hidden are fp32 holding TF32-rounded values, and so are the weights (rounded once when packed); q/k/v and the
+softmax probabilities stay bf16 (the emulation in tests/quant_emulation.py shows their format does not move the
+end-to-end error). The FFN hidden activations and w3 / fc2, where DINOv2's large-magnitude channels are born, get 10
+mantissa bits at fp32 range, so the error tracks the reference's own arithmetic on ill-conditioned (trained-like)
+weights too, at half the tensor-core rate of the 16-bit modes. The features are written as fp16 in every mode.
+
+op16 = the operand format of the 16-bit modes, chosen by ``operands`` (``"mixed-attn"`` default | ``"mixed"`` | ``"fp16"`` | ``"bf16"``). The reference runs
 these GEMMs in TF32 (10 mantissa bits). ln and the attention output are bounded (LayerNorm output times gamma; convex
 combinations of v), so ``mixed`` / ``fp16`` give them and the weights they meet (qkv, proj, w12 / fc1) the same 10 bits
 as IEEE fp16 at the same bytes (bf16 has 7); the FFN hidden activations, where DINOv2's large-magnitude channels are
@@ -66,7 +74,7 @@ def _swiglu_hidden(dim: int) -> int:
     return (int(4 * dim * 2 / 3) + 7) // 8 * 8
 
 
-OPERAND_MODES = ("mixed-attn", "mixed", "fp16", "bf16")
+OPERAND_MODES = ("mixed-attn", "mixed", "fp16", "bf16", "tf32")
 DEFAULT_OPERANDS = "mixed-attn"
 
 CONFIGS = {
@@ -159,11 +167,14 @@ class DinoVisionTransformerB200:
         if operands not in OPERAND_MODES:
             raise CryovitB200Error(f"operands must be one of {OPERAND_MODES} (or torch.float16 / torch.bfloat16), got {operands!r}")
         self.operands = operands
+        self.tf32 = operands == "tf32"
         # ln / attention output / qkv, proj, w12 weights  |  q, k, v and the softmax probabilities
-        self.operand_dtype = torch.bfloat16 if operands == "bf16" else torch.float16
+        self.operand_dtype = torch.float32 if self.tf32 else torch.bfloat16 if operands == "bf16" else torch.float16
         self.qkv_dtype = torch.float16 if operands == "fp16" else torch.bfloat16
         # norm2 output and the w12 / fc1 weights it meets: "mixed-attn" keeps the FFN (44 % of the FLOPs) all-bf16
-        self.ffn_dtype = torch.bfloat16 if operands in ("bf16", "mixed-attn") else torch.float16
+        self.ffn_dtype = self.operand_dtype if operands in ("tf32", "mixed", "fp16") else torch.bfloat16
+        # patches, FFN hidden activations and the patch-embed / w3 / fc2 weights: bf16 in every 16-bit mode
+        self.hidden_dtype = torch.float32 if self.tf32 else torch.bfloat16
         self.device: torch.device | None = None
         self._sd_cpu: dict[str, torch.Tensor] | None = None
         self._w: dict = {}
@@ -221,12 +232,14 @@ class DinoVisionTransformerB200:
     def _pack(self) -> None:
         cfg, sd, dev = self.cfg, self._sd_cpu, self.device
         C = cfg.embed_dim
-        bf = lambda t: t.to(dev).to(torch.bfloat16).contiguous()
         f32 = lambda t: t.to(dev).float().contiguous()
+        # weights of the bf16 side (patch embedding, w3 / fc2): TF32-rounded fp32 in tf32 mode
+        bf = (lambda t: round_tf32(f32(t))) if self.tf32 else (lambda t: t.to(dev).to(torch.bfloat16).contiguous())
         if self.operand_dtype == torch.float16:
             def op(t):  # weights that meet an fp16 activation; fail loudly rather than store an inf
                 if float(t.abs().max()) > 6.0e4:
-                    raise CryovitB200Error("a weight exceeds the fp16 range: construct the model with operand_dtype=torch.bfloat16")
+                    raise CryovitB200Error("a weight exceeds the fp16 range: construct the model with operands='bf16' "
+                                           "or operands='tf32'")
                 return t.to(dev).to(torch.float16).contiguous()
         else:
             op = bf
@@ -277,17 +290,17 @@ class DinoVisionTransformerB200:
         if key not in self._ws:
             cfg, dev = self.cfg, self.device
             C, Fh, M = cfg.embed_dim, cfg.hidden, B * T
-            bf16 = dict(device=dev, dtype=torch.bfloat16)
+            hid = dict(device=dev, dtype=self.hidden_dtype)
             op16 = dict(device=dev, dtype=self.operand_dtype)
             self._ws = {  # keep one shape alive: a different batch shape replaces the buffers
                 key: {
-                    "patches": torch.empty(B * Np, kp, **bf16),
+                    "patches": torch.empty(B * Np, kp, **hid),
                     "x": torch.empty(M, C, device=dev, dtype=torch.float32),
                     "ln": torch.empty(M, C, **op16),
                     "ln2": torch.empty(M if self.ffn_dtype != self.operand_dtype else 0, C, device=dev, dtype=self.ffn_dtype),
                     "qkv": torch.empty(M, 3 * C, device=dev, dtype=self.qkv_dtype),
                     "attn": torch.empty(M, C, **op16),
-                    "hidden": torch.empty(M, Fh, **bf16),
+                    "hidden": torch.empty(M, Fh, **hid),
                 }
             }
         return self._ws[key]
@@ -303,12 +316,12 @@ class DinoVisionTransformerB200:
         ln2 = ws["ln2"] if self.ffn_dtype != self.operand_dtype else ln
         for i, b in enumerate(self._w["blocks"]):
             with nvtx.span(f"vit.block{i}.attn"):
-                ops.layernorm(x, b["n1w"], b["n1b"], ln, cfg.ln_eps)
+                ops.layernorm(x, b["n1w"], b["n1b"], ln, cfg.ln_eps, tf32=self.tf32)
                 ops.linear_bias(ln, b["qkv_w"], b["qkv_b"], qkv)
                 ops.attention(qkv, attn, B, T, cfg.num_heads)
                 ops.linear_scale_residual(attn, b["proj_w"], b["proj_b"], b["ls1"], x)
             with nvtx.span(f"vit.block{i}.ffn"):
-                ops.layernorm(x, b["n2w"], b["n2b"], ln2, cfg.ln_eps)
+                ops.layernorm(x, b["n2w"], b["n2b"], ln2, cfg.ln_eps, tf32=self.tf32)
                 if cfg.ffn == "swiglu":
                     ops.linear_swiglu(ln2, b["w12i"], b["b12i"], hidden)
                 else:
@@ -386,6 +399,15 @@ class DinoVisionTransformerB200:
         self.launches += 2
 
 
+def round_tf32(t: torch.Tensor) -> torch.Tensor:
+    """fp32 -> the nearest TF32 value (8 exponent, 10 mantissa bits), ties away from zero, in fp32 with the 13 low
+    mantissa bits zero: what cvt.rna.tf32.f32 gives for finite inputs. Non-finite values are refused."""
+    t = t.float().contiguous()
+    if not bool(torch.isfinite(t).all()):
+        raise CryovitB200Error("round_tf32: the tensor holds inf or nan")
+    return ((t.view(torch.int32) + 0x1000) & ~0x1FFF).view(torch.float32)
+
+
 def random_state_dict_keys(cfg: ViTConfig) -> list[str]:
     keys = ["cls_token", "pos_embed", "register_tokens", "patch_embed.proj.weight", "patch_embed.proj.bias",
             "norm.weight", "norm.bias"]
@@ -401,7 +423,7 @@ def random_state_dict_keys(cfg: ViTConfig) -> list[str]:
 def build_model(name: str = "dinov2_vitg14_reg", state_dict: dict | None = None, seed: int = 0,
                 operands: str | torch.dtype | None = None) -> DinoVisionTransformerB200:
     """Stand-in for torch.hub.load(*dino_model): random-init (seeded) unless a state dict is given. ``operands``
-    None reads CRYOVIT_B200_OPERANDS (``mixed-attn`` | ``mixed`` | ``fp16`` | ``bf16``, default mixed-attn), so the Hydra entry points can
+    None reads CRYOVIT_B200_OPERANDS (``mixed-attn`` | ``mixed`` | ``fp16`` | ``bf16`` | ``tf32``, default mixed-attn), so the Hydra entry points can
     switch it without a config key the reference does not have."""
     if operands is None:
         import os

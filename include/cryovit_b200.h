@@ -66,6 +66,15 @@ int cvit_preproc_resize_f32_3ch(const void* src, int src_is_u8, float* out, int6
 int cvit_patchify_f32_3ch(const float* src, void* patches_bf16, int64_t B, int64_t OH, int64_t OW, int64_t Kp,
                           void* stream);
 
+/* The two patchify entry points above with fp32 output rounded to TF32 (nearest, ties away from zero; the 13 low
+ * mantissa bits zero): the patch rows of the TF32 patch embedding (cvit_patch_embed_gemm_fmt with
+ * CVIT_FMT_OPERANDS_TF32), which keeps the 10-bit-exact pixels the reference embeds in TF32
+ * (run/dino_features.py:24, set_float32_matmul_precision("high")) where bf16 would keep 8 bits. */
+int cvit_preproc_patchify_tf32(const void* src, int src_is_u8, float* patches, int64_t D, int64_t H, int64_t W,
+                               int64_t Kp, void* stream);
+int cvit_patchify_f32_3ch_tf32(const float* src, float* patches, int64_t B, int64_t OH, int64_t OW, int64_t Kp,
+                               void* stream);
+
 /* Patch-embed GEMM: x[b, first_patch_token + p, :] = patches[b*Np + p, :] @ W^T + pos_bias_table[p, :].
  * Replaces upstream PatchEmbed.proj (conv 14/14 as a GEMM) + the pos-embed add of prepare_tokens_with_masks
  * (HF:61-71,147-173).  W: bf16 [N, K] row-major; table: fp32 [Np, N] = interpolated pos-embed + conv bias;
@@ -73,6 +82,12 @@ int cvit_patchify_f32_3ch(const float* src, void* patches_bf16, int64_t B, int64
 int cvit_patch_embed_gemm(const void* patches, int64_t lda, const void* W, const float* pos_bias_table, float* x,
                           int64_t ldx, int64_t n_slices, int64_t n_patches, int64_t tokens_per_slice,
                           int64_t first_patch_token, int64_t N, int64_t K, void* stream);
+/* The same GEMM by format flags: fmt = 0 (bf16 patches and W, = cvit_patch_embed_gemm) or CVIT_FMT_OPERANDS_TF32
+ * (patches and W fp32 holding TF32 values: the reference's TF32 conv, run/dino_features.py:24; lda and K in fp32
+ * elements).  Other flags return CVIT_ERR_UNSUPPORTED. */
+int cvit_patch_embed_gemm_fmt(const void* patches, int64_t lda, const void* W, const float* pos_bias_table, float* x,
+                              int64_t ldx, int64_t n_slices, int64_t n_patches, int64_t tokens_per_slice,
+                              int64_t first_patch_token, int64_t N, int64_t K, int fmt, void* stream);
 
 /* x[b, s, :] = special[s, :] for s < S (cls + pos[0], then the register tokens; HF:147-173). */
 int cvit_assemble_special_tokens(float* x, const float* special, int64_t B, int64_t T, int64_t C, int64_t S,
@@ -91,6 +106,12 @@ int cvit_layernorm_f32_f16(const float* x, int64_t ldx, const float* gamma, cons
  * the fused fp16 write-out below. */
 int cvit_layernorm_f32_f32(const float* x, int64_t ldx, const float* gamma, const float* beta, float* out,
                            int64_t ldo, int64_t M, int64_t C, float eps, void* stream);
+
+/* Same with fp32 output rounded to TF32 (nearest, ties away from zero; the 13 low mantissa bits zero): Block.norm1 /
+ * norm2 as the A operand of the TF32 linears (CVIT_FMT_OPERANDS_TF32), which the reference runs in TF32
+ * (run/dino_features.py:24). */
+int cvit_layernorm_f32_tf32(const float* x, int64_t ldx, const float* gamma, const float* beta, float* out,
+                            int64_t ldo, int64_t M, int64_t C, float eps, void* stream);
 
 /* out_bf16[M, N] = A[M, K] @ W[N, K]^T + bias, optionally followed by exact-erf GELU.  Replaces attn.qkv
  * (HF:219-221) and, with gelu=1, Mlp.fc1 + GELU of ViT-S/B/L and the head's 1x1x1 Conv3d + GELU
@@ -116,10 +137,20 @@ int cvit_linear_scale_residual_f32(const void* A, int64_t lda, const void* W, co
  * choice where range matters (the FFN hidden activations).  `fmt` is a combination of:
  *   CVIT_FMT_OPERANDS_F16  A and W hold IEEE fp16 instead of bf16 (always both: a tcgen05 kind::f16 MMA takes one
  *                          16-bit type for both operands);
- *   CVIT_FMT_OUT_F16       the 16-bit output of linear_bias / linear_swiglu is stored as fp16 instead of bf16.
- * fmt = 0 is exactly the *_bf16 / *_f32 entry point of the same name. */
+ *   CVIT_FMT_OUT_F16       the 16-bit output of linear_bias / linear_swiglu is stored as fp16 instead of bf16;
+ *   CVIT_FMT_OPERANDS_TF32 A and W are fp32 holding TF32 values (tcgen05 kind::tf32, half the kind::f16 rate): the
+ *                          reference's own matmul precision (run/dino_features.py:24).  lda and K in fp32 elements,
+ *                          multiples of 4, K >= 32;
+ *   CVIT_FMT_OUT_F32       with CVIT_FMT_OPERANDS_TF32, and required there by linear_bias with gelu = 1 and by
+ *                          linear_swiglu: the output is fp32 rounded to TF32, the A operand of the next TF32 linear.
+ *                          linear_bias without GELU (qkv) keeps its 16-bit output under TF32 operands.
+ * Combinations without an instantiated kernel (TF32 with fp16 operands, CVIT_FMT_OUT_F32 without TF32 operands or
+ * on the 16-bit outputs) return CVIT_ERR_UNSUPPORTED.  fmt = 0 is exactly the *_bf16 / *_f32 entry point of the
+ * same name. */
 #define CVIT_FMT_OPERANDS_F16 1
 #define CVIT_FMT_OUT_F16 2
+#define CVIT_FMT_OPERANDS_TF32 4
+#define CVIT_FMT_OUT_F32 8
 int cvit_linear_bias_fmt(const void* A, int64_t lda, const void* W, const float* bias, void* out, int64_t ldo,
                          int64_t M, int64_t N, int64_t K, int gelu, int fmt, void* stream);
 int cvit_linear_swiglu_fmt(const void* A, int64_t lda, const void* W12i, const float* bias12i, void* out,
@@ -146,7 +177,9 @@ int cvit_attention_fwd_f16(const void* qkv, void* out, int64_t n_slices, int64_t
                            int64_t head_dim, void* stream);
 /* The same kernel by format flags: fmt = 0 (all bf16), CVIT_FMT_OUT_F16 (bf16 q/k/v and probabilities, fp16 output:
  * the default ViT path -- the format of q/k/v/P does not move the end-to-end error, the format of the output that
- * meets the projection weights does), or CVIT_FMT_OPERANDS_F16 | CVIT_FMT_OUT_F16 (= cvit_attention_fwd_f16). */
+ * meets the projection weights does), CVIT_FMT_OPERANDS_F16 | CVIT_FMT_OUT_F16 (= cvit_attention_fwd_f16), or
+ * CVIT_FMT_OUT_F32 (bf16 q/k/v and probabilities, output fp32 rounded to TF32 for a TF32 projection).  Other flags
+ * return CVIT_ERR_UNSUPPORTED. */
 int cvit_attention_fwd_fmt(const void* qkv, void* out, int64_t n_slices, int64_t tokens, int64_t heads,
                            int64_t head_dim, int fmt, void* stream);
 /* Same contract on the legacy warp-level mma.sync path: kept only as an A/B comparison kernel for profiles. */
