@@ -69,6 +69,8 @@ SIGNATURES: dict[str, list] = {
     "cvit_conv3d_wpack8_aux": [P, P, P, P, I64, I64, I64, I32, P, P],
     "cvit_conv3d_rows8": [P, P, P, P, I64, I64, I64, I32, P, P, P],
     "cvit_conv3d_rows8_final": [P, P, P, P, P, I64, I64, I64, P],
+    "cvit_conv3d_rows8_score": [P, P, P, P, I64, I64, I64, F32, P, P, P],
+    "cvit_conv3d_rows8_score_partials": [I64, I64, I64],  # returns a size, not an error code (restype set in load())
     "cvit_conv3d_rows_ndhwc": [P, P, P, P, I64, I64, I64, I64, I64, I64, I32, P, P, P],
     "cvit_gelu_fwd_bf16": [P, P, I64, P],
     "cvit_gelu_bwd_bf16": [P, P, P, I64, P],
@@ -136,6 +138,7 @@ def load() -> ctypes.CDLL:
         fn = getattr(lib, name)  # AttributeError if the symbol is not exported
         fn.restype = c_int
         fn.argtypes = argtypes
+    lib.cvit_conv3d_rows8_score_partials.restype = c_int64
     _lib = lib
     return lib
 

@@ -72,6 +72,9 @@ struct CrArgs {
   float* logits;               // FINAL: [D, H, W] clipped logits (may be null)
   float* probs;                // FINAL: [D, H, W] sigmoid of the clipped logits (may be null)
   int D, H, W, act;
+  const int8_t* labels;        // SCORE: [D, H, W], -1 = ignore
+  double* partials;            // SCORE: [gridDim.x][8], one row per CTA
+  float thr;                   // SCORE: threshold of sums 3 and 4
 };
 
 __device__ __forceinline__ uint64_t cr_desc(uint32_t addr, uint32_t lbo, uint32_t sbo) {  // K-major SWIZZLE_NONE
@@ -84,10 +87,21 @@ __device__ __forceinline__ void cr_tmem_ld8(uint32_t taddr, uint32_t (&r)[8]) {
                : "r"(taddr));
 }
 
-// FINAL: output_layer.2 (8 -> 1): the same MMAs on a weight image whose channels 1..7 are zero (an M = 128 MMA costs the
+// R8_FINAL: output_layer.2 (8 -> 1): the same MMAs on a weight image whose channels 1..7 are zero (an M = 128 MMA costs the
 // same for any N <= 128), the epilogue keeps column 0: clip(-5, 5) (+ sigmoid), fp32, 128 contiguous bytes per warp.
-template <bool FINAL>
+// R8_SCORE: the same MMAs, clip and sigmoid, but the epilogue stores nothing: it reads the voxel's int8 label and
+// accumulates the eight masked sums of cvit_seg_stats (csrc/head_elementwise.cu) over the voxels whose label is > -1.
+//   - Exact counts: labels are integers, so sums 1 and 3..7 are integer counts. They are accumulated in integers (per
+//     thread), then reduced in fp64, which is exact below 2^53. The soft sums 0 and 2 accumulate per thread in fp32 over
+//     one work unit (64 voxels), then in fp64.
+//   - Deterministic: each CTA reduces its threads in a fixed order (shuffle tree, then warp by warp) and writes ONE fp64 row
+//     of 8 into args.partials; cvit_conv3d_rows8_score's one-block finalize kernel adds the rows in a fixed order. No
+//     atomics: two runs give bit-identical sums.
+enum Rows8Mode { R8_CONV = 0, R8_FINAL = 1, R8_SCORE = 2 };
+
+template <int MODE>
 __global__ void __launch_bounds__(CR_THREADS, 1) conv3d_rows8_kernel(const __grid_constant__ CUtensorMap tmX, const CrArgs args) {
+  constexpr bool FINAL = MODE != R8_CONV;  // one output channel (R8_FINAL, R8_SCORE)
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t sX = smem_base, sW = smem_base + CR_STAGES * CR_STAGE, sBar = sW + CR_IMG_BYTES;
@@ -225,6 +239,10 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv3d_rows8_kernel(const __gri
     }
     uint32_t nd = 0;  // planes drained per segment (phase of bar_done)
     float bsum[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};  // ACT_GELU_GRAD: column sums of what this thread stores
+    // R8_SCORE: soft sums 0, 2 (fp32 over the current unit, fp64 over all) and the counts 1, 3, 4, 5, 6, 7
+    float soft32[2] = {0.f, 0.f};
+    double soft64[2] = {0.0, 0.0};
+    int cnt[6] = {0, 0, 0, 0, 0, 0};
     for (int u = blockIdx.x; u < num_units; u += gridDim.x) {
       int xp, yt0, za, zb;
       unit_of(u, xp, yt0, za, zb);
@@ -235,6 +253,16 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv3d_rows8_kernel(const __gri
           const int x = xp + g * CR_SEG + q * 32 + lane;
           // ACT_GELU_GRAD: the z values of the plane about to be drained are requested before the wait for its MMAs
           uint4 zz[RH];
+          // R8_SCORE: so are the labels
+          int lab[RH];
+          if constexpr (MODE == R8_SCORE) {
+#pragma unroll
+            for (int r = 0; r < RH; ++r) {
+              const int y = yt0 + half * RH + r;
+              lab[r] = -1;
+              if (zo >= za && zo < zb && y < args.H && x < args.W) lab[r] = __ldg(args.labels + ((size_t)zo * args.H + y) * args.W + x);
+            }
+          }
           if (!FINAL && args.act == ACT_GELU_GRAD && zo >= za && zo < zb) {
 #pragma unroll
             for (int r = 0; r < RH; ++r) {
@@ -266,7 +294,22 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv3d_rows8_kernel(const __gri
             for (int r = 0; r < RH; ++r) {
               const int y = yt0 + half * RH + r;
               if (y < args.H && x < args.W) {
-                if (FINAL) {
+                if constexpr (MODE == R8_SCORE) {
+                  if (lab[r] > -1) {
+                    const float lg = fminf(fmaxf(__uint_as_float(v[r][0]) + bias[0], -5.0f), 5.0f);
+                    const float p = 1.0f / (1.0f + __expf(-lg));
+                    const int yl = lab[r], hge = p >= args.thr, hgt = p > 0.5f;
+                    soft32[0] += p;
+                    soft32[1] += p * (float)yl;
+                    cnt[0] += yl;
+                    cnt[1] += yl * hge;
+                    cnt[2] += hge;
+                    cnt[3] += yl * hgt;
+                    cnt[4] += (1 - yl) * hgt;
+                    cnt[5] += yl * (1 - hgt);
+                  }
+                  continue;
+                } else if (FINAL) {
                   const size_t vox = ((size_t)zo * args.H + y) * args.W + x;
                   const float lg = fminf(fmaxf(__uint_as_float(v[r][0]) + bias[0], -5.0f), 5.0f);
                   if (args.logits) args.logits[vox] = lg;
@@ -306,6 +349,27 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv3d_rows8_kernel(const __gri
           }
         }
       }
+      if constexpr (MODE == R8_SCORE) {
+        soft64[0] += soft32[0];
+        soft64[1] += soft32[1];
+        soft32[0] = soft32[1] = 0.f;
+      }
+    }
+    if constexpr (MODE == R8_SCORE) {  // this warp's eight sums -> shared memory (summed per CTA below, in warp order)
+      double t[8] = {soft64[0], (double)cnt[0], soft64[1], (double)cnt[1], (double)cnt[2], (double)cnt[3], (double)cnt[4],
+                     (double)cnt[5]};
+#pragma unroll
+      for (int k = 0; k < 8; ++k) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) t[k] += __shfl_xor_sync(0xffffffffu, t[k], o);
+      }
+      if (lane < 8) {
+        double mine = t[0];
+#pragma unroll
+        for (int k = 1; k < 8; ++k)
+          if (lane == k) mine = t[k];
+        reinterpret_cast<double*>(smem_gen + (sX - smem_base))[(warp - 2) * 8 + lane] = mine;  // stages idle: every MMA retired
+      }
     }
     if (!FINAL && args.act == ACT_GELU_GRAD && args.db) {  // bias gradient: one shuffle tree and 8 atomics per warp
 #pragma unroll
@@ -318,10 +382,33 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv3d_rows8_kernel(const __gri
 
   tcgen05_fence_before();
   __syncthreads();
+  if constexpr (MODE == R8_SCORE) {
+    if (threadIdx.x < 8) {
+      const double* red = reinterpret_cast<const double*>(smem_gen + (sX - smem_base));
+      double s = 0.0;
+      for (int w = 0; w < 8; ++w) s += red[w * 8 + threadIdx.x];
+      args.partials[(size_t)blockIdx.x * 8 + threadIdx.x] = s;
+    }
+  }
   if (warp == 1) {
     __syncwarp();
     tcgen05_fence_after();
     tmem_dealloc<512>(tmem_base);
+  }
+}
+
+// R8_SCORE's second step: out8[k] = the sum of partials[r][k] over the rows r = 0 .. rows - 1, in a fixed order.
+__global__ void __launch_bounds__(256) rows8_score_finalize_kernel(const double* __restrict__ partials, int rows, double* __restrict__ out8) {
+  __shared__ double red[32][8];
+  const int k = threadIdx.x & 7, j = threadIdx.x >> 3;
+  double s = 0.0;
+  for (int r = j; r < rows; r += 32) s += partials[(size_t)r * 8 + k];
+  red[j][k] = s;
+  __syncthreads();
+  if (threadIdx.x < 8) {
+    double t = 0.0;
+    for (int i = 0; i < 32; ++i) t += red[i][threadIdx.x];
+    out8[threadIdx.x] = t;
   }
 }
 
@@ -334,7 +421,11 @@ extern "C" int64_t cvit_conv3d_rows8_weight_bytes() { return CR_IMG_BYTES; }
 // out (bf16 [D,H,W,8]) = conv3d(x bf16 [D,H,W,8], 3x3x3, "same", dilation 1) + bias, act: 0 none, 1 GELU, 2 out = pre-activation
 // and aux = GELU of it, 3 out = result * gelu'(aux) with db (fp32 [8], may be null) += the column sums of what is stored (ptx.cuh ACT_*). w_img: cvit_conv3d_rows8_weight_bytes() bytes in the layout of
 // cryovit_b200.head.rows8_weight_image. W must be a multiple of 8.
-static int rows8_launch(const void* x, CrArgs a, bool final, cudaStream_t stream) {
+static int64_t rows8_units(int64_t D, int64_t H, int64_t W) {
+  return ((W + 2 * CR_SEG - 1) / (2 * CR_SEG)) * ((H + CR_HT - 1) / CR_HT) * ((D + CR_ZC - 1) / CR_ZC);
+}
+
+static int rows8_launch(const void* x, CrArgs a, int mode, cudaStream_t stream, double* out8 = nullptr) {
   CUtensorMap tmX;
   uint64_t dims[4] = {64, (uint64_t)(a.W / 8), (uint64_t)a.H, (uint64_t)a.D};
   uint64_t strides[4] = {0, 128, (uint64_t)a.W * 16, (uint64_t)a.H * a.W * 16};
@@ -343,19 +434,26 @@ static int rows8_launch(const void* x, CrArgs a, bool final, cudaStream_t stream
   if (rc) return rc;
   static bool configured = false;
   if (!configured) {
-    cudaError_t e = cudaFuncSetAttribute(conv3d_rows8_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, CR_SMEM);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3d_rows8_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, CR_SMEM);
+    cudaError_t e = cudaFuncSetAttribute(conv3d_rows8_kernel<R8_CONV>, cudaFuncAttributeMaxDynamicSharedMemorySize, CR_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3d_rows8_kernel<R8_FINAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, CR_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3d_rows8_kernel<R8_SCORE>, cudaFuncAttributeMaxDynamicSharedMemorySize, CR_SMEM);
     if (e != cudaSuccess) {
       set_error("conv3d_rows8: cudaFuncSetAttribute(smem=%d): %s", CR_SMEM, cudaGetErrorString(e));
       return CVIT_ERR_CUDA;
     }
     configured = true;
   }
-  const int64_t units = (int64_t)((a.W + 2 * CR_SEG - 1) / (2 * CR_SEG)) * ((a.H + CR_HT - 1) / CR_HT) * ((a.D + CR_ZC - 1) / CR_ZC);
+  const int64_t units = rows8_units(a.D, a.H, a.W);
   int grid = num_sms();
   if (grid > units) grid = (int)units;
-  if (final) conv3d_rows8_kernel<true><<<grid, CR_THREADS, CR_SMEM, stream>>>(tmX, a);
-  else conv3d_rows8_kernel<false><<<grid, CR_THREADS, CR_SMEM, stream>>>(tmX, a);
+  if (mode == R8_SCORE) {
+    conv3d_rows8_kernel<R8_SCORE><<<grid, CR_THREADS, CR_SMEM, stream>>>(tmX, a);
+    if (int rc2 = check_launch("conv3d_rows8_kernel<score>")) return rc2;
+    rows8_score_finalize_kernel<<<1, 256, 0, stream>>>(a.partials, grid, out8);
+    return check_launch("rows8_score_finalize_kernel");
+  }
+  if (mode == R8_FINAL) conv3d_rows8_kernel<R8_FINAL><<<grid, CR_THREADS, CR_SMEM, stream>>>(tmX, a);
+  else conv3d_rows8_kernel<R8_CONV><<<grid, CR_THREADS, CR_SMEM, stream>>>(tmX, a);
   return check_launch("conv3d_rows8_kernel");
 }
 
@@ -394,7 +492,10 @@ extern "C" int cvit_conv3d_rows8(const void* x, const void* w_img, const float* 
   a.H = (int)H;
   a.W = (int)W;
   a.act = act;
-  return rows8_launch(x, a, false, (cudaStream_t)stream);
+  a.labels = nullptr;
+  a.partials = nullptr;
+  a.thr = 0.f;
+  return rows8_launch(x, a, R8_CONV, (cudaStream_t)stream);
 }
 
 // output_layer.2 (8 -> 1) + bias + clip(-5, 5) -> logits fp32 [D,H,W] and/or sigmoid of them -> probs; w_img: the rows8 image of
@@ -418,5 +519,43 @@ extern "C" int cvit_conv3d_rows8_final(const void* x, const void* w_img, const f
   a.H = (int)H;
   a.W = (int)W;
   a.act = 0;
-  return rows8_launch(x, a, true, (cudaStream_t)stream);
+  a.labels = nullptr;
+  a.partials = nullptr;
+  a.thr = 0.f;
+  return rows8_launch(x, a, R8_FINAL, (cudaStream_t)stream);
+}
+
+// Doubles of the partials buffer cvit_conv3d_rows8_score needs for a [D, H, W] volume (one row of 8 per work unit: at least
+// one per CTA of any grid); depends on the shape only.
+extern "C" int64_t cvit_conv3d_rows8_score_partials(int64_t D, int64_t H, int64_t W) {
+  if (D <= 0 || H <= 0 || W <= 0) return 0;
+  return 8 * rows8_units(D, H, W);
+}
+
+// output_layer.2 (8 -> 1) + bias + clip(-5, 5) + sigmoid as cvit_conv3d_rows8_final, scored instead of stored: out8 (fp64 [8],
+// overwritten) = the eight masked sums of cvit_seg_stats of (probabilities, labels) with labels int8 [D,H,W] (-1 = ignore).
+// partials: cvit_conv3d_rows8_score_partials(D, H, W) doubles of scratch. Counts (1, 3..7) exact; bit-identical across runs.
+extern "C" int cvit_conv3d_rows8_score(const void* x, const void* w_img, const float* bias, const int8_t* labels, int64_t D,
+                                       int64_t H, int64_t W, float threshold, double* partials, double* out8, void* stream) {
+  if (int rc = rows8_check(x, w_img, bias, D, H, W)) return rc;
+  if (!labels || !partials || !out8) {
+    set_error("conv3d_rows8_score: need labels, partials and out8");
+    return CVIT_ERR_INVALID;
+  }
+  CrArgs a;
+  a.w_img = static_cast<const __nv_bfloat16*>(w_img);
+  a.bias = bias;
+  a.out = nullptr;
+  a.aux = nullptr;
+  a.db = nullptr;
+  a.logits = nullptr;
+  a.probs = nullptr;
+  a.D = (int)D;
+  a.H = (int)H;
+  a.W = (int)W;
+  a.act = 0;
+  a.labels = labels;
+  a.partials = partials;
+  a.thr = threshold;
+  return rows8_launch(x, a, R8_SCORE, (cudaStream_t)stream, out8);
 }

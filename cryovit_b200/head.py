@@ -18,6 +18,7 @@ import torch
 
 from . import ops
 from ._lib import CryovitB200Error
+from .operand_gather import OperandGather
 
 BLOCKS = [(1024, 192, 128, 32, 24), (128, 64, 32, 16, 12), (32, 32, 32, 8, 4), (32, 16, 8, 2, 1)]
 
@@ -152,6 +153,7 @@ class CryoVITHeadB200:
         self._sd_cpu: dict | None = None
         self._w: dict = {}
         self._bufs: dict = {}
+        self._bucket = None  # attach_bucket: (OperandGather, index-valued operand tree, id -> operand name, projection range)
         self.launches = 0
 
     # ----------------------------------------------------------------------------- nn.Module-like surface
@@ -181,14 +183,30 @@ class CryoVITHeadB200:
     def eval(self):
         return self
 
-    def _pack(self) -> None:
-        sd, dev = self._sd_cpu, self.device
-        bf = lambda t: t.to(dev).to(torch.bfloat16).contiguous()
-        f32 = lambda t: t.to(dev).float().contiguous()
+    def _pack(self, sd: dict | None = None, gather: OperandGather | None = None) -> tuple[dict, dict]:
+        """Every operand of the forward pass from the (CPU, fp32) state dict ``sd`` (default: the loaded one). With
+        ``gather``, ``sd`` holds index-valued stand-ins of the parameters (``OperandGather.indices``): each operand is
+        registered there as a gather table, and the returned tree holds the index-valued operands (``attach_bucket``).
+        Returns (operand tree, id of each gathered operand -> its name in ``gather``)."""
+        dev = self.device
+        ids = {}
+
+        def cast(t, dtype):
+            if gather is None:
+                return t.to(dev).to(dtype).contiguous()
+            t = t.to(dev).float().contiguous().clone()
+            ids[id(t)] = name = str(len(ids))
+            gather.add(name, t, dtype)
+            return t
+
+        if sd is None:
+            sd = self._sd_cpu
+        bf = lambda t: cast(t, torch.bfloat16)
+        f32 = lambda t: cast(t, torch.float32)
         w = {"proj_w": bf(sd["layers.0.weight"].reshape(1024, self.in_channels)), "proj_b": f32(sd["layers.0.bias"])}
         pw = sd["layers.0.weight"].reshape(1024, self.in_channels).float()
-        if float(pw.abs().max()) < 6.0e4:  # fp16 image of the projection for the transposed-A kernel (fp16 features)
-            w["proj_w16"] = pw.to(self.device).to(torch.float16).contiguous()
+        if gather is not None or float(pw.abs().max()) < 6.0e4:  # fp16 image of the projection for the transposed-A kernel
+            w["proj_w16"] = cast(pw, torch.float16)                # (fp16 features); with gather, checked per refresh
         blocks = []
         for bi, (c1, c2, c3, d1, d2) in enumerate(BLOCKS):
             p = f"layers.{bi + 2}.layers."
@@ -200,7 +218,7 @@ class CryoVITHeadB200:
             for tag, key, cin in (("a", "1", c1), ("b", "3", c2)):
                 if ops.rows_supported(cin, c2):  # one voxel per tensor-core row (csrc/conv_rows.cu): the 16 / 32-channel layers
                     img32 = f32(rowsn_weight_image(sd[p + key + ".weight"]))
-                    rws[tag] = {"w32": img32, "w": img32.to(torch.bfloat16), "bias": f32(sd[p + key + ".bias"]),
+                    rws[tag] = {"w32": img32, "w": bf(img32), "bias": f32(sd[p + key + ".bias"]),
                                 "table": f32(sd[p + key + ".bias"].repeat(64)), "fold": torch.empty_like(img32, dtype=torch.bfloat16),
                                 "gn_table": torch.empty(64 * c2, device=dev, dtype=torch.float32)}
                 if cin in (8, 16, 32):  # narrow layer: shared-memory halo kernel (csrc/conv_halo.cu)
@@ -211,14 +229,14 @@ class CryoVITHeadB200:
                     P = ops.wpackn_group(cin, cp)
                     if P:  # ... or, on planes whose width is a multiple of P, P voxels per tensor-core row (csrc/conv_wpackn.cu)
                         img32 = f32(wpackn_weight_image(sd[p + key + ".weight"], cp, P))
-                        wpn[tag] = {"P": P, "cp": cp, "w32": img32, "w": img32.to(torch.bfloat16),
+                        wpn[tag] = {"P": P, "cp": cp, "w32": img32, "w": bf(img32),
                                     "table": f32(hb.repeat(64)), "fold": torch.empty_like(img32, dtype=torch.bfloat16)}
             # fp32 originals in the operand layout of the convolution that follows the GroupNorm (folded per volume)
             if "a" in halo:
                 a32, a_layout, a_cp = f32(halo_weight_image(sd[p + "1.weight"], halo["a"][2])), ops.LAYOUT_HALO, halo["a"][2]
                 a_bias = halo["a"][1]
             else:
-                a32, a_layout, a_cp, a_bias = f32(_conv_taps(sd[p + "1.weight"], c2p)).reshape(-1), ops.LAYOUT_TAPS, c2p, f32(ba)
+                a32, a_layout, a_cp, a_bias = f32(_conv_taps(sd[p + "1.weight"], c2p).reshape(-1)), ops.LAYOUT_TAPS, c2p, f32(ba)
             blocks.append({
                 "wpn": wpn, "rows": rws,
                 "halo": halo, "a_w32": a32, "a_layout": a_layout, "a_cp": a_cp, "a_bias": a_bias,
@@ -243,7 +261,51 @@ class CryoVITHeadB200:
         # one voxel per MMA row, partial sums meeting in tensor memory (csrc/conv_rows8.cu; widths that are a multiple of 8)
         w["o1_r8"], w["o1_r8_b"] = bf(rows8_weight_image(sd["output_layer.0.weight"])), f32(sd["output_layer.0.bias"])
         w["o2_r8"], w["o2_r8_b"] = bf(rows8_weight_image(sd["output_layer.2.weight"])), f32(sd["output_layer.2.bias"])
+        if gather is None:
+            self._w = w
+        return w, ids
+
+    # ----------------------------------------------------------------------------- weights that follow a trainer
+    def attach_bucket(self, store: torch.Tensor, offsets: dict[str, int], shapes: dict[str, tuple]) -> "CryoVITHeadB200":
+        """Take the weights from a flat fp32 parameter bucket (``CryoVITHeadTrainerB200.parameter_bucket()``: the
+        parameters at ``offsets`` with ``shapes``, a zero at the end) instead of a state dict. ``_pack`` runs ONCE, on
+        the parameters' global indices, and leaves a gather table per operand; every :meth:`refresh` then rebuilds all
+        operands from the bucket's current values with one ``index_select`` per dtype, no host round trip."""
+        if self.device is None:
+            raise CryovitB200Error("attach_bucket: call .cuda() first")
+        if shapes["layers.0.weight"][1] != self.in_channels:
+            raise CryovitB200Error(f"bucket's layers.0.weight expects {shapes['layers.0.weight'][1]} input channels, "
+                                   f"head was built for {self.in_channels}")
+        gather = OperandGather(store)
+        sd = {k: gather.indices(offsets[k], shapes[k], device="cpu") for k in state_dict_keys()}
+        tree, ids = self._pack(sd, gather)
+        o = offsets["layers.0.weight"]
+        self._bucket = (gather, tree, ids, (o, o + 1024 * self.in_channels))
+        self._sd_cpu = None  # the weights now live in the bucket
+        return self.refresh()
+
+    def refresh(self) -> "CryoVITHeadB200":
+        """Operands from the attached bucket's current values. The fp16 projection (fp16 features) exists while the
+        projection weight fits in fp16, as with ``load_state_dict``: one host read per refresh."""
+        if self._bucket is None:
+            raise CryovitB200Error("refresh: no bucket attached (attach_bucket)")
+        gather, tree, ids, (p0, p1) = self._bucket
+        views = gather.refresh()
+
+        def sub(x):
+            if isinstance(x, dict):
+                return {k: sub(v) for k, v in x.items()}
+            if isinstance(x, (list, tuple)):
+                return type(x)(sub(v) for v in x)
+            if isinstance(x, torch.Tensor) and id(x) in ids:
+                return views[ids[id(x)]]
+            return x
+
+        w = sub(tree)
+        if not float(gather.store[p0:p1].abs().max()) < 6.0e4:
+            del w["proj_w16"]
         self._w = w
+        return self
 
     def _buf(self, name: str, numel: int, dtype=torch.bfloat16) -> torch.Tensor:
         b = self._bufs.get(name)
@@ -253,9 +315,9 @@ class CryoVITHeadB200:
         return b[:numel]
 
     # ----------------------------------------------------------------------------- forward
-    @torch.inference_mode()
-    def segment_volume(self, features: torch.Tensor, want_probs: bool = True, want_logits: bool = True):
-        """features: CUDA (C, D, h, w) fp16 or fp32 -> (logits, probs), each fp32 [D, 16h, 16w] (or None)."""
+    def _trunk(self, features: torch.Tensor):
+        """Every layer before output_layer: features (C, D, h, w) -> (bf16 [D, 16h, 16w, 8] in one of the ping-pong
+        buffers, the name of the other one)."""
         if self.device is None or not self._w:
             raise CryovitB200Error("head not ready: call load_state_dict(...) and .cuda() first")
         if features.dim() != 4 or features.shape[0] != self.in_channels:
@@ -353,7 +415,15 @@ class CryoVITHeadB200:
             H, W = 2 * H, 2 * W
             self.launches += 5 if fuse else 6  # fused: finalize + fold + 3 layers; else memset + 2 GroupNorm kernels + 3 layers
             self.launches += sum(c2 // 16 - 1 for r_ in (ra, rb) if r_ is not None)  # conv3d_rows: one kernel per 16 output channels
-        scratch = self._buf(names[flip], D * H * W * 8).view(D, H, W, 8)
+        return cur, names[flip]
+
+    @torch.inference_mode()
+    def segment_volume(self, features: torch.Tensor, want_probs: bool = True, want_logits: bool = True):
+        """features: CUDA (C, D, h, w) fp16 or fp32 -> (logits, probs), each fp32 [D, 16h, 16w] (or None)."""
+        cur, free = self._trunk(features)
+        D, H, W, _ = cur.shape
+        w_ = self._w
+        scratch = self._buf(free, D * H * W * 8).view(D, H, W, 8)
         logits = torch.empty(D, H, W, device=self.device) if want_logits else None
         probs = torch.empty(D, H, W, device=self.device) if want_probs else None
         if W % 8 == 0 and self.rows8:  # always true downstream of the ViT (W = 16 w): one voxel per MMA row (conv_rows8.cu)
@@ -367,6 +437,31 @@ class CryoVITHeadB200:
             ops.head_out_conv(scratch, w_["o2_w"], w_["o2_b"], logits, probs)
         self.launches += 2
         return logits, probs
+
+    @torch.inference_mode()
+    def score_volume(self, features: torch.Tensor, labels: torch.Tensor, threshold: float = 0.5) -> torch.Tensor:
+        """features: CUDA (C, D, h, w) fp16 or fp32, labels [D, 16h, 16w] (-1 = ignore) -> the eight masked sums of
+        ``SegStats(probs, labels, threshold)`` over segment_volume's probabilities, fp64 [8] on the device.
+
+        int8 labels (the caller guarantees values in {-1, 0, 1}) on planes whose width is a multiple of 8: output_layer.2
+        scores inside its epilogue (``ops.conv3d_rows8_score``) and no probability volume is written. Other labels, or
+        ``CVIT_HEAD_ROWS8=0``: segment_volume + seg_stats."""
+        D, W = features.shape[1], 16 * features.shape[3]
+        if labels.dtype != torch.int8 or W % 8 or not self.rows8:
+            _, probs = self.segment_volume(features, want_logits=False)
+            return ops.seg_stats(probs.reshape(-1), labels.to(self.device).reshape(-1).float().contiguous(), threshold)
+        cur, free = self._trunk(features)
+        D, H, W, _ = cur.shape
+        w_ = self._w
+        if tuple(labels.shape) != (D, H, W):
+            raise CryovitB200Error(f"labels {tuple(labels.shape)} do not match the output volume {(D, H, W)}")
+        scratch = self._buf(free, D * H * W * 8).view(D, H, W, 8)
+        partials = self._buf("score_partials", ops.rows8_score_partials(D, H, W), torch.float64)
+        out8 = torch.empty(8, device=self.device, dtype=torch.float64)
+        ops.conv3d_rows8(cur, w_["o1_r8"], w_["o1_r8_b"], scratch)                                        # output_layer.0 + GELU
+        ops.conv3d_rows8_score(scratch, w_["o2_r8"], w_["o2_r8_b"], labels.contiguous(), partials, out8, threshold)
+        self.launches += 3  # + the finalize kernel
+        return out8
 
     @torch.inference_mode()
     def forward_volume(self, x: torch.Tensor) -> torch.Tensor:

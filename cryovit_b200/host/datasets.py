@@ -212,10 +212,15 @@ class ResidentTomoCache:
     19 ms step. A B200 holds 180 GB: ~400 tomograms of BASELINE's size fit next to the trainer. ``get(i)`` is
     ``dataset[i]`` with the tensors already on the device: same record order, same crop draws (the crop is drawn from
     the shape and applied as a view of the resident volume). Items past ``budget_bytes`` are not kept and come from
-    their file every time, as before."""
+    their file every time, as before.
 
-    def __init__(self, dataset: "TomoDataset", device, budget_bytes: int):
+    ``int8_labels`` (validation): a label volume whose values are all in {-1, 0, 1} is kept as int8, the operand of
+    ``CryoVITHeadB200.score_volume``'s fused path (a quarter of fp32's HBM); the values are checked once per file read,
+    and other labels stay as they are."""
+
+    def __init__(self, dataset: "TomoDataset", device, budget_bytes: int, int8_labels: bool = False):
         self.dataset, self.device, self.budget = dataset, torch.device(device), int(budget_bytes)
+        self.int8_labels = int8_labels
         self.used = 0
         self.file_reads = 0
         self._items: dict[int, tuple[torch.Tensor, torch.Tensor, dict]] = {}
@@ -225,7 +230,10 @@ class ResidentTomoCache:
         rec = ds._row(idx)
         data = ds._load_tomogram(rec)
         self.file_reads += 1
-        inp, lab = torch.as_tensor(np.ascontiguousarray(data["input"])), torch.as_tensor(np.ascontiguousarray(data["label"]))
+        label = data["label"]
+        if self.int8_labels and label.dtype != np.int8 and np.isin(label, (-1, 0, 1)).all():
+            label = label.astype(np.int8)
+        inp, lab = torch.as_tensor(np.ascontiguousarray(data["input"])), torch.as_tensor(np.ascontiguousarray(label))
         meta = {"sample": rec["sample"], "tomo_name": rec["tomo_name"], "split_id": data.get("split_id"),
                 "aux": {k: data[k] for k in ds.aux_keys if k in data}}
         return inp, lab, meta

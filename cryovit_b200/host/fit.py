@@ -33,9 +33,20 @@ def _cache_budget_bytes(cache_gb: float | None) -> int:
     return int(0.6 * free)
 
 
+def _append_row(path: Path, row: dict, first: bool) -> None:
+    """One csv row (a header first), flushed to the file before the next epoch starts."""
+    path.parent.mkdir(parents=True, exist_ok=True)
+    with open(path, "w" if first else "a") as f:
+        if first:
+            f.write(",".join(row) + "\n")
+        f.write(",".join(str(v) for v in row.values()) + "\n")
+        f.flush()
+
+
 def fit_head(dataset: TomoDataset, in_channels: int = 1536, max_epochs: int = 50, lr: float = 1e-4, weight_decay: float = 1e-3,
              swa_epoch_start: int | None = 40, seed: int = 42, exp_dir: Path | str | None = None, state_dict: dict | None = None,
-             log_every: int = 10, cache_gb: float | None = None, epoch_seconds: list | None = None) -> dict[str, torch.Tensor]:
+             log_every: int = 10, cache_gb: float | None = None, epoch_seconds: list | None = None, validator=None,
+             val_history: list | None = None) -> dict[str, torch.Tensor]:
     """Trains on the items of ``dataset`` (``train=True`` gives the reference's random 128 x 32 x 32 feature crops);
     with several ranks (torchrun) every rank walks its own round-robin share of a common shuffled order and the
     gradients are averaged over the ranks each step. Returns the final (SWA-averaged if enabled) state dict.
@@ -43,7 +54,12 @@ def fit_head(dataset: TomoDataset, in_channels: int = 1536, max_epochs: int = 50
     The tomograms this rank trains on stay resident in HBM after their first read (:class:`ResidentTomoCache`, up to
     ``cache_gb``), and the next item's file read (first epoch) and crop draw happen on a helper thread under the current
     step; crops and order are those of the plain ``dataset[i]`` loop. ``epoch_seconds`` (a list) receives the wall clock of
-    every epoch, device work included."""
+    every epoch's training, device work included.
+
+    ``validator`` (a :class:`~cryovit_b200.host.validate.Validator`): after the training steps of every epoch it schedules,
+    the validation tomograms are scored with the current (not SWA-averaged) weights, as Lightning's ``fit`` does. Its
+    resident tomograms share the HBM budget, after the training set's. Rank 0 appends a row per validated epoch to
+    ``<exp_dir>/validation.csv``; ``val_history`` (a list) receives the same rows as dicts."""
     rank, world = rank_world()
     require_process_group("fit_head")  # the data is sharded by rank below: the gradients must really be exchanged
     torch.manual_seed(seed)
@@ -55,14 +71,16 @@ def fit_head(dataset: TomoDataset, in_channels: int = 1536, max_epochs: int = 50
     swa_avg, swa_n = None, 0
     step = 0
     cache = None
-    if hasattr(dataset, "_crop_slices") and hasattr(dataset, "_load_tomogram"):
-        budget = _cache_budget_bytes(cache_gb)
+    cacheable = hasattr(dataset, "_crop_slices") and hasattr(dataset, "_load_tomogram")
+    budget = _cache_budget_bytes(cache_gb) if cacheable or validator is not None else 0
+    if cacheable:
         if budget > 0:
             cache = ResidentTomoCache(dataset, trainer.device, budget)  # where the trainer lives
     # the helper thread does host work only (file read, crop draw): the trainer captures CUDA graphs on this thread, and a
     # CUDA call from another thread during a capture is an error. ONE helper thread: the crop draws stay in order.
     fetch = (lambda i: cache.prepare(int(i))) if cache is not None else (lambda i: dataset[int(i)])
     pool = ThreadPoolExecutor(max_workers=1, thread_name_prefix="cryovit-fit-fetch")
+    val_rows = 0
     try:
         for epoch in range(max_epochs):
             # Lightning's StochasticWeightAveraging.on_train_epoch_START: epochs swa_start .. max_epochs - 1 each add the
@@ -93,6 +111,13 @@ def fit_head(dataset: TomoDataset, in_channels: int = 1536, max_epochs: int = 50
             if rank == 0:
                 logging.info("epoch %d: %d steps/rank, DiceLoss %.4f, %.2f s", epoch, usable // world,
                              float(np.mean(losses)) if losses else float("nan"), time.perf_counter() - t_epoch)
+            if validator is not None and validator.scheduled(epoch):
+                row = validator.run(trainer, epoch, cache_budget=budget - (cache.used if cache is not None else 0))
+                if val_history is not None:
+                    val_history.append(row)
+                if exp_dir is not None and rank == 0:
+                    _append_row(Path(exp_dir) / "validation.csv", row, first=val_rows == 0)
+                val_rows += 1
     finally:
         pool.shutdown(wait=True)
     if cache is not None and rank == 0:

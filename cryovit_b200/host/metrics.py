@@ -17,6 +17,13 @@ class SegStats:
         y = labels.reshape(-1).float().contiguous()
         self.v = ops.seg_stats(p, y, threshold)  # fp64 [8] on the device
 
+    @classmethod
+    def from_sums(cls, v: torch.Tensor) -> "SegStats":
+        """The same object over sums computed elsewhere (``CryoVITHeadB200.score_volume``): fp64 [8] in the order above."""
+        st = cls.__new__(cls)
+        st.v = v
+        return st
+
     def dice_loss(self) -> torch.Tensor:
         """losses.py:17-32: 1 - 2*sum(y*p) / (sum(y) + sum(p) + 1e-3)."""
         v = self.v
@@ -25,7 +32,10 @@ class SegStats:
 
 class DiceLoss:
     def __call__(self, probs: torch.Tensor, labels: torch.Tensor) -> torch.Tensor:
-        return SegStats(probs, labels).dice_loss()
+        return self.from_stats(SegStats(probs, labels))
+
+    def from_stats(self, stats: SegStats) -> torch.Tensor:
+        return stats.dice_loss()
 
 
 class _MeanOfBatchesMetric:
@@ -47,12 +57,13 @@ class _MeanOfBatchesMetric:
             return torch.tensor(0.0)
         return self.score / self.total
 
-    def all_reduce(self) -> None:
-        """Data-parallel evaluation: sum both states over ranks (torchmetrics' dist_reduce_fx="sum")."""
+    def all_reduce(self, device=None) -> None:
+        """Data-parallel evaluation: sum both states over ranks (torchmetrics' dist_reduce_fx="sum"). ``device``: where a
+        rank that saw no batch puts its zeros (NCCL needs the GPU; default CPU)."""
         import torch.distributed as dist
 
         if dist.is_available() and dist.is_initialized():
-            dev = self.score.device if self.score is not None else "cpu"
+            dev = self.score.device if self.score is not None else (device or "cpu")
             st = torch.stack([(self.score if self.score is not None else torch.zeros((), dtype=torch.float64, device=dev)),
                               torch.tensor(self.total, dtype=torch.float64, device=dev)])
             dist.all_reduce(st, op=dist.ReduceOp.SUM)
@@ -67,7 +78,11 @@ class DiceMetric(_MeanOfBatchesMetric):
         self.threshold = threshold
 
     def update(self, probs, labels) -> None:
-        v = SegStats(probs, labels, self.threshold).v
+        self.update_stats(SegStats(probs, labels, self.threshold))
+
+    def update_stats(self, stats: SegStats) -> None:
+        """``stats``: sums taken with this metric's threshold."""
+        v = stats.v
         self._add(2.0 * v[3] / (v[1] + v[4] + 1e-3))
 
 
@@ -75,7 +90,10 @@ class F1Metric(_MeanOfBatchesMetric):
     """metrics.py:56-93: tp / fp / fn with the strict decision p > 0.5; eps 1e-6 in precision, recall and F1."""
 
     def update(self, probs, labels) -> None:
-        v = SegStats(probs, labels).v
+        self.update_stats(SegStats(probs, labels))
+
+    def update_stats(self, stats: SegStats) -> None:
+        v = stats.v
         tp, fp, fn = v[5], v[6], v[7]
         precision = tp / (tp + fp + 1e-6)
         recall = tp / (tp + fn + 1e-6)

@@ -14,6 +14,7 @@ from .._lib import CryovitB200Error
 from .config import instantiate
 from .fit import fit_head
 from .shard import process_group
+from .validate import Validator
 
 
 def _joined(x):
@@ -42,6 +43,25 @@ def build_datamodule(cfg):
     dataset_fn = instantiate(cfg.datamodule.dataset)
     split_file = Path(cfg.paths.data_dir) / cfg.paths.csv_name / cfg.paths.split_name
     return instantiate(node, split_file=split_file, dataset_fn=dataset_fn, dataloader_fn=None)
+
+
+def build_validator(cfg, datamodule, in_channels: int) -> Validator | None:
+    """Lightning's ``fit`` validates after every epoch by default: the datamodule's ``val_df()`` scored whole
+    (``train=False``) with ``cfg.model``'s losses and metrics, on the schedule of ``trainer.check_val_every_n_epoch``
+    and ``trainer.limit_val_batches``. None when that schedule validates nothing or the validation split is empty."""
+    tr = cfg.trainer
+    records = datamodule.val_df()
+    if records.empty:
+        logging.info("No validation data in the split file: training without validation.")
+        return None
+    losses = {k: instantiate(v) for k, v in (cfg.model.get("losses") or {}).items()}
+    metrics = {k: instantiate(v) for k, v in (cfg.model.get("metrics") or {}).items()}
+    v = Validator(datamodule.dataset_fn(records, train=False), in_channels, losses, metrics,
+                  tr.get("check_val_every_n_epoch", 1), tr.get("limit_val_batches", 1.0))
+    if v.count == 0:
+        logging.info("trainer.limit_val_batches=%s: training without validation.", tr.get("limit_val_batches"))
+        return None
+    return v
 
 
 def run_trainer(cfg) -> Path:
@@ -79,9 +99,11 @@ def _run_trainer(cfg) -> Path:
             state = torch.load(ckpt)
         else:
             raise ValueError(f"Unsupported checkpoint format: {Path(ckpt).suffix}. Use .pt or .model files.")
+    in_channels = int(cfg.model.get("in_channels", 1536))
+    validator = build_validator(cfg, datamodule, in_channels)
     logging.info("Starting training.")
-    fit_head(dataset, in_channels=int(cfg.model.get("in_channels", 1536)), max_epochs=max_epochs, lr=float(cfg.model.lr),
+    fit_head(dataset, in_channels=in_channels, max_epochs=max_epochs, lr=float(cfg.model.lr),
              weight_decay=float(cfg.model.get("weight_decay", 1e-3)), swa_epoch_start=swa_start, seed=int(cfg.random_seed),
-             exp_dir=cfg.paths.exp_dir, state_dict=state)
+             exp_dir=cfg.paths.exp_dir, state_dict=state, validator=validator)
     logging.info("Saving model.")
     return cfg.paths.exp_dir / "weights.pt"

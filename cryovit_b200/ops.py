@@ -344,6 +344,27 @@ def conv3d_rows8_final(x, w_img, bias1, logits=None, probs=None) -> None:
               D, H, W, _stream())
 
 
+def conv3d_rows8_score(x, w_img, bias1, labels, partials, out8, threshold: float = 0.5) -> torch.Tensor:
+    """output_layer.2 (8 -> 1, k3) + bias + clip(-5, 5) + sigmoid as ``conv3d_rows8_final``, scored instead of stored: ``out8``
+    (fp64 [8], overwritten) = the eight masked sums of ``seg_stats`` against int8 ``labels`` [D, H, W] (-1 = ignore).
+    ``partials``: fp64 scratch of at least ``rows8_score_partials(D, H, W)`` numbers. W % 8 == 0."""
+    D, H, W, Cin = x.shape
+    if Cin != 8 or w_img.numel() * 2 != _lib.load().cvit_conv3d_rows8_weight_bytes():
+        raise _lib.CryovitB200Error("conv3d_rows8_score: needs 8 input channels and the rows8 weight image")
+    if tuple(labels.shape) != (D, H, W) or out8.numel() != 8 or partials.numel() < rows8_score_partials(D, H, W):
+        raise _lib.CryovitB200Error(f"conv3d_rows8_score: labels {tuple(labels.shape)} must be {(D, H, W)}, out8 fp64 [8], "
+                                    f"partials >= {rows8_score_partials(D, H, W)} doubles")
+    _lib.call("cvit_conv3d_rows8_score", _chk(x, BF16, "x"), _chk(w_img, BF16, "w_img"), _chk(bias1, F32, "bias1"),
+              _chk(labels, torch.int8, "labels"), D, H, W, float(threshold), _chk(partials, torch.float64, "partials"),
+              _chk(out8, torch.float64, "out8"), _stream())
+    return out8
+
+
+def rows8_score_partials(D: int, H: int, W: int) -> int:
+    """fp64 scratch numbers ``conv3d_rows8_score`` needs for a [D, H, W] volume."""
+    return int(_lib.load().cvit_conv3d_rows8_score_partials(D, H, W))
+
+
 def conv3d_wpack8_final(x, w_img, bias_n, logits=None, probs=None) -> None:
     """output_layer.2 (8 -> 1, k3) + bias + clip(-5, 5) (+ sigmoid) with 16 output voxels of a row per MMA row."""
     D, H, W, Cin = x.shape

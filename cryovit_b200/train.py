@@ -23,6 +23,7 @@ import torch
 from . import nvtx, ops
 from . import train_ops as T
 from ._lib import CryovitB200Error
+from .operand_gather import OperandGather
 from .head import BLOCKS, rows8_weight_image, rowsn_weight_image, state_dict_keys, wpack_weight_image, wpackn_weight_image
 
 BF16, F32 = torch.bfloat16, torch.float32
@@ -200,10 +201,7 @@ class CryoVITHeadTrainerB200:
         self.flat_g = torch.zeros(n, device=self.device, dtype=F32)  # gradients, all-reduced as one flat bucket
         self.flat_m = torch.zeros(n, device=self.device, dtype=F32)
         self.flat_v = torch.zeros(n, device=self.device, dtype=F32)
-        self.p, self.g, self._offsets, self._nparams = {}, {}, {}, n
-        self._pk_tables: dict = {}  # operand name -> (gather table into _flat_store, shape)
-        self._pk_views: dict = {}   # operand name -> this step's bf16 operand
-        self._pk_cat = None
+        self.p, self.g, self._offsets = {}, {}, {}
         off = 0
         for k, sz in zip(self.keys, sizes):
             shape = state_dict[k].shape
@@ -215,6 +213,7 @@ class CryoVITHeadTrainerB200:
         self.step_count = 0
         self.launches = 0
         self._retired: list = []  # superseded scratch buffers, kept alive for the graphs captured over them
+        self._gather = OperandGather(self._flat_store, self._retired)  # bf16 operand images of the weights (_pk)
         self._bufs: dict = _KeepAlivePool(self._retired)
         self._bufs["wgrad_pool"] = _KeepAlivePool(self._retired)
         self._graphs: dict = {}
@@ -226,36 +225,24 @@ class CryoVITHeadTrainerB200:
         shared-memory images, flips / transposes for input gradients ...). The weights change every step and the
         re-arrangements are dozens of small torch kernels per layer, so on first use fn runs on the parameter's GLOBAL
         INDICES (exact in fp32 up to 2^24) and the result is kept as a gather table; from the next step on ONE
-        ``index_select`` over the flat bucket plus one cast produce every operand of the step (``_pk_refresh``)."""
-        v = self._pk_views.get(name)
+        ``index_select`` over the flat bucket plus one cast produce every operand of the step (``_pk_refresh``,
+        :class:`~cryovit_b200.operand_gather.OperandGather`)."""
+        v = self._gather.views.get(name)
         if v is not None:
             return v
         w = self.p[key]
-        if name not in self._pk_tables:
-            idx = (torch.arange(w.numel(), device=self.device, dtype=F32) + float(self._offsets[key] + 1)).view(w.shape)
-            t = fn(idx)
-            table = t.round().long().flatten() - 1
-            table[table < 0] = self._nparams  # padding -> the zero slot
-            self._pk_tables[name] = (table, tuple(t.shape))
-            if self._pk_cat is not None:
-                self._retired.append(self._pk_cat)  # an already captured graph gathers through the old table
-            self._pk_cat = None
+        if name not in self._gather.tables:
+            self._gather.add(name, fn(self._gather.indices(self._offsets[key], w.shape)), BF16)
         return fn(w).to(BF16).contiguous()
 
     def _pk_refresh(self) -> None:
         """One gather + one cast for all operand images whose tables exist (called at the start of a step)."""
-        self._pk_views = {}
-        if not self._pk_tables:
-            return
-        if self._pk_cat is None:
-            self._pk_names = list(self._pk_tables)
-            self._pk_cat = torch.cat([self._pk_tables[k][0] for k in self._pk_names])
-        packed = self._flat_store.index_select(0, self._pk_cat).to(BF16)
-        off = 0
-        for k in self._pk_names:
-            table, shape = self._pk_tables[k]
-            self._pk_views[k] = packed[off:off + table.numel()].view(shape)
-            off += table.numel()
+        self._gather.refresh()
+
+    def parameter_bucket(self) -> tuple[torch.Tensor, dict[str, int], dict[str, tuple]]:
+        """(fp32 [n + 1] bucket: the master weights and a trailing zero, offset and shape of every parameter): what
+        ``CryoVITHeadB200.attach_bucket`` gathers its operands from."""
+        return self._flat_store, dict(self._offsets), {k: tuple(v.shape) for k, v in self.p.items()}
 
     # ------------------------------------------------------------------ helpers
     def state_dict(self) -> dict[str, torch.Tensor]:

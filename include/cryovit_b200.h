@@ -305,6 +305,14 @@ int cvit_conv3d_rows8(const void* x, const void* w_img, const float* bias, void*
  * fp32 [D,H,W] and/or their sigmoid -> probs (cryovit.py:39,49); either pointer may be null. */
 int cvit_conv3d_rows8_final(const void* x, const void* w_img, const float* bias, float* logits, float* probs, int64_t D,
                             int64_t H, int64_t W, void* stream);
+/* ... scored instead of stored (a validation pass): the same MMAs, clip and sigmoid, and an epilogue that reads the voxel's
+ * int8 label (labels [D,H,W], -1 = ignore) and accumulates the eight masked sums of cvit_seg_stats with threshold; out8 fp64 [8]
+ * is overwritten. Each CTA writes one fp64 row of 8 into partials (cvit_conv3d_rows8_score_partials(D, H, W) doubles the caller
+ * provides), a one-block kernel adds the rows in a fixed order: counts (sums 1, 3..7) are exact, and two runs give
+ * bit-identical sums. W % 8 != 0: CVIT_ERR_UNSUPPORTED; null labels / partials / out8: CVIT_ERR_INVALID. */
+int64_t cvit_conv3d_rows8_score_partials(int64_t D, int64_t H, int64_t W);
+int cvit_conv3d_rows8_score(const void* x, const void* w_img, const float* bias, const int8_t* labels, int64_t D, int64_t H,
+                            int64_t W, float threshold, double* partials, double* out8, void* stream);
 
 /* The 16- / 32-channel depth-dilated convolutions of SynthesisBlocks 3-4 the same way (csrc/conv_rows.cu): 8-channel chunk arrays
  * of the input rows as K-major operands (column taps = 16-byte shifts), a 144-column accumulator window per input row sliding
