@@ -98,6 +98,27 @@ SIGNATURES: dict[str, list] = {
     "cvit_conv3d_halo_ndhwc_tab": [P, P, P, P, I64, I64, I64, I64, I64, I64, I64, P],
     "cvit_conv3d_wpackn_ndhwc": [P, P, P, P, I64, I64, I64, I64, I64, I64, I64, I32, P],
     "cvit_wgrad_mn_ndhwc": [P, P, P, I64, I64, I64, I64, I64, I64, I64, I32, P],
+    # deterministic mode of head training: *_det take (..., scratch, scratch_elems, stream); *_det_partials return a size
+    "cvit_groupnorm_ndhwc_bf16_det": [P, P, P, P, P, I64, I64, I64, F32, P, I64, P],
+    "cvit_groupnorm_ndhwc_bf16_det_partials": [I64, I64, I64],
+    "cvit_seg_stats_det": [P, P, I64, F32, P, P, I64, P],
+    "cvit_seg_stats_det_partials": [I64],
+    "cvit_colsum_bf16_det": [P, P, I64, I64, P, I64, P],
+    "cvit_colsum_bf16_det_partials": [I64, I64],
+    "cvit_gelu_bwd_colsum_bf16_det": [P, P, P, P, I64, I64, P, I64, P],
+    "cvit_gelu_bwd_colsum_bf16_det_partials": [I64, I64],
+    "cvit_gelu_bwd_colsum_unshuffle_bf16_det": [P, P, P, P, I64, I64, I64, I64, P, I64, P],
+    "cvit_gelu_bwd_colsum_unshuffle_bf16_det_partials": [I64, I64, I64, I64],
+    "cvit_groupnorm_bwd_gelu_ndhwc_bf16_det": [P, P, P, P, P, P, P, I64, I64, I64, F32, P, P, I64, P, I64, P],
+    "cvit_groupnorm_bwd_gelu_ndhwc_bf16_det_partials": [I64, I64, I64],
+    "cvit_wgrad_tc8_ndhwc_det": [P, P, P, I64, I64, I64, I64, P, I64, P],
+    "cvit_wgrad_tc8_ndhwc_det_partials": [I64, I64, I64],
+    "cvit_wgrad_tcn_ndhwc_det": [P, P, P, I64, I64, I64, I64, I64, I64, P, I64, P],
+    "cvit_wgrad_tcn_ndhwc_det_partials": [I64, I64, I64, I64, I64],
+    "cvit_wgrad_mn_ndhwc_det": [P, P, P, I64, I64, I64, I64, I64, I64, I64, I32, P, I64, P],
+    "cvit_wgrad_mn_ndhwc_det_partials": [I64, I64, I64, I64, I64, I64],
+    "cvit_wgrad_splitk_det": [P, P, P, P, I64, I64, I64, I64, I64, I64, P, I64, P],
+    "cvit_wgrad_splitk_det_partials": [I64, I64, I64, I64],
     "cvit_set_gemm_pair": [I32],  # returns the previous setting, not an error code (use load().cvit_set_gemm_pair)
 }
 
@@ -139,6 +160,9 @@ def load() -> ctypes.CDLL:
         fn.restype = c_int
         fn.argtypes = argtypes
     lib.cvit_conv3d_rows8_score_partials.restype = c_int64
+    for name in SIGNATURES:
+        if name.endswith("_det_partials"):
+            getattr(lib, name).restype = c_int64
     _lib = lib
     return lib
 

@@ -15,7 +15,7 @@ ROOT = Path(__file__).resolve().parent
 CSRC = ROOT / "csrc"
 LIBDIR = ROOT / "lib"
 LIB = LIBDIR / "libcryovit_b200.so"
-SOURCES = ["host_common.cu", "gemm.cu", "vit_elementwise.cu", "attention.cu", "attention_tcgen05.cu", "head_elementwise.cu", "gn_fold.cu", "conv_halo.cu", "conv_wpackn.cu", "conv_wpack.cu", "conv_rows8.cu", "conv_rows.cu", "wgrad.cu", "wgrad_mn.cu", "wgrad_narrow.cu", "wgrad_tc.cu", "train_elementwise.cu"]
+SOURCES = ["host_common.cu", "gemm.cu", "vit_elementwise.cu", "attention.cu", "attention_tcgen05.cu", "head_elementwise.cu", "gn_fold.cu", "conv_halo.cu", "conv_wpackn.cu", "conv_wpack.cu", "conv_rows8.cu", "conv_rows.cu", "wgrad.cu", "wgrad_mn.cu", "wgrad_narrow.cu", "wgrad_tc.cu", "train_elementwise.cu", "det_reduce.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr",

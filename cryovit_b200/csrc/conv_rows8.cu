@@ -29,6 +29,7 @@
 // (ONE box of whole 128-byte lines for the ten input rows of a (plane, segment) -- with a box per row the TMA issue rate
 // bounded the kernel at 0.46 ms -- zero fill = padding), warp 1 MMA issuer (row loop unrolled, descriptors = base + constant),
 // warps 2-9 epilogue (two warps per TMEM lane quarter, half of the tile's rows each).
+#include "det_reduce.cuh"
 #include "ptx.cuh"
 #include "tmap.h"
 
@@ -410,6 +411,11 @@ __global__ void __launch_bounds__(256) rows8_score_finalize_kernel(const double*
     for (int i = 0; i < 32; ++i) t += red[i][threadIdx.x];
     out8[threadIdx.x] = t;
   }
+}
+
+int rows8_score_finalize(const double* partials, int rows, double* out8, cudaStream_t stream) {
+  rows8_score_finalize_kernel<<<1, 256, 0, stream>>>(partials, rows, out8);
+  return check_launch("rows8_score_finalize_kernel");
 }
 
 }  // namespace cvit

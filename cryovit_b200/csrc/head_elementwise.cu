@@ -1,6 +1,7 @@
 // HBM-bound pieces of the CryoVIT 3-D head (reference src/cryovit/models/cryovit.py:10-83):
 // feature-volume layout change, GroupNorm, and the narrow (8-channel) tail convolutions that are too thin
 // for a tensor-core tile and run as direct convolutions on the CUDA cores from a shared-memory halo tile.
+#include "det_reduce.cuh"
 #include "ptx.cuh"
 #include "tmap.h"
 
@@ -75,13 +76,18 @@ __global__ void __launch_bounds__(256) features_f16_to_ndhwc_vec_kernel(const __
 // GroupNorm over channels-last bf16 [DHW, C]. Pass 1: per-group sum / sum of squares (fp32, block-reduced,
 // one atomicAdd pair per (block, group)). Pass 2: normalise + affine.
 // Thread t owns the 8-channel vector (t % (C/8)) and strides over rows.
-__global__ void __launch_bounds__(256) groupnorm_stats_kernel(const __nv_bfloat16* __restrict__ x, float* __restrict__ stats,
-                                                               int64_t DHW, int C, int G, int rows_per_block) {
-  extern __shared__ float s_part[];  // [2][G]
+// DET (deterministic mode): no atomics; stats is a [gridDim.x][2G] partial slab, each block's row summed over its threads in
+// thread order.
+template <bool DET>
+__device__ __forceinline__ void groupnorm_stats_body(const __nv_bfloat16* __restrict__ x, float* __restrict__ stats, int64_t DHW, int C,
+                                                     int G, int rows_per_block) {
+  extern __shared__ float s_part[];  // [2][G] | DET: [256][4] = (s0, q0, s1, q1) per thread
   const int nvec = C / 8;
   const int cpg = C / G;  // channels per group: 8 or 4 (a vector spans 1 or 2 groups)
-  for (int i = threadIdx.x; i < 2 * G; i += blockDim.x) s_part[i] = 0.f;
-  __syncthreads();
+  if constexpr (!DET) {
+    for (int i = threadIdx.x; i < 2 * G; i += blockDim.x) s_part[i] = 0.f;
+    __syncthreads();
+  }
   const int vec = threadIdx.x % nvec;
   const int rsub = threadIdx.x / nvec, rstep = blockDim.x / nvec;
   const int64_t r0 = (int64_t)blockIdx.x * rows_per_block;
@@ -99,7 +105,12 @@ __global__ void __launch_bounds__(256) groupnorm_stats_kernel(const __nv_bfloat1
         q[half] += f.x * f.x + f.y * f.y;
       }
     }
-    if (cpg >= 8) {
+    if constexpr (DET) {
+      s_part[threadIdx.x * 4 + 0] = s[0];
+      s_part[threadIdx.x * 4 + 1] = q[0];
+      s_part[threadIdx.x * 4 + 2] = s[1];
+      s_part[threadIdx.x * 4 + 3] = q[1];
+    } else if (cpg >= 8) {
       const int g = (vec * 8) / cpg;
       atomicAdd(&s_part[g], s[0]);
       atomicAdd(&s_part[G + g], q[0]);
@@ -112,7 +123,37 @@ __global__ void __launch_bounds__(256) groupnorm_stats_kernel(const __nv_bfloat1
     }
   }
   __syncthreads();
-  for (int i = threadIdx.x; i < 2 * G; i += blockDim.x) atomicAdd(&stats[i], s_part[i]);
+  if constexpr (DET) {
+    // entry i of the row: group g = i % G, sum (i < G) or sum of squares; threads t < rstep * nvec in order
+    const int tn = (blockDim.x / nvec) * nvec;
+    for (int i = threadIdx.x; i < 2 * G; i += blockDim.x) {
+      const int g = i % G, sq = i >= G ? 1 : 0;
+      float a = 0.f;
+      for (int t = 0; t < tn; ++t) {
+        const int vec = t % nvec;
+        if (cpg >= 8) {
+          if ((vec * 8) / cpg == g) a += s_part[t * 4 + sq];
+        } else if (vec * 2 == g) {
+          a += s_part[t * 4 + sq];
+        } else if (vec * 2 + 1 == g) {
+          a += s_part[t * 4 + 2 + sq];
+        }
+      }
+      stats[(size_t)blockIdx.x * 2 * G + i] = a;
+    }
+  } else {
+    for (int i = threadIdx.x; i < 2 * G; i += blockDim.x) atomicAdd(&stats[i], s_part[i]);
+  }
+}
+
+__global__ void __launch_bounds__(256) groupnorm_stats_kernel(const __nv_bfloat16* __restrict__ x, float* __restrict__ stats,
+                                                               int64_t DHW, int C, int G, int rows_per_block) {
+  groupnorm_stats_body<false>(x, stats, DHW, C, G, rows_per_block);
+}
+
+__global__ void __launch_bounds__(256) groupnorm_stats_det_kernel(const __nv_bfloat16* __restrict__ x, float* __restrict__ partials,
+                                                                   int64_t DHW, int C, int G, int rows_per_block) {
+  groupnorm_stats_body<true>(x, partials, DHW, C, G, rows_per_block);
 }
 
 __global__ void __launch_bounds__(256) groupnorm_apply_kernel(const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __restrict__ out,
@@ -325,6 +366,49 @@ int cvit_groupnorm_ndhwc_bf16(const void* x, void* out, const float* gamma, cons
   return check_launch("groupnorm_apply_kernel");
 }
 
+// Deterministic mode: the same two passes, the statistics as [blocks][2G] partial rows added in a fixed order.
+static int groupnorm_stats_grid(int64_t DHW, int64_t* rpb_out) {
+  int blocks = num_sms() * 8;
+  int64_t rows_per_block = (DHW + blocks - 1) / blocks;
+  if (rows_per_block < 1) rows_per_block = 1;
+  *rpb_out = rows_per_block;
+  return (int)((DHW + rows_per_block - 1) / rows_per_block);
+}
+
+int64_t cvit_groupnorm_ndhwc_bf16_det_partials(int64_t DHW, int64_t C, int64_t G) {
+  int64_t rpb;
+  return DHW > 0 && C > 0 && G > 0 ? (int64_t)groupnorm_stats_grid(DHW, &rpb) * 2 * G : 0;
+}
+
+int cvit_groupnorm_ndhwc_bf16_det(const void* x, void* out, const float* gamma, const float* beta, float* stats, int64_t DHW, int64_t C,
+                                  int64_t G, float eps, float* scratch, int64_t scratch_elems, void* stream) {
+  if (!x || !out || !gamma || !beta || !stats || DHW <= 0 || C <= 0 || G <= 0 || (C % 8) || (C % G)) {
+    set_error("groupnorm_det: bad arguments");
+    return CVIT_ERR_INVALID;
+  }
+  const int cpg = (int)(C / G);
+  const int nvec = (int)(C / 8);
+  if (!(cpg == 4 || (cpg % 8) == 0) || nvec > 256 || (256 % nvec) != 0) {
+    set_error("groupnorm_det: C=%lld G=%lld unsupported (channels per group must be 4 or a multiple of 8; C / 8 a divisor of 256)",
+              (long long)C, (long long)G);
+    return CVIT_ERR_UNSUPPORTED;
+  }
+  if (int rc = det_check_scratch(scratch, scratch_elems, cvit_groupnorm_ndhwc_bf16_det_partials(DHW, C, G), "groupnorm_det")) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  int64_t rows_per_block;
+  const int blocks = groupnorm_stats_grid(DHW, &rows_per_block);
+  groupnorm_stats_det_kernel<<<blocks, 256, 256 * 4 * sizeof(float), st>>>(static_cast<const __nv_bfloat16*>(x), scratch, DHW, (int)C,
+                                                                          (int)G, (int)rows_per_block);
+  if (int rc = check_launch("groupnorm_stats_det_kernel")) return rc;
+  if (int rc = det_finalize(scratch, blocks, 2 * G, 2 * G, stats, false, st)) return rc;
+  const int64_t total = DHW * nvec;
+  int64_t g2 = (total + 255) / 256;
+  if (g2 > (int64_t)num_sms() * 16) g2 = (int64_t)num_sms() * 16;
+  groupnorm_apply_kernel<<<(int)g2, 256, 0, st>>>(static_cast<const __nv_bfloat16*>(x), static_cast<__nv_bfloat16*>(out), gamma, beta,
+                                                  stats, DHW, (int)C, (int)G, eps);
+  return check_launch("groupnorm_apply_kernel");
+}
+
 int cvit_head_tail_fused(const void* x, const float* w1, const float* b1, const float* w2, const float* b2,
                          float* logits, float* probs, void* scratch_bf16, int64_t D, int64_t H, int64_t W,
                          void* stream) {
@@ -389,8 +473,10 @@ int cvit_head_out_conv(const void* x, const float* w2, const float* b2, float* l
 //   3 sum y*[p >= thr]   4 sum [p >= thr]                  (DiceMetric: "pred < thr -> 0 else 1")
 //   5 sum y*[p > .5]   6 sum (1-y)*[p > .5]   7 sum y*(1-[p > .5])     (F1Metric: strict ">")
 namespace cvit {
-__global__ void __launch_bounds__(256) seg_stats_kernel(const float* __restrict__ probs, const float* __restrict__ labels,
-                                                        int64_t n, float thr, double* __restrict__ out) {
+// DET (deterministic mode): out is a [gridDim.x][8] partial slab, one row per block, added by rows8_score_finalize.
+template <bool DET>
+__device__ __forceinline__ void seg_stats_body(const float* __restrict__ probs, const float* __restrict__ labels, int64_t n, float thr,
+                                               double* __restrict__ out) {
   float v[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     const float y = labels[i], p = probs[i];
@@ -418,8 +504,28 @@ __global__ void __launch_bounds__(256) seg_stats_kernel(const float* __restrict_
   if (threadIdx.x < 8) {
     double t = 0.0;
     for (int w = 0; w < 8; ++w) t += red[threadIdx.x][w];
-    atomicAdd(out + threadIdx.x, t);
+    if constexpr (DET) {
+      out[(size_t)blockIdx.x * 8 + threadIdx.x] = t;
+    } else {
+      atomicAdd(out + threadIdx.x, t);
+    }
   }
+}
+
+__global__ void __launch_bounds__(256) seg_stats_kernel(const float* __restrict__ probs, const float* __restrict__ labels,
+                                                        int64_t n, float thr, double* __restrict__ out) {
+  seg_stats_body<false>(probs, labels, n, thr, out);
+}
+
+__global__ void __launch_bounds__(256) seg_stats_det_kernel(const float* __restrict__ probs, const float* __restrict__ labels,
+                                                            int64_t n, float thr, double* __restrict__ partials) {
+  seg_stats_body<true>(probs, labels, n, thr, partials);
+}
+
+static int64_t seg_stats_grid(int64_t n) {
+  int64_t blocks = (n + 256 * 16 - 1) / (256 * 16);
+  const int64_t cap = (int64_t)num_sms() * 8;
+  return blocks > cap ? cap : blocks;
 }
 }  // namespace cvit
 
@@ -434,5 +540,21 @@ extern "C" int cvit_seg_stats(const float* probs, const float* labels, int64_t n
   if (blocks > cap) blocks = cap;
   cvit::seg_stats_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(probs, labels, n, threshold, out8);
   return cvit::check_launch("seg_stats_kernel");
+}
+
+extern "C" int64_t cvit_seg_stats_det_partials(int64_t n) { return n > 0 ? cvit::seg_stats_grid(n) * 8 : 0; }
+
+// Deterministic mode: out8 is OVERWRITTEN with the fixed-order sum of one fp64 row of 8 per block (scratch: doubles).
+extern "C" int cvit_seg_stats_det(const float* probs, const float* labels, int64_t n, float threshold, double* out8, double* scratch,
+                                  int64_t scratch_elems, void* stream) {
+  if (!probs || !labels || !out8 || n <= 0) {
+    cvit::set_error("seg_stats_det: bad arguments");
+    return cvit::CVIT_ERR_INVALID;
+  }
+  if (int rc = cvit::det_check_scratch(scratch, scratch_elems, cvit_seg_stats_det_partials(n), "seg_stats_det")) return rc;
+  const int64_t blocks = cvit::seg_stats_grid(n);
+  cvit::seg_stats_det_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(probs, labels, n, threshold, scratch);
+  if (int rc = cvit::check_launch("seg_stats_det_kernel")) return rc;
+  return cvit::rows8_score_finalize(scratch, (int)blocks, out8, (cudaStream_t)stream);
 }
 

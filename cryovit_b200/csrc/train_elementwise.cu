@@ -3,6 +3,7 @@
 // sigmoid and the clip, GroupNorm backward, bias gradients, the pixel un-shuffle that turns the transposed
 // convolution's input gradient into a GEMM, and AdamW. The tensor-core work (dgrad = the forward convolution
 // kernels run on flipped / transposed weights, wgrad = csrc/wgrad.cu) lives elsewhere.
+#include "det_reduce.cuh"
 #include "ptx.cuh"
 #include "tmap.h"
 
@@ -53,12 +54,15 @@ __global__ void __launch_bounds__(256) gelu_bwd_kernel(const uint4* __restrict__
 // W2 > 0: the rows are the voxels of a [D, H2, W2, C] volume (H2, W2 even) and dz is written PIXEL-UNSHUFFLED, as
 // [D, H2/2, W2/2, (i, j, C)] with (i, j) the sub-pixel -- the row layout the transposed convolution's input-gradient and
 // weight-gradient GEMMs read -- instead of through a separate permutation pass over the largest gradient volumes.
-__global__ void __launch_bounds__(256) gelu_bwd_colsum_kernel(const uint4* __restrict__ da, const uint4* __restrict__ z,
-                                                               uint4* __restrict__ dz, float* __restrict__ db, int64_t R, int C,
-                                                               int64_t rows_per_block, int W2) {
-  extern __shared__ float s_db[];  // [C]
-  for (int i = threadIdx.x; i < C; i += blockDim.x) s_db[i] = 0.f;
-  __syncthreads();
+// DET (deterministic mode): no atomics; db is a [gridDim.x][C] partial slab, one fixed-order row per block.
+template <bool DET>
+__device__ __forceinline__ void gelu_bwd_colsum_body(const uint4* __restrict__ da, const uint4* __restrict__ z, uint4* __restrict__ dz,
+                                                     float* __restrict__ db, int64_t R, int C, int64_t rows_per_block, int W2) {
+  extern __shared__ float s_db[];  // [C] | DET: [256][8]
+  if constexpr (!DET) {
+    for (int i = threadIdx.x; i < C; i += blockDim.x) s_db[i] = 0.f;
+    __syncthreads();
+  }
   const int nvec = C / 8;
   const int vec = threadIdx.x % nvec, rsub = threadIdx.x / nvec, rstep = blockDim.x / nvec;
   const int64_t r0 = (int64_t)blockIdx.x * rows_per_block;
@@ -88,11 +92,32 @@ __global__ void __launch_bounds__(256) gelu_bwd_colsum_kernel(const uint4* __res
       }
       dz[io] = make_uint4(o[0], o[1], o[2], o[3]);
     }
+    if constexpr (DET) {
 #pragma unroll
-    for (int k = 0; k < 8; ++k) atomicAdd(&s_db[vec * 8 + k], acc[k]);
+      for (int k = 0; k < 8; ++k) s_db[threadIdx.x * 8 + k] = acc[k];
+    } else {
+#pragma unroll
+      for (int k = 0; k < 8; ++k) atomicAdd(&s_db[vec * 8 + k], acc[k]);
+    }
   }
   __syncthreads();
-  for (int i = threadIdx.x; i < C; i += blockDim.x) atomicAdd(db + i, s_db[i]);
+  if constexpr (DET) {
+    det_block_colsum(s_db, C, nvec, rstep * nvec, 0, db + (size_t)blockIdx.x * C);
+  } else {
+    for (int i = threadIdx.x; i < C; i += blockDim.x) atomicAdd(db + i, s_db[i]);
+  }
+}
+
+__global__ void __launch_bounds__(256) gelu_bwd_colsum_kernel(const uint4* __restrict__ da, const uint4* __restrict__ z,
+                                                               uint4* __restrict__ dz, float* __restrict__ db, int64_t R, int C,
+                                                               int64_t rows_per_block, int W2) {
+  gelu_bwd_colsum_body<false>(da, z, dz, db, R, C, rows_per_block, W2);
+}
+
+__global__ void __launch_bounds__(256) gelu_bwd_colsum_det_kernel(const uint4* __restrict__ da, const uint4* __restrict__ z,
+                                                                   uint4* __restrict__ dz, float* __restrict__ db_partials, int64_t R,
+                                                                   int C, int64_t rows_per_block, int W2) {
+  gelu_bwd_colsum_body<true>(da, z, dz, db_partials, R, C, rows_per_block, W2);
 }
 
 // Dice loss L = 1 - 2 I / (Sy + Sp + eps) over the voxels with label > -1, p = sigmoid(clip(x, -5, 5)):
@@ -114,11 +139,15 @@ __global__ void __launch_bounds__(256) dice_bwd_kernel(const float* __restrict__
 }
 
 // column sums of a bf16 [R, C] matrix into fp32 [C] (bias gradients; caller zeroes `out`). C multiple of 8, <= 2048.
-__global__ void __launch_bounds__(256) colsum_kernel(const __nv_bfloat16* __restrict__ x, float* __restrict__ out,
-                                                      int64_t R, int C, int64_t rows_per_block) {
-  extern __shared__ float s_acc[];  // [C]
-  for (int i = threadIdx.x; i < C; i += blockDim.x) s_acc[i] = 0.f;
-  __syncthreads();
+// DET: out is a [gridDim.x][C] partial slab, one fixed-order row per block.
+template <bool DET>
+__device__ __forceinline__ void colsum_body(const __nv_bfloat16* __restrict__ x, float* __restrict__ out, int64_t R, int C,
+                                            int64_t rows_per_block) {
+  extern __shared__ float s_acc[];  // [C] | DET: [256][8]
+  if constexpr (!DET) {
+    for (int i = threadIdx.x; i < C; i += blockDim.x) s_acc[i] = 0.f;
+    __syncthreads();
+  }
   const int nvec = C / 8;
   const int vec = threadIdx.x % nvec, rsub = threadIdx.x / nvec, rstep = blockDim.x / nvec;
   const int64_t r0 = (int64_t)blockIdx.x * rows_per_block, r1 = min(r0 + rows_per_block, R);
@@ -134,22 +163,45 @@ __global__ void __launch_bounds__(256) colsum_kernel(const __nv_bfloat16* __rest
         acc[2 * k + 1] += f.y;
       }
     }
+    if constexpr (DET) {
 #pragma unroll
-    for (int k = 0; k < 8; ++k) atomicAdd(&s_acc[vec * 8 + k], acc[k]);
+      for (int k = 0; k < 8; ++k) s_acc[threadIdx.x * 8 + k] = acc[k];
+    } else {
+#pragma unroll
+      for (int k = 0; k < 8; ++k) atomicAdd(&s_acc[vec * 8 + k], acc[k]);
+    }
   }
   __syncthreads();
-  for (int i = threadIdx.x; i < C; i += blockDim.x) atomicAdd(out + i, s_acc[i]);
+  if constexpr (DET) {
+    det_block_colsum(s_acc, C, nvec, rstep * nvec, 0, out + (size_t)blockIdx.x * C);
+  } else {
+    for (int i = threadIdx.x; i < C; i += blockDim.x) atomicAdd(out + i, s_acc[i]);
+  }
+}
+
+__global__ void __launch_bounds__(256) colsum_kernel(const __nv_bfloat16* __restrict__ x, float* __restrict__ out,
+                                                      int64_t R, int C, int64_t rows_per_block) {
+  colsum_body<false>(x, out, R, C, rows_per_block);
+}
+
+__global__ void __launch_bounds__(256) colsum_det_kernel(const __nv_bfloat16* __restrict__ x, float* __restrict__ partials,
+                                                          int64_t R, int C, int64_t rows_per_block) {
+  colsum_body<true>(x, partials, R, C, rows_per_block);
 }
 
 // GroupNorm backward, pass 1: per channel  A_c = sum dy * xhat,  B_c = sum dy  (these ARE dgamma and dbeta).
 // xhat = (x - mean_g) * rstd_g from the forward statistics (sum, sum of squares per group).
-__global__ void __launch_bounds__(256) groupnorm_bwd_reduce_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
-                                                                    const float* __restrict__ stats, float* __restrict__ dgamma,
-                                                                    float* __restrict__ dbeta, int64_t DHW, int C, int G, float eps,
-                                                                    int64_t rows_per_block) {
-  extern __shared__ float s_ab[];  // [2][C]
-  for (int i = threadIdx.x; i < 2 * C; i += blockDim.x) s_ab[i] = 0.f;
-  __syncthreads();
+// DET: dgamma is a [gridDim.x][2C] partial slab (row = A then B), dbeta unused; one fixed-order row per block.
+template <bool DET>
+__device__ __forceinline__ void groupnorm_bwd_reduce_body(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
+                                                          const float* __restrict__ stats, float* __restrict__ dgamma,
+                                                          float* __restrict__ dbeta, int64_t DHW, int C, int G, float eps,
+                                                          int64_t rows_per_block) {
+  extern __shared__ float s_ab[];  // [2][C] | DET: [2][256][8]
+  if constexpr (!DET) {
+    for (int i = threadIdx.x; i < 2 * C; i += blockDim.x) s_ab[i] = 0.f;
+    __syncthreads();
+  }
   const int nvec = C / 8, cpg = C / G;
   const float inv_n = 1.0f / (static_cast<float>(DHW) * cpg);
   const int vec = threadIdx.x % nvec, rsub = threadIdx.x / nvec, rstep = blockDim.x / nvec;
@@ -177,30 +229,59 @@ __global__ void __launch_bounds__(256) groupnorm_bwd_reduce_kernel(const __nv_bf
         b[2 * k + 1] += fd.y;
       }
     }
+    if constexpr (DET) {
 #pragma unroll
-    for (int k = 0; k < 8; ++k) {
-      atomicAdd(&s_ab[vec * 8 + k], a[k]);
-      atomicAdd(&s_ab[C + vec * 8 + k], b[k]);
+      for (int k = 0; k < 8; ++k) {
+        s_ab[threadIdx.x * 8 + k] = a[k];
+        s_ab[256 * 8 + threadIdx.x * 8 + k] = b[k];
+      }
+    } else {
+#pragma unroll
+      for (int k = 0; k < 8; ++k) {
+        atomicAdd(&s_ab[vec * 8 + k], a[k]);
+        atomicAdd(&s_ab[C + vec * 8 + k], b[k]);
+      }
     }
   }
   __syncthreads();
-  for (int i = threadIdx.x; i < C; i += blockDim.x) {
-    atomicAdd(dgamma + i, s_ab[i]);
-    atomicAdd(dbeta + i, s_ab[C + i]);
+  if constexpr (DET) {
+    float* row = dgamma + (size_t)blockIdx.x * 2 * C;
+    det_block_colsum(s_ab, C, nvec, rstep * nvec, 0, row);
+    det_block_colsum(s_ab + 256 * 8, C, nvec, rstep * nvec, 0, row + C);
+  } else {
+    for (int i = threadIdx.x; i < C; i += blockDim.x) {
+      atomicAdd(dgamma + i, s_ab[i]);
+      atomicAdd(dbeta + i, s_ab[C + i]);
+    }
   }
 }
 
+__global__ void __launch_bounds__(256) groupnorm_bwd_reduce_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
+                                                                    const float* __restrict__ stats, float* __restrict__ dgamma,
+                                                                    float* __restrict__ dbeta, int64_t DHW, int C, int G, float eps,
+                                                                    int64_t rows_per_block) {
+  groupnorm_bwd_reduce_body<false>(x, dy, stats, dgamma, dbeta, DHW, C, G, eps, rows_per_block);
+}
+
+__global__ void __launch_bounds__(256) groupnorm_bwd_reduce_det_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
+                                                                        const float* __restrict__ stats, float* __restrict__ partials,
+                                                                        int64_t DHW, int C, int G, float eps, int64_t rows_per_block) {
+  groupnorm_bwd_reduce_body<true>(x, dy, stats, partials, nullptr, DHW, C, G, eps, rows_per_block);
+}
+
 // pass 2: dx = rstd_g * ( gamma_c dy - ( s1_g + xhat s2_g ) / N_g ),  s1_g = sum_c gamma_c B_c, s2_g = sum_c gamma_c A_c
-__global__ void __launch_bounds__(256) groupnorm_bwd_apply_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
-                                                                   __nv_bfloat16* __restrict__ dx, const float* __restrict__ gamma,
-                                                                   const float* __restrict__ stats, const float* __restrict__ dgamma,
-                                                                   const float* __restrict__ dbeta, int64_t DHW, int C, int G, float eps,
-                                                                   const __nv_bfloat16* __restrict__ z, float* __restrict__ db, int W2) {
+// DET (z != null only): db is a [gridDim.x][C] partial slab, one fixed-order row per block.
+template <bool DET>
+__device__ __forceinline__ void groupnorm_bwd_apply_body(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
+                                                         __nv_bfloat16* __restrict__ dx, const float* __restrict__ gamma,
+                                                         const float* __restrict__ stats, const float* __restrict__ dgamma,
+                                                         const float* __restrict__ dbeta, int64_t DHW, int C, int G, float eps,
+                                                         const __nv_bfloat16* __restrict__ z, float* __restrict__ db, int W2) {
   // z != null: the GroupNorm's input was gelu(z) (the block before ends in a transposed convolution + GELU, or the
   // projection + GELU): the result is multiplied by gelu'(z) right here -- dx is then the gradient of z -- its column sums
   // (that layer's bias gradient) go to db, and with W2 > 0 it is stored pixel-unshuffled ([D, H2/2, W2/2, 4C], see
   // gelu_bwd_colsum_kernel): one pass instead of two over the step's largest gradient volumes.
-  extern __shared__ float s_g[];  // [4][G]: mean, rstd, s1/N, s2/N | z != null: + [C] column sums
+  extern __shared__ float s_g[];  // [4][G]: mean, rstd, s1/N, s2/N | z != null: + [C] column sums (DET: + [256][8])
   const int cpg = C / G;
   const float inv_n = 1.0f / (static_cast<float>(DHW) * cpg);
   for (int g = threadIdx.x; g < G; g += blockDim.x) {
@@ -220,7 +301,7 @@ __global__ void __launch_bounds__(256) groupnorm_bwd_apply_kernel(const __nv_bfl
   const int nvec = C / 8;
   const int64_t total = DHW * nvec;
   float* s_db = s_g + 4 * G;
-  if (z)
+  if (!DET && z)
     for (int i = threadIdx.x; i < C; i += blockDim.x) s_db[i] = 0.f;
   float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};  // this thread's 8 channels (the grid stride is a multiple of nvec)
   __syncthreads();
@@ -261,13 +342,37 @@ __global__ void __launch_bounds__(256) groupnorm_bwd_apply_kernel(const __nv_bfl
     }
     *reinterpret_cast<uint4*>(dx + io * 8) = make_uint4(o[0], o[1], o[2], o[3]);
   }
-  if (z) {
+  if constexpr (DET) {
+    if (z) {
+#pragma unroll
+      for (int k = 0; k < 8; ++k) s_db[threadIdx.x * 8 + k] = acc[k];
+      __syncthreads();
+      det_block_colsum(s_db, C, nvec, blockDim.x, (int)(((int64_t)blockIdx.x * blockDim.x) % nvec), db + (size_t)blockIdx.x * C);
+    }
+  } else if (z) {
     const int vec = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) % nvec);
 #pragma unroll
     for (int k = 0; k < 8; ++k) atomicAdd(&s_db[vec * 8 + k], acc[k]);
     __syncthreads();
     for (int i = threadIdx.x; i < C; i += blockDim.x) atomicAdd(db + i, s_db[i]);
   }
+}
+
+__global__ void __launch_bounds__(256) groupnorm_bwd_apply_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
+                                                                   __nv_bfloat16* __restrict__ dx, const float* __restrict__ gamma,
+                                                                   const float* __restrict__ stats, const float* __restrict__ dgamma,
+                                                                   const float* __restrict__ dbeta, int64_t DHW, int C, int G, float eps,
+                                                                   const __nv_bfloat16* __restrict__ z, float* __restrict__ db, int W2) {
+  groupnorm_bwd_apply_body<false>(x, dy, dx, gamma, stats, dgamma, dbeta, DHW, C, G, eps, z, db, W2);
+}
+
+__global__ void __launch_bounds__(256) groupnorm_bwd_apply_det_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
+                                                                       __nv_bfloat16* __restrict__ dx, const float* __restrict__ gamma,
+                                                                       const float* __restrict__ stats, const float* __restrict__ dgamma,
+                                                                       const float* __restrict__ dbeta, int64_t DHW, int C, int G, float eps,
+                                                                       const __nv_bfloat16* __restrict__ z, float* __restrict__ db_partials,
+                                                                       int W2) {
+  groupnorm_bwd_apply_body<true>(x, dy, dx, gamma, stats, dgamma, dbeta, DHW, C, G, eps, z, db_partials, W2);
 }
 
 // [D, 2H, 2W, C] -> [D, H, W, 4C], column (i*2 + j) * C + c : the transposed convolution's output gradient as rows of
@@ -348,6 +453,62 @@ int cvit_gelu_bwd_colsum_unshuffle_bf16(const void* da, const void* z, void* dzu
   return gelu_bwd_colsum_launch(da, z, dzun, db, D * H2 * W2, C, (int)W2, stream);
 }
 
+// ---------------------------------------------------------------------------------------------- deterministic mode
+// The column-sum kernels below have the grid of their default twins (num_sms() * 8 blocks of rows_per_block rows); each
+// block writes one [C] row of the scratch slab and det_finalize adds the rows in order (csrc/det_reduce.cuh).
+static int64_t colsum_grid(int64_t R, int64_t* rpb_out) {
+  int64_t blocks = (int64_t)num_sms() * 8;
+  int64_t rpb = (R + blocks - 1) / blocks;
+  if (rpb < 1) rpb = 1;
+  *rpb_out = rpb;
+  return (R + rpb - 1) / rpb;
+}
+
+int64_t cvit_colsum_bf16_det_partials(int64_t R, int64_t C) {
+  int64_t rpb;
+  return R > 0 && C > 0 ? colsum_grid(R, &rpb) * C : 0;
+}
+
+int cvit_colsum_bf16_det(const void* x, float* out, int64_t R, int64_t C, float* scratch, int64_t scratch_elems, void* stream) {
+  if (!x || !out || R <= 0 || C <= 0 || (C % 8) || C > 2048) { set_error("colsum_det: bad arguments"); return CVIT_ERR_INVALID; }
+  if (int rc = det_check_scratch(scratch, scratch_elems, cvit_colsum_bf16_det_partials(R, C), "colsum_det")) return rc;
+  int64_t rpb;
+  const int64_t blocks = colsum_grid(R, &rpb);
+  colsum_det_kernel<<<(unsigned)blocks, 256, 256 * 8 * sizeof(float), (cudaStream_t)stream>>>(static_cast<const __nv_bfloat16*>(x), scratch,
+                                                                                             R, (int)C, rpb);
+  if (int rc = check_launch("colsum_det_kernel")) return rc;
+  return det_finalize(scratch, blocks, C, C, out, true, (cudaStream_t)stream);
+}
+
+static int gelu_bwd_colsum_det_launch(const void* da, const void* z, void* dz, float* db, int64_t R, int64_t C, int W2, float* scratch,
+                                      int64_t scratch_elems, void* stream) {
+  if (!da || !z || !dz || !db || R <= 0 || C <= 0 || (C % 8) || C > 2048) { set_error("gelu_bwd_colsum_det: bad arguments"); return CVIT_ERR_INVALID; }
+  if (int rc = det_check_scratch(scratch, scratch_elems, cvit_colsum_bf16_det_partials(R, C), "gelu_bwd_colsum_det")) return rc;
+  int64_t rpb;
+  const int64_t blocks = colsum_grid(R, &rpb);
+  gelu_bwd_colsum_det_kernel<<<(unsigned)blocks, 256, 256 * 8 * sizeof(float), (cudaStream_t)stream>>>(
+      static_cast<const uint4*>(da), static_cast<const uint4*>(z), static_cast<uint4*>(dz), scratch, R, (int)C, rpb, W2);
+  if (int rc = check_launch("gelu_bwd_colsum_det_kernel")) return rc;
+  return det_finalize(scratch, blocks, C, C, db, true, (cudaStream_t)stream);
+}
+
+int64_t cvit_gelu_bwd_colsum_bf16_det_partials(int64_t R, int64_t C) { return cvit_colsum_bf16_det_partials(R, C); }
+
+int cvit_gelu_bwd_colsum_bf16_det(const void* da, const void* z, void* dz, float* db, int64_t R, int64_t C, float* scratch,
+                                  int64_t scratch_elems, void* stream) {
+  return gelu_bwd_colsum_det_launch(da, z, dz, db, R, C, 0, scratch, scratch_elems, stream);
+}
+
+int64_t cvit_gelu_bwd_colsum_unshuffle_bf16_det_partials(int64_t D, int64_t H2, int64_t W2, int64_t C) {
+  return cvit_colsum_bf16_det_partials(D * H2 * W2, C);
+}
+
+int cvit_gelu_bwd_colsum_unshuffle_bf16_det(const void* da, const void* z, void* dzun, float* db, int64_t D, int64_t H2, int64_t W2,
+                                            int64_t C, float* scratch, int64_t scratch_elems, void* stream) {
+  if (D <= 0 || H2 <= 0 || W2 <= 0 || (H2 & 1) || (W2 & 1)) { set_error("gelu_bwd_colsum_unshuffle_det: H2 and W2 must be even"); return CVIT_ERR_INVALID; }
+  return gelu_bwd_colsum_det_launch(da, z, dzun, db, D * H2 * W2, C, (int)W2, scratch, scratch_elems, stream);
+}
+
 int cvit_dice_bwd(const float* logits, const float* probs, const float* labels, const double* stats8, float scale,
                   void* dlogit8_bf16, int64_t n, void* stream) {
   if (!logits || !probs || !labels || !stats8 || !dlogit8_bf16 || n <= 0) { set_error("dice_bwd: bad arguments"); return CVIT_ERR_INVALID; }
@@ -403,6 +564,49 @@ int cvit_groupnorm_bwd_gelu_ndhwc_bf16(const void* x, const void* dy, void* dx, 
       static_cast<const __nv_bfloat16*>(x), static_cast<const __nv_bfloat16*>(dy), static_cast<__nv_bfloat16*>(dx), gamma, stats,
       dgamma, dbeta, DHW, (int)C, (int)G, eps, static_cast<const __nv_bfloat16*>(z), db, (int)W2);
   return check_launch("groupnorm_bwd_apply_kernel");
+}
+
+// Deterministic mode: the reduce pass writes [blocks][2C] rows (dgamma | dbeta), two finalizes write dgamma and dbeta; with z
+// the apply pass writes [blocks][C] rows of db (the same scratch, reused after the first finalizes) and a third adds them.
+static int64_t gn_bwd_reduce_grid(int64_t DHW, int64_t* rpb_out) { return colsum_grid(DHW, rpb_out); }
+
+int64_t cvit_groupnorm_bwd_gelu_ndhwc_bf16_det_partials(int64_t DHW, int64_t C, int64_t G) {
+  if (DHW <= 0 || C <= 0 || G <= 0) return 0;
+  int64_t rpb;
+  const int64_t a = gn_bwd_reduce_grid(DHW, &rpb) * 2 * C, b = (int64_t)ew_grid(DHW * (C / 8), 4) * C;
+  return a > b ? a : b;
+}
+
+int cvit_groupnorm_bwd_gelu_ndhwc_bf16_det(const void* x, const void* dy, void* dx, const float* gamma, const float* stats, float* dgamma,
+                                           float* dbeta, int64_t DHW, int64_t C, int64_t G, float eps, const void* z, float* db,
+                                           int64_t W2, float* scratch, int64_t scratch_elems, void* stream) {
+  if (!x || !dy || !dx || !gamma || !stats || !dgamma || !dbeta || DHW <= 0 || C <= 0 || G <= 0 || (C % 8) || (C % G) || C > 2048 ||
+      (z && !db) || (!z && W2 != 0) || W2 < 0 || (W2 & 1) || (W2 > 0 && (DHW % (2 * W2)) != 0)) {
+    set_error("groupnorm_bwd_det: bad arguments");
+    return CVIT_ERR_INVALID;
+  }
+  if (int rc = det_check_scratch(scratch, scratch_elems, cvit_groupnorm_bwd_gelu_ndhwc_bf16_det_partials(DHW, C, G), "groupnorm_bwd_det"))
+    return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  int64_t rpb;
+  const int64_t blocks = gn_bwd_reduce_grid(DHW, &rpb);
+  groupnorm_bwd_reduce_det_kernel<<<(unsigned)blocks, 256, 2 * 256 * 8 * sizeof(float), st>>>(
+      static_cast<const __nv_bfloat16*>(x), static_cast<const __nv_bfloat16*>(dy), stats, scratch, DHW, (int)C, (int)G, eps, rpb);
+  if (int rc = check_launch("groupnorm_bwd_reduce_det_kernel")) return rc;
+  if (int rc = det_finalize(scratch, blocks, C, 2 * C, dgamma, false, st)) return rc;
+  if (int rc = det_finalize(scratch + C, blocks, C, 2 * C, dbeta, false, st)) return rc;
+  const int g2 = ew_grid(DHW * (C / 8), 4);
+  if (!z) {
+    groupnorm_bwd_apply_kernel<<<g2, 256, 4 * G * sizeof(float), st>>>(
+        static_cast<const __nv_bfloat16*>(x), static_cast<const __nv_bfloat16*>(dy), static_cast<__nv_bfloat16*>(dx), gamma, stats, dgamma,
+        dbeta, DHW, (int)C, (int)G, eps, nullptr, nullptr, 0);
+    return check_launch("groupnorm_bwd_apply_kernel");
+  }
+  groupnorm_bwd_apply_det_kernel<<<g2, 256, (4 * G + 256 * 8) * sizeof(float), st>>>(
+      static_cast<const __nv_bfloat16*>(x), static_cast<const __nv_bfloat16*>(dy), static_cast<__nv_bfloat16*>(dx), gamma, stats, dgamma,
+      dbeta, DHW, (int)C, (int)G, eps, static_cast<const __nv_bfloat16*>(z), scratch, (int)W2);
+  if (int rc = check_launch("groupnorm_bwd_apply_det_kernel")) return rc;
+  return det_finalize(scratch, g2, C, C, db, true, st);
 }
 
 int cvit_pixel_unshuffle_1x2x2_bf16(const void* src, void* dst, int64_t D, int64_t H, int64_t W, int64_t C, void* stream) {

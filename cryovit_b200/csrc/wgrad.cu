@@ -20,6 +20,7 @@
 // item accumulates in TMEM and adds its partial tile into the fp32 result with red.global.add (the result buffer is
 // zeroed by the caller). One CTA per SM, 192 threads: TMA producer, MMA issuer (warp-uniform, elect.sync), four
 // epilogue warps (thread = output row).
+#include "det_reduce.cuh"
 #include "ptx.cuh"
 #include "tmap.h"
 
@@ -38,7 +39,7 @@ struct WgCfg {
 };
 
 struct WgArgs {
-  float* out;           // [ntaps][M][N] fp32, accumulated into
+  float* out;           // [ntaps][M][N] fp32, accumulated into (deterministic mode: [ksplit][ntaps][M][N], stored)
   const int* koffs;     // [ntaps] shift of the B operand along K (elements), device memory
   int M, N, ntaps;      // valid rows of A (co), valid rows of B (ci)
   int k_chunks;         // ceil(K / 64)
@@ -47,9 +48,10 @@ struct WgArgs {
   int Mp;               // rows per packed tap (co rounded up to 8), pack * Mp <= 128
 };
 
-template <int BN>
-__global__ void __launch_bounds__(WG_THREADS, 1)
-wgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const WgArgs args) {
+// DET (deterministic mode): an item's tile is STORED into K slice ks of the [ksplit][ntaps][M][N] slab (zeros for an empty
+// K range), and det_finalize adds the slices in ks order.
+template <int BN, bool DET>
+__device__ __forceinline__ void wgrad_tcgen05_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const WgArgs& args) {
   using Cfg = WgCfg<BN>;
   constexpr int STAGES = Cfg::STAGES;
   extern __shared__ uint8_t smem_raw[];
@@ -174,12 +176,19 @@ wgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
         live = r < pack * args.Mp && otap < args.ntaps && row < args.M;
       }
       float* orow = args.out + ((size_t)otap * args.M + row) * args.N + n0;
+      if constexpr (DET) orow += (size_t)((item % per_tap) % args.ksplit) * args.ntaps * args.M * args.N;
 #pragma unroll 1
       for (int c0 = 0; c0 < BN; c0 += 32) {
         uint32_t v[32];
         tmem_ld_32x32(t_acc + c0, v);
         tmem_ld_wait();
-        if (live && kc1 > kc0) {
+        if constexpr (DET) {
+          if (live) {
+#pragma unroll
+            for (int i = 0; i < 32; ++i)
+              if (n0 + c0 + i < args.N) orow[c0 + i] = kc1 > kc0 ? __uint_as_float(v[i]) : 0.f;
+          }
+        } else if (live && kc1 > kc0) {
 #pragma unroll
           for (int i = 0; i < 32; ++i)
             if (n0 + c0 + i < args.N) atomicAdd(orow + c0 + i, __uint_as_float(v[i]));
@@ -202,9 +211,21 @@ wgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
 }
 
 template <int BN>
+__global__ void __launch_bounds__(WG_THREADS, 1)
+wgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const WgArgs args) {
+  wgrad_tcgen05_body<BN, false>(tmA, tmB, args);
+}
+
+template <int BN>
+__global__ void __launch_bounds__(WG_THREADS, 1)
+wgrad_tcgen05_det_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const WgArgs args) {
+  wgrad_tcgen05_body<BN, true>(tmA, tmB, args);
+}
+
+template <int BN, bool DET = false>
 static int launch_wgrad(const CUtensorMap& tmA, const CUtensorMap& tmB, const WgArgs& a, cudaStream_t st) {
   using Cfg = WgCfg<BN>;
-  auto kern = wgrad_tcgen05_kernel<BN>;
+  auto kern = DET ? wgrad_tcgen05_det_kernel<BN> : wgrad_tcgen05_kernel<BN>;
   static bool configured = false;
   if (!configured) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM);
@@ -219,7 +240,7 @@ static int launch_wgrad(const CUtensorMap& tmA, const CUtensorMap& tmB, const Wg
   int grid = num_sms();
   if (grid > items) grid = items;
   kern<<<grid, WG_THREADS, Cfg::SMEM, st>>>(tmA, tmB, a);
-  return check_launch("wgrad_tcgen05_kernel");
+  return check_launch(DET ? "wgrad_tcgen05_det_kernel" : "wgrad_tcgen05_kernel");
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -403,6 +424,87 @@ extern "C" int cvit_ndhwc_to_cfirst_padded(const void* src, void* dst, int64_t D
       static_cast<const __nv_bfloat16*>(src), static_cast<__nv_bfloat16*>(dst), (int)D, (int)H, (int)W, (int)C, (int)pd,
       (int)ph, (int)pw, (int)Wp, (int)wshift, pitch);
   return check_launch("ndhwc_to_cfirst_padded_kernel");
+}
+
+// Launch geometry of cvit_wgrad_splitk: N tile, taps per A tile and K split.
+static void splitk_geometry(int64_t M, int64_t N, int64_t K, int64_t ntaps, int* bn, int* pack, int* Mp, int* k_chunks, int* ksplit) {
+  *bn = N > 192 ? 256 : N > 128 ? 192 : N > 64 ? 128 : N > 32 ? 64 : 32;  // 192: one exact tile for the 192-channel layers
+  // narrow outputs: pack several taps into the 128 MMA rows (see the header comment)
+  *Mp = (int)((M + 7) / 8 * 8);
+  *pack = (M <= 64 && ntaps > 1) ? WG_BM / *Mp : 1;
+  if (*pack > ntaps) *pack = (int)ntaps;
+  *k_chunks = (int)((K + WG_KC - 1) / WG_KC);
+  const int m_tiles = *pack > 1 ? 1 : (int)((M + WG_BM - 1) / WG_BM), n_tiles = (int)((N + *bn - 1) / *bn);
+  const int64_t tiles = ((ntaps + *pack - 1) / *pack) * m_tiles * n_tiles;
+  // enough K ranges for ~4 items per SM, but never K ranges shorter than 32 chunks (2048 reduction steps)
+  int ks = (int)((4 * (int64_t)num_sms() + tiles - 1) / tiles);
+  const int max_split = *k_chunks / 32 > 0 ? *k_chunks / 32 : 1;
+  if (ks > max_split) ks = max_split;
+  if (ks < 1) ks = 1;
+  *ksplit = ks;
+}
+
+extern "C" int64_t cvit_wgrad_splitk_det_partials(int64_t M, int64_t N, int64_t K, int64_t ntaps) {
+  if (M <= 0 || N <= 0 || K <= 0 || ntaps <= 0) return 0;
+  int bn, pack, Mp, k_chunks, ksplit;
+  splitk_geometry(M, N, K, ntaps, &bn, &pack, &Mp, &k_chunks, &ksplit);
+  return (int64_t)ksplit * ntaps * M * N;
+}
+
+// Deterministic mode: out += the same product, every item's tile stored into its K slice of scratch
+// (cvit_wgrad_splitk_det_partials floats) and the slices added in K order.
+extern "C" int cvit_wgrad_splitk_det(const void* At, const void* Bt, float* out, const int* koffs, int64_t M, int64_t N, int64_t K,
+                                     int64_t pitch_a, int64_t pitch_b, int64_t ntaps, float* scratch, int64_t scratch_elems, void* stream) {
+  if (!At || !Bt || !out || !koffs || M <= 0 || N <= 0 || K <= 0 || ntaps <= 0 || pitch_a < K || pitch_b < K ||
+      (pitch_a % 8) != 0 || (pitch_b % 8) != 0) {
+    set_error("wgrad_splitk_det: bad arguments (M=%lld N=%lld K=%lld pitches %lld %lld taps %lld)", (long long)M, (long long)N,
+              (long long)K, (long long)pitch_a, (long long)pitch_b, (long long)ntaps);
+    return CVIT_ERR_INVALID;
+  }
+  if (int rc = det_check_scratch(scratch, scratch_elems, cvit_wgrad_splitk_det_partials(M, N, K, ntaps), "wgrad_splitk_det")) return rc;
+  if (((reinterpret_cast<uintptr_t>(At) | reinterpret_cast<uintptr_t>(Bt)) & 15u) != 0) {
+    set_error("wgrad_splitk_det: operands must be 16-byte aligned");
+    return CVIT_ERR_INVALID;
+  }
+  int bn, pack, Mp, k_chunks, ksplit;
+  splitk_geometry(M, N, K, ntaps, &bn, &pack, &Mp, &k_chunks, &ksplit);
+  CUtensorMap tmA, tmB;
+  {
+    uint64_t dims[2] = {(uint64_t)K, (uint64_t)M};
+    uint64_t strides[2] = {0, (uint64_t)pitch_a * 2};
+    uint32_t box[2] = {WG_KC, pack > 1 ? (uint32_t)Mp : (uint32_t)WG_BM};
+    int rc = encode_tmap(&tmA, TmapDtype::BF16, 2, At, dims, strides, box, 128);
+    if (rc) return rc;
+  }
+  {
+    uint64_t dims[2] = {(uint64_t)K, (uint64_t)N};
+    uint64_t strides[2] = {0, (uint64_t)pitch_b * 2};
+    uint32_t box[2] = {WG_KC, (uint32_t)bn};
+    int rc = encode_tmap(&tmB, TmapDtype::BF16, 2, Bt, dims, strides, box, 128);
+    if (rc) return rc;
+  }
+  WgArgs a;
+  a.out = scratch;
+  a.koffs = koffs;
+  a.M = (int)M;
+  a.N = (int)N;
+  a.ntaps = (int)ntaps;
+  a.k_chunks = k_chunks;
+  a.pack = pack;
+  a.Mp = Mp;
+  a.ksplit = ksplit;
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc;
+  switch (bn) {
+    case 256: rc = launch_wgrad<256, true>(tmA, tmB, a, st); break;
+    case 192: rc = launch_wgrad<192, true>(tmA, tmB, a, st); break;
+    case 128: rc = launch_wgrad<128, true>(tmA, tmB, a, st); break;
+    case 64: rc = launch_wgrad<64, true>(tmA, tmB, a, st); break;
+    default: rc = launch_wgrad<32, true>(tmA, tmB, a, st); break;
+  }
+  if (rc) return rc;
+  const int64_t n = ntaps * M * N;
+  return det_finalize(scratch, ksplit, n, n, out, true, st);
 }
 
 extern "C" int cvit_wgrad_splitk(const void* At, const void* Bt, float* out, const int* koffs, int64_t M, int64_t N,

@@ -17,6 +17,7 @@
 // of K chunks); items accumulate in TMEM (two buffers) and add their partial tile into the fp32 result with
 // red.global.add (the caller zeroes it). One CTA per SM, 192 threads: TMA producer, MMA issuer (warp-uniform,
 // elect.sync), four epilogue warps (thread = output row).
+#include "det_reduce.cuh"
 #include "ptx.cuh"
 #include "tmap.h"
 
@@ -37,7 +38,7 @@ struct WmCfg {
 };
 
 struct WmArgs {
-  float* out;          // [ntaps][M][N] fp32, accumulated into
+  float* out;          // [ntaps][M][N] fp32, accumulated into (deterministic mode: [ksplit][ntaps][M][N], stored)
   int M, N;            // channels of the A operand / of the B operand
   int D, H, W, dil;    // voxel grid both operands live on (rows mode: W = rows, H = D = 1)
   int BW, BH;          // K chunk = BW x BH voxels of one plane (BW * BH == 64)
@@ -46,9 +47,10 @@ struct WmArgs {
   int ksplit;
 };
 
-template <int BN>
-__global__ void __launch_bounds__(WM_THREADS, 1)
-wgrad_mn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const WmArgs args) {
+// DET (deterministic mode): an item's tile is STORED into K slice ks of the [ksplit][ntaps][M][N] slab (zeros when every
+// chunk was skipped), and det_finalize adds the slices in ks order.
+template <int BN, bool DET>
+__device__ __forceinline__ void wgrad_mn_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const WmArgs& args) {
   using Cfg = WmCfg<BN>;
   constexpr int STAGES = Cfg::STAGES;
   extern __shared__ uint8_t smem_raw[];
@@ -199,12 +201,19 @@ wgrad_mn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       const int row = m0 + r;
       const bool live = any && row < args.M;
       float* orow = args.out + ((size_t)tap * args.M + row) * args.N + n0;
+      if constexpr (DET) orow += (size_t)((item % per_tap) % args.ksplit) * args.ntaps * args.M * args.N;
 #pragma unroll 1
       for (int c0 = 0; c0 < BN; c0 += 32) {
         uint32_t v[32];
         tmem_ld_32x32(t_acc + c0, v);
         tmem_ld_wait();
-        if (live) {
+        if constexpr (DET) {
+          if (row < args.M) {
+#pragma unroll
+            for (int i = 0; i < 32; ++i)
+              if (n0 + c0 + i < args.N) orow[c0 + i] = any ? __uint_as_float(v[i]) : 0.f;
+          }
+        } else if (live) {
 #pragma unroll
           for (int i = 0; i < 32; ++i)
             if (n0 + c0 + i < args.N) atomicAdd(orow + c0 + i, __uint_as_float(v[i]));
@@ -227,9 +236,21 @@ wgrad_mn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
 }
 
 template <int BN>
+__global__ void __launch_bounds__(WM_THREADS, 1)
+wgrad_mn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const WmArgs args) {
+  wgrad_mn_body<BN, false>(tmA, tmB, args);
+}
+
+template <int BN>
+__global__ void __launch_bounds__(WM_THREADS, 1)
+wgrad_mn_det_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const WmArgs args) {
+  wgrad_mn_body<BN, true>(tmA, tmB, args);
+}
+
+template <int BN, bool DET>
 static int launch_wgrad_mn(const CUtensorMap& tmA, const CUtensorMap& tmB, const WmArgs& a, cudaStream_t st) {
   using Cfg = WmCfg<BN>;
-  auto kern = wgrad_mn_kernel<BN>;
+  auto kern = DET ? wgrad_mn_det_kernel<BN> : wgrad_mn_kernel<BN>;
   static bool configured = false;
   if (!configured) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM);
@@ -244,12 +265,29 @@ static int launch_wgrad_mn(const CUtensorMap& tmA, const CUtensorMap& tmB, const
   int grid = num_sms();
   if (grid > items) grid = items;
   kern<<<grid, WM_THREADS, Cfg::SMEM, st>>>(tmA, tmB, a);
-  return check_launch("wgrad_mn_kernel");
+  return check_launch(DET ? "wgrad_mn_det_kernel" : "wgrad_mn_kernel");
 }
 
 }  // namespace cvit
 
 using namespace cvit;
+
+// The K split of a launch: enough K ranges for ~4 items per SM, but never K ranges shorter than 32 chunks (2048 reduction steps)
+static int64_t wgrad_mn_ksplit(int64_t D, int64_t H, int64_t W, int64_t Ca, int64_t Cb, int64_t ntaps, int* BW_out, int* bn_out) {
+  int BW = 8;
+  while (BW < W && BW < 64) BW <<= 1;
+  const int BH = 64 / BW;
+  const int bn = Cb > 192 ? 256 : Cb > 128 ? 192 : Cb > 64 ? 128 : 64;
+  const int64_t k_chunks = D * ((H + BH - 1) / BH) * ((W + BW - 1) / BW);
+  const int64_t tiles = ntaps * ((Ca + WM_BM - 1) / WM_BM) * ((Cb + bn - 1) / bn);
+  int64_t ksplit = (4 * (int64_t)num_sms() + tiles - 1) / tiles;
+  const int64_t max_split = k_chunks / 32 > 0 ? k_chunks / 32 : 1;
+  if (ksplit > max_split) ksplit = max_split;
+  if (ksplit < 1) ksplit = 1;
+  if (BW_out) *BW_out = BW;
+  if (bn_out) *bn_out = bn;
+  return ksplit;
+}
 
 // See include/cryovit_b200.h.
 extern "C" int cvit_wgrad_mn_ndhwc(const void* a, const void* b, float* out, int64_t D, int64_t H, int64_t W, int64_t Ca, int64_t Cb,
@@ -304,9 +342,72 @@ extern "C" int cvit_wgrad_mn_ndhwc(const void* a, const void* b, float* out, int
   args.ksplit = (int)ksplit;
   cudaStream_t st = (cudaStream_t)stream;
   switch (bn) {
-    case 256: return launch_wgrad_mn<256>(tmA, tmB, args, st);
-    case 192: return launch_wgrad_mn<192>(tmA, tmB, args, st);
-    case 128: return launch_wgrad_mn<128>(tmA, tmB, args, st);
-    default: return launch_wgrad_mn<64>(tmA, tmB, args, st);
+    case 256: return launch_wgrad_mn<256, false>(tmA, tmB, args, st);
+    case 192: return launch_wgrad_mn<192, false>(tmA, tmB, args, st);
+    case 128: return launch_wgrad_mn<128, false>(tmA, tmB, args, st);
+    default: return launch_wgrad_mn<64, false>(tmA, tmB, args, st);
   }
+}
+
+// Deterministic mode: the same GEMM with every item's tile stored into its K slice of scratch ([ksplit][ntaps][Ca][Cb] fp32,
+// cvit_wgrad_mn_ndhwc_det_partials floats), then out += the slices added in K order.
+extern "C" int64_t cvit_wgrad_mn_ndhwc_det_partials(int64_t D, int64_t H, int64_t W, int64_t Ca, int64_t Cb, int64_t ntaps) {
+  if (D <= 0 || H <= 0 || W <= 0 || Ca <= 0 || Cb <= 0 || ntaps <= 0) return 0;
+  return wgrad_mn_ksplit(D, H, W, Ca, Cb, ntaps, nullptr, nullptr) * ntaps * Ca * Cb;
+}
+
+extern "C" int cvit_wgrad_mn_ndhwc_det(const void* a, const void* b, float* out, int64_t D, int64_t H, int64_t W, int64_t Ca, int64_t Cb,
+                                       int64_t dil, int64_t ntaps, int shift_a, float* scratch, int64_t scratch_elems, void* stream) {
+  if (!a || !b || !out || D <= 0 || H <= 0 || W <= 0 || Ca <= 0 || Cb <= 0 || dil <= 0 || (ntaps != 1 && ntaps != 27) ||
+      (Ca % 8) != 0 || (Cb % 8) != 0 || Ca < 64 || Cb < 64) {
+    set_error("wgrad_mn_det: bad arguments (D=%lld H=%lld W=%lld Ca=%lld Cb=%lld dil=%lld taps=%lld): channels >= 64, multiples of 8",
+              (long long)D, (long long)H, (long long)W, (long long)Ca, (long long)Cb, (long long)dil, (long long)ntaps);
+    return CVIT_ERR_INVALID;
+  }
+  if (int rc = det_check_scratch(scratch, scratch_elems, cvit_wgrad_mn_ndhwc_det_partials(D, H, W, Ca, Cb, ntaps), "wgrad_mn_det")) return rc;
+  if (((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b)) & 15u) != 0) {
+    set_error("wgrad_mn_det: operands must be 16-byte aligned");
+    return CVIT_ERR_INVALID;
+  }
+  int BW, bn;
+  const int64_t ksplit = wgrad_mn_ksplit(D, H, W, Ca, Cb, ntaps, &BW, &bn);
+  WmArgs args;
+  args.out = scratch;
+  args.M = (int)Ca;
+  args.N = (int)Cb;
+  args.D = (int)D;
+  args.H = (int)H;
+  args.W = (int)W;
+  args.dil = (int)dil;
+  args.ntaps = (int)ntaps;
+  args.shift_a = shift_a ? 1 : 0;
+  args.BW = BW;
+  args.BH = 64 / BW;
+  args.ksplit = (int)ksplit;
+  CUtensorMap tmA, tmB;
+  {
+    uint64_t dims[4] = {(uint64_t)Ca, (uint64_t)W, (uint64_t)H, (uint64_t)D};
+    uint64_t strides[4] = {0, (uint64_t)Ca * 2, (uint64_t)W * Ca * 2, (uint64_t)H * W * Ca * 2};
+    uint32_t box[4] = {64, (uint32_t)args.BW, (uint32_t)args.BH, 1};
+    int rc = encode_tmap(&tmA, TmapDtype::BF16, 4, a, dims, strides, box, 128);
+    if (rc) return rc;
+  }
+  {
+    uint64_t dims[4] = {(uint64_t)Cb, (uint64_t)W, (uint64_t)H, (uint64_t)D};
+    uint64_t strides[4] = {0, (uint64_t)Cb * 2, (uint64_t)W * Cb * 2, (uint64_t)H * W * Cb * 2};
+    uint32_t box[4] = {64, (uint32_t)args.BW, (uint32_t)args.BH, 1};
+    int rc = encode_tmap(&tmB, TmapDtype::BF16, 4, b, dims, strides, box, 128);
+    if (rc) return rc;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc;
+  switch (bn) {
+    case 256: rc = launch_wgrad_mn<256, true>(tmA, tmB, args, st); break;
+    case 192: rc = launch_wgrad_mn<192, true>(tmA, tmB, args, st); break;
+    case 128: rc = launch_wgrad_mn<128, true>(tmA, tmB, args, st); break;
+    default: rc = launch_wgrad_mn<64, true>(tmA, tmB, args, st); break;
+  }
+  if (rc) return rc;
+  const int64_t n = ntaps * Ca * Cb;
+  return det_finalize(scratch, ksplit, n, n, out, true, st);
 }

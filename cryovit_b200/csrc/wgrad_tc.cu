@@ -26,6 +26,7 @@
 // One CTA per SM, 192 threads: warp 0 TMA producer, warp 1 MMA issuer + TMEM owner, warp 4 the final read-out.
 #include <cstdlib>
 
+#include "det_reduce.cuh"
 #include "ptx.cuh"
 #include "tmap.h"
 
@@ -50,7 +51,8 @@ constexpr int WT_N = 80, WT_TMEM_COLS = 128;
 constexpr uint32_t WT_TX_BYTES = WT_R * WT_XARR + (WT_R + 2) * 3 * WT_ZARR;
 
 struct WtArgs {
-  float* dw;  // [27][Cout][Cin] fp32, accumulated into (tap = (kd*3+kh)*3+kw, then co, then ci)
+  float* dw;  // [27][Cout][Cin] fp32, accumulated into (tap = (kd*3+kh)*3+kw, then co, then ci); deterministic mode:
+              // [gridDim.x][27][Cout][Cin], one row per CTA, stored
   const __nv_bfloat16* x;   // [D, H, W, Cin]  (read directly by the cp.async loaders of the 16 / 32-channel kernel)
   const __nv_bfloat16* dz;  // [D, H, W, Cout]
   int D, H, W, dil;
@@ -66,8 +68,11 @@ __device__ __forceinline__ uint64_t wt_desc(uint32_t addr, uint32_t lbo, uint32_
          (static_cast<uint64_t>(sbo >> 4) << 32) | (1ull << 46);
 }
 
-__global__ void __launch_bounds__(WT_THREADS, 1)
-wgrad_tc8_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmZ, const WtArgs args) {
+// DET (deterministic mode): the CTA's accumulator is STORED into its own row of the dw slab (every one of the 27 x 8 x 8 entries
+// is written once); det_finalize adds the rows in CTA order. A CTA's blocks are blockIdx.x + k gridDim.x, so a row's content
+// depends on the grid size only.
+template <bool DET>
+__device__ __forceinline__ void wgrad_tc8_body(const CUtensorMap& tmX, const CUtensorMap& tmZ, const WtArgs& args) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t sBar = smem_base + WT_STAGES * WT_STAGE;
@@ -157,7 +162,10 @@ wgrad_tc8_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant_
             const int n = c * 16 + i;
             if (n < 72) {
               const int co = n & 7, blkn = n >> 3, yr = blkn / 3, kd = blkn - 3 * yr, kh = 2 - yr;
-              atomicAdd(args.dw + ((((kd * 3 + kh) * 3 + kw) * 8 + co) * 8 + ci), __uint_as_float(v[i]));
+              if constexpr (DET)
+                args.dw[(size_t)blockIdx.x * 27 * 64 + (((kd * 3 + kh) * 3 + kw) * 8 + co) * 8 + ci] = __uint_as_float(v[i]);
+              else
+                atomicAdd(args.dw + ((((kd * 3 + kh) * 3 + kw) * 8 + co) * 8 + ci), __uint_as_float(v[i]));
             }
           }
         }
@@ -173,6 +181,16 @@ wgrad_tc8_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant_
     tcgen05_fence_after();
     tmem_dealloc<WT_TMEM_COLS>(tmem_base);
   }
+}
+
+__global__ void __launch_bounds__(WT_THREADS, 1)
+wgrad_tc8_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmZ, const WtArgs args) {
+  wgrad_tc8_body<false>(tmX, tmZ, args);
+}
+
+__global__ void __launch_bounds__(WT_THREADS, 1)
+wgrad_tc8_det_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmZ, const WtArgs args) {
+  wgrad_tc8_body<true>(tmX, tmZ, args);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -458,9 +476,9 @@ struct WtsCfg {
   static_assert(16 <= XA - 3 * NCX * (R - 1) + ZA, "M = 128 over-reads 16 arrays from the last row's first");
 };
 
-template <int CIN, int COUT, int R, int KSEG, int RS>
-__global__ void __launch_bounds__(WT_THREADS, 1)
-wgrad_tcs_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmZ, const WtArgs args) {
+// DET: as wgrad_tc8_body, one [27][COUT][CIN] row per CTA.
+template <int CIN, int COUT, int R, int KSEG, int RS, bool DET>
+__device__ __forceinline__ void wgrad_tcs_body(const CUtensorMap& tmX, const CUtensorMap& tmZ, const WtArgs& args) {
   using Cfg = WtsCfg<CIN, COUT, R, KSEG, RS>;
   constexpr int S = Cfg::S, NCX = Cfg::NCX, NCZ = Cfg::NCZ;
   extern __shared__ uint8_t smem_raw[];
@@ -610,8 +628,14 @@ wgrad_tcs_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant_
             const int c = 2 * c2 + hb;
             const int jz = c % NCZ, rest = c / NCZ, yr = rest / 3, kd = rest - 3 * yr, kh = 2 - yr;
             float* dst = args.dw + ((size_t)(((kd * 3 + kh) * 3 + kw) * COUT + jz * 8) * CIN + ci);
+            if constexpr (DET) {
+              dst += (size_t)blockIdx.x * 27 * COUT * CIN;
 #pragma unroll
-            for (int i = 0; i < 8; ++i) atomicAdd(dst + (size_t)i * CIN, __uint_as_float(v[hb * 8 + i]));
+              for (int i = 0; i < 8; ++i) dst[(size_t)i * CIN] = __uint_as_float(v[hb * 8 + i]);
+            } else {
+#pragma unroll
+              for (int i = 0; i < 8; ++i) atomicAdd(dst + (size_t)i * CIN, __uint_as_float(v[hb * 8 + i]));
+            }
           }
         }
       }
@@ -629,7 +653,29 @@ wgrad_tcs_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant_
 }
 
 template <int CIN, int COUT, int R, int KSEG, int RS>
-static int launch_wgrad_tcs(const void* x, const void* dz, float* dw, int64_t D, int64_t H, int64_t W, int64_t dil, cudaStream_t stream) {
+__global__ void __launch_bounds__(WT_THREADS, 1)
+wgrad_tcs_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmZ, const WtArgs args) {
+  wgrad_tcs_body<CIN, COUT, R, KSEG, RS, false>(tmX, tmZ, args);
+}
+
+template <int CIN, int COUT, int R, int KSEG, int RS>
+__global__ void __launch_bounds__(WT_THREADS, 1)
+wgrad_tcs_det_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmZ, const WtArgs args) {
+  wgrad_tcs_body<CIN, COUT, R, KSEG, RS, true>(tmX, tmZ, args);
+}
+
+// Grid of the 16 / 32-channel kernels and of wgrad_tc8: one CTA per SM, at most one per block of rows.
+static int wgrad_tc_grid(int64_t D, int64_t H, int64_t W, int R, int KSEG) {
+  const int64_t blocks = D * ((H + R - 1) / R) * ((W + KSEG - 1) / KSEG);
+  int grid = num_sms();
+  if (grid > blocks) grid = (int)blocks;
+  return grid;
+}
+
+// det_slab != null: deterministic mode, dw += the rows of det_slab ([grid][27][COUT][CIN]) added in CTA order.
+template <int CIN, int COUT, int R, int KSEG, int RS>
+static int launch_wgrad_tcs(const void* x, const void* dz, float* dw, int64_t D, int64_t H, int64_t W, int64_t dil, cudaStream_t stream,
+                            float* det_slab = nullptr) {
   using Cfg = WtsCfg<CIN, COUT, R, KSEG, RS>;
   CUtensorMap tmX, tmZ;
   uint64_t dimsX[4] = {(uint64_t)CIN, (uint64_t)W, (uint64_t)H, (uint64_t)D};
@@ -641,21 +687,21 @@ static int launch_wgrad_tcs(const void* x, const void* dz, float* dw, int64_t D,
   if (rc) return rc;
   rc = encode_tmap(&tmZ, TmapDtype::BF16, 4, dz, dimsZ, strZ, boxZ, 0);
   if (rc) return rc;
-  auto kern = wgrad_tcs_kernel<CIN, COUT, R, KSEG, RS>;
-  static bool configured = false;
-  if (!configured) {
+  auto kern = det_slab ? wgrad_tcs_det_kernel<CIN, COUT, R, KSEG, RS> : wgrad_tcs_kernel<CIN, COUT, R, KSEG, RS>;
+  static bool configured[2] = {false, false};
+  if (!configured[det_slab != nullptr]) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM);
     if (e != cudaSuccess) {
       set_error("wgrad_tcs: cudaFuncSetAttribute(smem=%d): %s", Cfg::SMEM, cudaGetErrorString(e));
       return CVIT_ERR_CUDA;
     }
-    configured = true;
+    configured[det_slab != nullptr] = true;
   }
   const int64_t blocks = D * ((H + R - 1) / R) * ((W + KSEG - 1) / KSEG);
   int grid = num_sms();
   if (grid > blocks) grid = (int)blocks;
   WtArgs a;
-  a.dw = dw;
+  a.dw = det_slab ? det_slab : dw;
   a.x = static_cast<const __nv_bfloat16*>(x);
   a.dz = static_cast<const __nv_bfloat16*>(dz);
   a.D = (int)D;
@@ -663,7 +709,9 @@ static int launch_wgrad_tcs(const void* x, const void* dz, float* dw, int64_t D,
   a.W = (int)W;
   a.dil = (int)dil;
   kern<<<grid, WT_THREADS, Cfg::SMEM, stream>>>(tmX, tmZ, a);
-  return check_launch("wgrad_tcs_kernel");
+  if (!det_slab) return check_launch("wgrad_tcs_kernel");
+  if (int rc = check_launch("wgrad_tcs_det_kernel")) return rc;
+  return det_finalize(det_slab, grid, 27 * COUT * CIN, 27 * COUT * CIN, dw, true, stream);
 }
 
 }  // namespace cvit
@@ -672,8 +720,30 @@ using namespace cvit;
 
 // dw (fp32 [27][8][8], tap = (kd*3+kh)*3+kw, then co, then ci) += weight gradient of an 8 -> 8 channel 3x3x3 depth-dilated
 // "same" convolution: x the forward input, dz the output gradient, both bf16 [D,H,W,8], W a multiple of 8.
+static int wgrad_tc8_run(const void* x, const void* dz, float* dw, int64_t D, int64_t H, int64_t W, int64_t dil, void* stream,
+                         float* det_slab);
+
 extern "C" int cvit_wgrad_tc8_ndhwc(const void* x, const void* dz, float* dw, int64_t D, int64_t H, int64_t W, int64_t dil,
                                     void* stream) {
+  return wgrad_tc8_run(x, dz, dw, D, H, W, dil, stream, nullptr);
+}
+
+// Deterministic mode (see wgrad_tc8_body): scratch holds cvit_wgrad_tc8_ndhwc_det_partials(D, H, W) floats, one [27][8][8] row per
+// CTA; dw += the rows added in CTA order.
+extern "C" int64_t cvit_wgrad_tc8_ndhwc_det_partials(int64_t D, int64_t H, int64_t W) {
+  return D > 0 && H > 0 && W > 0 ? (int64_t)wgrad_tc_grid(D, H, W, WT_R, WT_KSEG) * 27 * 64 : 0;
+}
+
+extern "C" int cvit_wgrad_tc8_ndhwc_det(const void* x, const void* dz, float* dw, int64_t D, int64_t H, int64_t W, int64_t dil,
+                                        float* scratch, int64_t scratch_elems, void* stream) {
+  if (D > 0 && H > 0 && W > 0) {
+    if (int rc = det_check_scratch(scratch, scratch_elems, cvit_wgrad_tc8_ndhwc_det_partials(D, H, W), "wgrad_tc8_det")) return rc;
+  }
+  return wgrad_tc8_run(x, dz, dw, D, H, W, dil, stream, scratch);
+}
+
+static int wgrad_tc8_run(const void* x, const void* dz, float* dw, int64_t D, int64_t H, int64_t W, int64_t dil, void* stream,
+                         float* det_slab) {
   if (!x || !dz || !dw || D <= 0 || H <= 0 || W <= 0 || dil <= 0) {
     set_error("wgrad_tc8: bad arguments (D=%lld H=%lld W=%lld dil=%lld)", (long long)D, (long long)H, (long long)W, (long long)dil);
     return CVIT_ERR_INVALID;
@@ -698,25 +768,29 @@ extern "C" int cvit_wgrad_tc8_ndhwc(const void* x, const void* dz, float* dw, in
   static bool configured = false;
   if (!configured) {
     cudaError_t e = cudaFuncSetAttribute(wgrad_tc8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, WT_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(wgrad_tc8_det_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, WT_SMEM);
     if (e != cudaSuccess) {
       set_error("wgrad_tc8: cudaFuncSetAttribute(smem=%d): %s", WT_SMEM, cudaGetErrorString(e));
       return CVIT_ERR_CUDA;
     }
     configured = true;
   }
-  const int64_t blocks = D * ((H + WT_R - 1) / WT_R) * ((W + WT_KSEG - 1) / WT_KSEG);
-  int grid = num_sms();
-  if (grid > blocks) grid = (int)blocks;
+  const int grid = wgrad_tc_grid(D, H, W, WT_R, WT_KSEG);
   WtArgs a;
-  a.dw = dw;
+  a.dw = det_slab ? det_slab : dw;
   a.x = static_cast<const __nv_bfloat16*>(x);
   a.dz = static_cast<const __nv_bfloat16*>(dz);
   a.D = (int)D;
   a.H = (int)H;
   a.W = (int)W;
   a.dil = (int)dil;
-  wgrad_tc8_kernel<<<grid, WT_THREADS, WT_SMEM, (cudaStream_t)stream>>>(tmX, tmZ, a);
-  return check_launch("wgrad_tc8_kernel");
+  if (!det_slab) {
+    wgrad_tc8_kernel<<<grid, WT_THREADS, WT_SMEM, (cudaStream_t)stream>>>(tmX, tmZ, a);
+    return check_launch("wgrad_tc8_kernel");
+  }
+  wgrad_tc8_det_kernel<<<grid, WT_THREADS, WT_SMEM, (cudaStream_t)stream>>>(tmX, tmZ, a);
+  if (int rc = check_launch("wgrad_tc8_det_kernel")) return rc;
+  return det_finalize(det_slab, grid, 27 * 64, 27 * 64, dw, true, (cudaStream_t)stream);
 }
 
 // The 16- / 32-channel layers (SynthesisBlocks 3-4): (Cin, Cout) in {(16,16), (32,16), (32,32)}, any W. Same contract as
@@ -743,5 +817,35 @@ extern "C" int cvit_wgrad_tcn_ndhwc(const void* x, const void* dz, float* dw, in
   if (Cin == 32 && Cout == 16) return launch_wgrad_tcn<32, 16, 4, 64>(x, dz, dw, D, H, W, dil, st);
   if (Cin == 32 && Cout == 32) return launch_wgrad_tcn<32, 32, 2, 64>(x, dz, dw, D, H, W, dil, st);
   set_error("wgrad_tcn: (Cin, Cout) = (%lld, %lld) unsupported: (16,16), (32,16), (32,32)", (long long)Cin, (long long)Cout);
+  return CVIT_ERR_UNSUPPORTED;
+}
+
+// Deterministic mode of cvit_wgrad_tcn_ndhwc: always the whole-row kernel (wgrad_tcs_body), one [27][Cout][Cin] row per CTA in
+// scratch (cvit_wgrad_tcn_ndhwc_det_partials floats), dw += the rows added in CTA order.
+extern "C" int64_t cvit_wgrad_tcn_ndhwc_det_partials(int64_t D, int64_t H, int64_t W, int64_t Cin, int64_t Cout) {
+  if (D <= 0 || H <= 0 || W <= 0) return 0;
+  int grid = 0;
+  if (Cin == 16 && Cout == 16) grid = wgrad_tc_grid(D, H, W, 4, 64);
+  else if (Cin == 32 && Cout == 16) grid = wgrad_tc_grid(D, H, W, 2, 64);
+  else if (Cin == 32 && Cout == 32) grid = wgrad_tc_grid(D, H, W, 2, 32);
+  return (int64_t)grid * 27 * Cin * Cout;
+}
+
+extern "C" int cvit_wgrad_tcn_ndhwc_det(const void* x, const void* dz, float* dw, int64_t D, int64_t H, int64_t W, int64_t Cin,
+                                        int64_t Cout, int64_t dil, float* scratch, int64_t scratch_elems, void* stream) {
+  if (!x || !dz || !dw || D <= 0 || H <= 0 || W <= 0 || dil <= 0) {
+    set_error("wgrad_tcn_det: bad arguments (D=%lld H=%lld W=%lld dil=%lld)", (long long)D, (long long)H, (long long)W, (long long)dil);
+    return CVIT_ERR_INVALID;
+  }
+  if (int rc = det_check_scratch(scratch, scratch_elems, cvit_wgrad_tcn_ndhwc_det_partials(D, H, W, Cin, Cout), "wgrad_tcn_det")) return rc;
+  if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dz)) & 15u) {
+    set_error("wgrad_tcn_det: x and dz must be 16-byte aligned");
+    return CVIT_ERR_INVALID;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  if (Cin == 16 && Cout == 16) return launch_wgrad_tcs<16, 16, 4, 64, 2>(x, dz, dw, D, H, W, dil, st, scratch);
+  if (Cin == 32 && Cout == 16) return launch_wgrad_tcs<32, 16, 2, 64, 3>(x, dz, dw, D, H, W, dil, st, scratch);
+  if (Cin == 32 && Cout == 32) return launch_wgrad_tcs<32, 32, 2, 32, 5>(x, dz, dw, D, H, W, dil, st, scratch);
+  set_error("wgrad_tcn_det: (Cin, Cout) = (%lld, %lld) unsupported: (16,16), (32,16), (32,32)", (long long)Cin, (long long)Cout);
   return CVIT_ERR_UNSUPPORTED;
 }

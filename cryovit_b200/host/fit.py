@@ -46,7 +46,7 @@ def _append_row(path: Path, row: dict, first: bool) -> None:
 def fit_head(dataset: TomoDataset, in_channels: int = 1536, max_epochs: int = 50, lr: float = 1e-4, weight_decay: float = 1e-3,
              swa_epoch_start: int | None = 40, seed: int = 42, exp_dir: Path | str | None = None, state_dict: dict | None = None,
              log_every: int = 10, cache_gb: float | None = None, epoch_seconds: list | None = None, validator=None,
-             val_history: list | None = None) -> dict[str, torch.Tensor]:
+             val_history: list | None = None, deterministic: bool | str = False) -> dict[str, torch.Tensor]:
     """Trains on the items of ``dataset`` (``train=True`` gives the reference's random 128 x 32 x 32 feature crops);
     with several ranks (torchrun) every rank walks its own round-robin share of a common shuffled order and the
     gradients are averaged over the ranks each step. Returns the final (SWA-averaged if enabled) state dict.
@@ -59,14 +59,40 @@ def fit_head(dataset: TomoDataset, in_channels: int = 1536, max_epochs: int = 50
     ``validator`` (a :class:`~cryovit_b200.host.validate.Validator`): after the training steps of every epoch it schedules,
     the validation tomograms are scored with the current (not SWA-averaged) weights, as Lightning's ``fit`` does. Its
     resident tomograms share the HBM budget, after the training set's. Rank 0 appends a row per validated epoch to
-    ``<exp_dir>/validation.csv``; ``val_history`` (a list) receives the same rows as dicts."""
+    ``<exp_dir>/validation.csv``; ``val_history`` (a list) receives the same rows as dicts.
+
+    ``deterministic`` (Lightning's ``trainer.deterministic``: False, True or ``"warn"``): the training step runs its fixed-order
+    reductions (``CryoVITHeadTrainerB200(deterministic=True)``), so a run with the same seed, data and build on the same GPU
+    model and world size gives bit-identical weights, losses and validation metrics. As Lightning does, torch's
+    ``use_deterministic_algorithms`` is set for the duration (warn-only with ``"warn"``) and restored on exit."""
+    if deterministic not in (False, True, "warn"):
+        raise ValueError(f"deterministic={deterministic!r}: expected False, True or 'warn'")
+    if not deterministic:
+        return _fit_head(dataset, in_channels, max_epochs, lr, weight_decay, swa_epoch_start, seed, exp_dir, state_dict, log_every,
+                         cache_gb, epoch_seconds, validator, val_history, False)
+    prev = (torch.are_deterministic_algorithms_enabled(), torch.is_deterministic_algorithms_warn_only_enabled())
+    torch.use_deterministic_algorithms(True, warn_only=deterministic == "warn")
+    try:
+        return _fit_head(dataset, in_channels, max_epochs, lr, weight_decay, swa_epoch_start, seed, exp_dir, state_dict, log_every,
+                         cache_gb, epoch_seconds, validator, val_history, True)
+    finally:
+        torch.use_deterministic_algorithms(prev[0], warn_only=prev[1])
+
+
+def _fit_head(dataset, in_channels, max_epochs, lr, weight_decay, swa_epoch_start, seed, exp_dir, state_dict, log_every, cache_gb,
+              epoch_seconds, validator, val_history, deterministic: bool) -> dict[str, torch.Tensor]:
     rank, world = rank_world()
     require_process_group("fit_head")  # the data is sharded by rank below: the gradients must really be exchanged
     torch.manual_seed(seed)
     np.random.seed(seed + rank)  # crops differ per rank, the shuffled ORDER (below) does not
     # the initial weights follow the seed (the reference's seed_everything(cfg.random_seed)) and are identical on
     # every rank
-    trainer = CryoVITHeadTrainerB200(in_channels, lr=lr, weight_decay=weight_decay, state_dict=state_dict, seed=seed)
+    # the default mode constructs the trainer exactly as before the switch existed
+    mode = {"deterministic": True} if deterministic else {}
+    trainer = CryoVITHeadTrainerB200(in_channels, lr=lr, weight_decay=weight_decay, state_dict=state_dict, seed=seed, **mode)
+    if deterministic and rank == 0:
+        logging.info("deterministic training: fixed-order reductions in every kernel of the step (bit-reproducible for this "
+                     "seed, GPU model and world size of %d)", world)
     order_rng = np.random.default_rng(seed)
     swa_avg, swa_n = None, 0
     step = 0

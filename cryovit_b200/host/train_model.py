@@ -64,6 +64,17 @@ def build_validator(cfg, datamodule, in_channels: int) -> Validator | None:
     return v
 
 
+def deterministic_setting(cfg) -> bool | str:
+    """Lightning's ``trainer.deterministic`` (added with ``+trainer.deterministic=...``): None / False -> False, True -> True,
+    "warn" -> "warn" (deterministic, torch in warn-only mode). Anything else is an error, as in Lightning."""
+    v = cfg.trainer.get("deterministic")
+    if v is None or v is False:
+        return False
+    if v is True or v == "warn":
+        return v
+    raise ValueError(f"trainer.deterministic={v!r}: expected true, false or 'warn'")
+
+
 def run_trainer(cfg) -> Path:
     """train_model.py:206-312. Returns the path of the saved ``weights.pt``. Under torchrun every rank binds its own
     GPU and joins one NCCL group for the gradient all-reduce (Lightning's DDP strategy in the reference)."""
@@ -100,10 +111,11 @@ def _run_trainer(cfg) -> Path:
         else:
             raise ValueError(f"Unsupported checkpoint format: {Path(ckpt).suffix}. Use .pt or .model files.")
     in_channels = int(cfg.model.get("in_channels", 1536))
+    deterministic = deterministic_setting(cfg)
     validator = build_validator(cfg, datamodule, in_channels)
     logging.info("Starting training.")
     fit_head(dataset, in_channels=in_channels, max_epochs=max_epochs, lr=float(cfg.model.lr),
              weight_decay=float(cfg.model.get("weight_decay", 1e-3)), swa_epoch_start=swa_start, seed=int(cfg.random_seed),
-             exp_dir=cfg.paths.exp_dir, state_dict=state, validator=validator)
+             exp_dir=cfg.paths.exp_dir, state_dict=state, validator=validator, deterministic=deterministic)
     logging.info("Saving model.")
     return cfg.paths.exp_dir / "weights.pt"

@@ -273,9 +273,22 @@ def features_to_ndhwc(features: torch.Tensor, out: torch.Tensor) -> None:
     _lib.call("cvit_features_to_ndhwc_bf16", _chk(features, F16, "features"), _chk(out, BF16, "out"), C, DHW, _stream())
 
 
-def groupnorm_ndhwc(x, out, gamma, beta, stats, groups: int, eps: float) -> None:
+def det_scratch(det, name: str, n: int, dtype=F32) -> tuple[int, int]:
+    """(pointer, elements) of the deterministic-mode scratch ``det(n, dtype)`` (a callable returning a CUDA tensor of at least
+    n elements: the trainer's keep-alive pool). The C entry points refuse a smaller one."""
+    t = det(int(n), dtype)
+    return _chk(t, dtype, name), t.numel()
+
+
+def groupnorm_ndhwc(x, out, gamma, beta, stats, groups: int, eps: float, det=None) -> None:
+    """``det``: deterministic mode (a scratch provider, see det_scratch): the statistics are summed in a fixed order."""
     C = x.shape[-1]
     DHW = x.numel() // C
+    if det is not None:
+        sp, sn = det_scratch(det, "scratch", _lib.load().cvit_groupnorm_ndhwc_bf16_det_partials(DHW, C, groups))
+        _lib.call("cvit_groupnorm_ndhwc_bf16_det", _chk(x, BF16, "x"), _chk(out, BF16, "out"), _chk(gamma, F32, "gamma"),
+                  _chk(beta, F32, "beta"), _chk(stats, F32, "stats"), DHW, C, groups, float(eps), sp, sn, _stream())
+        return
     _lib.call("cvit_groupnorm_ndhwc_bf16", _chk(x, BF16, "x"), _chk(out, BF16, "out"), _chk(gamma, F32, "gamma"),
               _chk(beta, F32, "beta"), _chk(stats, F32, "stats"), DHW, C, groups, float(eps), _stream())
 
@@ -398,8 +411,15 @@ def head_out_conv(x, w2, b2, logits=None, probs=None) -> None:
               _chk(probs, F32, "probs") if probs is not None else None, D, H, W, _stream())
 
 
-def seg_stats(probs: torch.Tensor, labels: torch.Tensor, threshold: float = 0.5) -> torch.Tensor:
-    """Masked (label > -1) reductions behind DiceLoss / DiceMetric / F1Metric, fp64 [8] on the device (see the header)."""
+def seg_stats(probs: torch.Tensor, labels: torch.Tensor, threshold: float = 0.5, det=None) -> torch.Tensor:
+    """Masked (label > -1) reductions behind DiceLoss / DiceMetric / F1Metric, fp64 [8] on the device (see the header).
+    ``det``: deterministic mode (a scratch provider, see det_scratch): per-block rows added in a fixed order."""
+    if det is not None:
+        out = torch.empty(8, device=probs.device, dtype=torch.float64)
+        sp, sn = det_scratch(det, "scratch", _lib.load().cvit_seg_stats_det_partials(probs.numel()), torch.float64)
+        _lib.call("cvit_seg_stats_det", _chk(probs, F32, "probs"), _chk(labels, F32, "labels"), probs.numel(), float(threshold),
+                  out.data_ptr(), sp, sn, _stream())
+        return out
     out = torch.zeros(8, device=probs.device, dtype=torch.float64)
     _lib.call("cvit_seg_stats", _chk(probs, F32, "probs"), _chk(labels, F32, "labels"), probs.numel(), float(threshold),
               out.data_ptr(), _stream())

@@ -167,7 +167,11 @@ class CryoVITHeadTrainerB200:
     """Data-parallel trainer of the CryoVIT head: one process per GPU, one tomogram crop per process and step."""
 
     def __init__(self, in_channels: int = 1536, lr: float = 1e-4, weight_decay: float = 1e-3, betas=(0.9, 0.999),
-                 eps: float = 1e-8, state_dict: dict | None = None, device=None, seed: int = 0):
+                 eps: float = 1e-8, state_dict: dict | None = None, device=None, seed: int = 0, deterministic: bool = False):
+        """deterministic: every reduction of the step that the default kernels finish with float atomics runs as its
+        fixed-order variant (per-block partial rows in scratch of the keep-alive pool, added in an order that depends on the
+        shapes and the SM count only), so two trainers with the same seed and inputs give bit-identical gradients, losses
+        and weights on one GPU. Switches that select a kernel without such a variant are refused."""
         if not torch.cuda.is_available():
             raise CryovitB200Error("no CUDA device: the B200 training path has no CPU fallback")
         self.device = torch.device("cuda", torch.cuda.current_device() if device is None else device)
@@ -189,6 +193,15 @@ class CryoVITHeadTrainerB200:
         self.fuse_dgrad_gelu = os.environ.get("CVIT_TRAIN_FUSE_DGRAD_GELU", "0") != "0"
         self.rows8 = os.environ.get("CVIT_HEAD_ROWS8", "1") != "0"  # 8-channel full-resolution convolutions on conv_rows8.cu
         self.rowsn = os.environ.get("CVIT_HEAD_ROWSN", "1") != "0"  # 16 / 32-channel convolutions on conv_rows.cu
+        self.deterministic = bool(deterministic)
+        if self.deterministic:
+            if self.fuse_dgrad_gelu:
+                raise CryovitB200Error("deterministic mode: CVIT_TRAIN_FUSE_DGRAD_GELU=1 sums bias gradients with atomics inside the "
+                                       "convolution epilogues; unset it or turn deterministic mode off")
+            off = T.narrow_wgrad_switches_off()
+            if off:
+                raise CryovitB200Error(f"deterministic mode: {'=0, '.join(off)}=0 selects the atomic cvit_wgrad_narrow_ndhwc kernel; "
+                                       "unset it or turn deterministic mode off")
         if state_dict is None:
             from .host.models import default_state_dict
 
@@ -216,6 +229,8 @@ class CryoVITHeadTrainerB200:
         self._gather = OperandGather(self._flat_store, self._retired)  # bf16 operand images of the weights (_pk)
         self._bufs: dict = _KeepAlivePool(self._retired)
         self._bufs["wgrad_pool"] = _KeepAlivePool(self._retired)
+        # the scratch provider of the deterministic kernel variants (train_ops ``det``), None in the default mode
+        self._det = self._det_scratch if self.deterministic else None
         self._graphs: dict = {}
         self._graph_broken = False
 
@@ -258,10 +273,15 @@ class CryoVITHeadTrainerB200:
             self._bufs[name] = b
         return b[:n].view(shape)
 
+    def _det_scratch(self, n: int, dtype=F32) -> torch.Tensor:
+        """Scratch of the deterministic kernel variants: one buffer per dtype, grown to the largest request and kept alive
+        (``_bufs``), so every captured graph's pointers stay valid. Launches are stream-ordered, so the sites share it."""
+        return self._buf(f"det_scratch_{str(dtype).split('.')[-1]}", (max(int(n), 1),), dtype)
+
     def _gelu_bwd_bias(self, da, z, dz, key_b):
         """dz = da * gelu'(z) and the layer's bias gradient (the column sums of dz) in the same pass."""
         db = torch.zeros(z.shape[-1], device=self.device, dtype=F32)
-        T.gelu_bwd(da, z, dz, db)
+        T.gelu_bwd(da, z, dz, db, det=self._det)
         self.g[key_b].copy_(db)
 
     def _dgrad_gelu(self, conv, dz, z_below, dz_out, key_b, tmp_name):
@@ -279,14 +299,14 @@ class CryoVITHeadTrainerB200:
     def _bias_grad(self, dz, key_b):
         """The bias gradient alone (column sums of dz), for layers whose gelu' was applied by the producing epilogue."""
         db = torch.zeros(dz.shape[-1], device=self.device, dtype=F32)
-        T.colsum(dz, db)
+        T.colsum(dz, db, det=self._det)
         self.g[key_b].copy_(db)
 
     def _wgrad_conv(self, x, dz, dil, key_w):
         """Accumulates the weight gradient of a 3x3x3 convolution into the flat bucket (the bias gradient comes out of
         ``_gelu_bwd_bias``, which produced dz)."""
         cin, cout = x.shape[-1], dz.shape[-1]
-        dw = T.conv_weight_gradient(x, dz, dil, self._bufs.setdefault("wgrad_pool", {}))  # [27, cout, cin]
+        dw = T.conv_weight_gradient(x, dz, dil, self._bufs.setdefault("wgrad_pool", {}), det=self._det)  # [27, cout, cin]
         self.g[key_w].copy_(dw.reshape(3, 3, 3, cout, cin).permute(3, 4, 0, 1, 2))
         self.launches += 7
 
@@ -294,7 +314,7 @@ class CryoVITHeadTrainerB200:
         """dW[M, N] = dz_rows^T @ x_rows for row-major bf16 [R, N] / [R, M] (1x1x1 and transposed convolutions). ``xt``:
         x already channels-first, bf16 [N, R] with R a multiple of 8 (then x_rows is not read)."""
         if xt is None:  # straight from the row-major operands when the MN-major kernel takes the shapes (no transposed copies)
-            direct = T.rows_weight_gradient(x_rows, dz_rows)
+            direct = T.rows_weight_gradient(x_rows, dz_rows, det=self._det)
             if direct is not None:
                 self.launches += 1
                 return direct
@@ -309,7 +329,7 @@ class CryoVITHeadTrainerB200:
             N = xt.shape[0]
         T.to_cfirst_padded(dz_rows.view(1, 1, R, M), dzt, 0, 0, 0)
         dw = torch.zeros(1, M, N, device=self.device, dtype=F32)
-        T.wgrad_splitk(dzt, xt, dw, torch.zeros(1, dtype=torch.int32, device=self.device), pitch)
+        T.wgrad_splitk(dzt, xt, dw, torch.zeros(1, dtype=torch.int32, device=self.device), pitch, det=self._det)
         self.launches += 3
         return dw[0]
 
@@ -353,7 +373,7 @@ class CryoVITHeadTrainerB200:
             G = max(8, c1 // 8)
             n_out = self._buf(f"gn{bi}", (D, H, W, c1))
             stats = self._buf(f"gn{bi}_stats", (2 * G,), F32)
-            ops.groupnorm_ndhwc(cur, n_out, p[pre + "0.weight"], p[pre + "0.bias"], stats, G, 1e-3)
+            ops.groupnorm_ndhwc(cur, n_out, p[pre + "0.weight"], p[pre + "0.bias"], stats, G, 1e-3, det=self._det)
             ca, cb = _Conv(self, pre + "1.weight", c1, c2, d1), _Conv(self, pre + "3.weight", c2, c2, d2)
             za, aa = self._buf(f"za{bi}", (D, H, W, c2)), self._buf(f"aa{bi}", (D, H, W, c2))
             if fuse:
@@ -396,17 +416,17 @@ class CryoVITHeadTrainerB200:
                               p["output_layer.2.bias"], logits, probs)
         lab = self._buf("labels", (D, H, W), F32)
         lab.copy_(labels.to(dev))
-        stats8 = ops.seg_stats(probs, lab)
+        stats8 = ops.seg_stats(probs, lab, det=self._det)
         loss = 1.0 - 2.0 * stats8[2] / (stats8[1] + stats8[0] + 1e-3)
         self.launches += 4
         # ---------------- backward
         dl8 = self._buf("dlogit8", (D, H, W, 8))
         T.dice_bwd(logits, probs, lab, stats8, dl8, grad_scale)
         # output_layer.2 (8 -> 1): operate on the 8-channel padded gradient (channel 0 live)
-        dw2 = T.conv_weight_gradient(a1, dl8, 1, self._bufs.setdefault("wgrad_pool", {}))  # [27, 8 (co, only 0 live), 8 (ci)]
+        dw2 = T.conv_weight_gradient(a1, dl8, 1, self._bufs.setdefault("wgrad_pool", {}), det=self._det)  # [27, 8 (co, only 0 live), 8 (ci)]
         g["output_layer.2.weight"].copy_(dw2[:, 0].view(3, 3, 3, 8).permute(3, 0, 1, 2)[None])
         db2 = torch.zeros(8, device=dev, dtype=F32)
-        T.colsum(dl8, db2)
+        T.colsum(dl8, db2, det=self._det)
         g["output_layer.2.bias"].copy_(db2[:1])
         # forward weight zero-padded to 8 output channels (the gradient volume carries 8 channels, channel 0 live)
         c_out2 = _Conv(self, "output_layer.2.weight", 8, 8, 1,
@@ -439,7 +459,7 @@ class CryoVITHeadTrainerB200:
                 # d(zt) = d(at) * gelu'(zt), written straight in the sub-pixel-major row layout of the GEMMs below; the bias
                 # gradient (summed over voxels AND sub-pixels) from the same pass
                 db = torch.zeros(c3, device=dev, dtype=F32)
-                T.gelu_bwd_unshuffle(dcur, zt, dzun, db)
+                T.gelu_bwd_unshuffle(dcur, zt, dzun, db, det=self._det)
                 g[pre + "5.bias"].copy_(db)
             rows = D * H * W
             dwt = self._wgrad_rows(ab.view(rows, c2), dzun.view(rows, 4 * c3))          # [(ij, c3), c2]
@@ -481,17 +501,18 @@ class CryoVITHeadTrainerB200:
                 if bi > 0:
                     c3p = BLOCKS[bi - 1][2]
                     dz_below = self._buf(f"dzun{bi - 1}", (D, H // 2, W // 2, 4 * c3p))
-                    T.groupnorm_bwd_gelu(blk_in, dn, dz_below, p[pre + "0.weight"], stats, dgam, dbet, G, 1e-3, saved[bi - 1][10], db, True)
+                    T.groupnorm_bwd_gelu(blk_in, dn, dz_below, p[pre + "0.weight"], stats, dgam, dbet, G, 1e-3, saved[bi - 1][10], db, True,
+                                         det=self._det)
                     g[f"layers.{bi + 1}.layers.5.bias"].copy_(db)
                     dzun_ready = True
                 else:
                     dzp = self._buf("dz_proj", (vox, 1024))
                     T.groupnorm_bwd_gelu(blk_in, dn, dzp.view(D, H, W, 1024), p[pre + "0.weight"], stats, dgam, dbet, G, 1e-3,
-                                         z_proj.view(D, H, W, 1024), db, False)
+                                         z_proj.view(D, H, W, 1024), db, False, det=self._det)
                     g["layers.0.bias"].copy_(db)
             else:
                 dblk = self._buf(f"dblk{bi}", (D, H, W, c1))
-                T.groupnorm_bwd(blk_in, dn, dblk, p[pre + "0.weight"], stats, dgam, dbet, G, 1e-3)
+                T.groupnorm_bwd(blk_in, dn, dblk, p[pre + "0.weight"], stats, dgam, dbet, G, 1e-3, det=self._det)
                 dcur = dblk
             g[pre + "0.weight"].copy_(dgam)
             g[pre + "0.bias"].copy_(dbet)

@@ -6,7 +6,10 @@ import os
 import torch
 
 from . import _lib
-from .ops import BF16, F32, _aux, _chk, _stream
+from .ops import BF16, F32, _aux, _chk, _stream, det_scratch
+
+# Every reduction below that ends in float atomics takes ``det``: None (default) keeps the atomic kernel; a scratch provider
+# (ops.det_scratch) selects its deterministic variant, per-block partial rows added in a fixed order (csrc/det_reduce.cuh).
 
 
 def conv3d_dilated_act(x, w_taps, bias, out, dil: int, act, aux=None) -> None:
@@ -48,22 +51,33 @@ def gelu_fwd(z, a) -> None:
     _lib.call("cvit_gelu_fwd_bf16", _chk(z, BF16, "z"), _chk(a, BF16, "a"), z.numel(), _stream())
 
 
-def gelu_bwd_unshuffle(da, z, dzun, db) -> None:
+def gelu_bwd_unshuffle(da, z, dzun, db, det=None) -> None:
     """dz = da * gelu'(z) over a [D, H2, W2, C] volume, stored pixel-unshuffled into dzun [D, H2/2, W2/2, 4C]
     ((i, j, c) channel order), db += column sums of dz."""
     D, H2, W2, C = z.shape
     if tuple(dzun.shape) != (D, H2 // 2, W2 // 2, 4 * C):
         raise _lib.CryovitB200Error(f"gelu_bwd_unshuffle: dzun {tuple(dzun.shape)} does not match z {tuple(z.shape)}")
+    if det is not None:
+        sp, sn = det_scratch(det, "scratch", _lib.load().cvit_gelu_bwd_colsum_unshuffle_bf16_det_partials(D, H2, W2, C))
+        _lib.call("cvit_gelu_bwd_colsum_unshuffle_bf16_det", _chk(da, BF16, "da"), _chk(z, BF16, "z"), _chk(dzun, BF16, "dzun"),
+                  _chk(db, F32, "db"), D, H2, W2, C, sp, sn, _stream())
+        return
     _lib.call("cvit_gelu_bwd_colsum_unshuffle_bf16", _chk(da, BF16, "da"), _chk(z, BF16, "z"), _chk(dzun, BF16, "dzun"),
               _chk(db, F32, "db"), D, H2, W2, C, _stream())
 
 
-def gelu_bwd(da, z, dz, db=None) -> None:
+def gelu_bwd(da, z, dz, db=None, det=None) -> None:
     """dz = da * gelu'(z); with ``db`` (fp32 [C], zeroed by the caller) also db += column sums of dz over the last axis."""
     if db is None:
         _lib.call("cvit_gelu_bwd_bf16", _chk(da, BF16, "da"), _chk(z, BF16, "z"), _chk(dz, BF16, "dz"), z.numel(), _stream())
         return
     C = z.shape[-1]
+    if det is not None:
+        R = z.numel() // C
+        sp, sn = det_scratch(det, "scratch", _lib.load().cvit_gelu_bwd_colsum_bf16_det_partials(R, C))
+        _lib.call("cvit_gelu_bwd_colsum_bf16_det", _chk(da, BF16, "da"), _chk(z, BF16, "z"), _chk(dz, BF16, "dz"), _chk(db, F32, "db"),
+                  R, C, sp, sn, _stream())
+        return
     _lib.call("cvit_gelu_bwd_colsum_bf16", _chk(da, BF16, "da"), _chk(z, BF16, "z"), _chk(dz, BF16, "dz"), _chk(db, F32, "db"),
               z.numel() // C, C, _stream())
 
@@ -73,23 +87,43 @@ def dice_bwd(logits, probs, labels, stats8, dlogit8, scale: float = 1.0) -> None
               _chk(stats8, torch.float64, "stats8"), float(scale), _chk(dlogit8, BF16, "dlogit8"), logits.numel(), _stream())
 
 
-def colsum(x, out) -> None:
+def colsum(x, out, det=None) -> None:
     R, C = x.numel() // x.shape[-1], x.shape[-1]
+    if det is not None:
+        sp, sn = det_scratch(det, "scratch", _lib.load().cvit_colsum_bf16_det_partials(R, C))
+        _lib.call("cvit_colsum_bf16_det", _chk(x, BF16, "x"), _chk(out, F32, "out"), R, C, sp, sn, _stream())
+        return
     _lib.call("cvit_colsum_bf16", _chk(x, BF16, "x"), _chk(out, F32, "out"), R, C, _stream())
 
 
-def groupnorm_bwd(x, dy, dx, gamma, stats, dgamma, dbeta, groups: int, eps: float) -> None:
+def groupnorm_bwd(x, dy, dx, gamma, stats, dgamma, dbeta, groups: int, eps: float, det=None) -> None:
     C = x.shape[-1]
+    if det is not None:
+        _groupnorm_bwd_det(x, dy, dx, gamma, stats, dgamma, dbeta, groups, eps, None, None, 0, det)
+        return
     _lib.call("cvit_groupnorm_bwd_ndhwc_bf16", _chk(x, BF16, "x"), _chk(dy, BF16, "dy"), _chk(dx, BF16, "dx"),
               _chk(gamma, F32, "gamma"), _chk(stats, F32, "stats"), _chk(dgamma, F32, "dgamma"), _chk(dbeta, F32, "dbeta"),
               x.numel() // C, C, groups, float(eps), _stream())
 
 
-def groupnorm_bwd_gelu(x, dy, dz, gamma, stats, dgamma, dbeta, groups: int, eps: float, z, db, unshuffle: bool) -> None:
+def _groupnorm_bwd_det(x, dy, dx, gamma, stats, dgamma, dbeta, groups, eps, z, db, W2, det) -> None:
+    C = x.shape[-1]
+    DHW = x.numel() // C
+    sp, sn = det_scratch(det, "scratch", _lib.load().cvit_groupnorm_bwd_gelu_ndhwc_bf16_det_partials(DHW, C, groups))
+    _lib.call("cvit_groupnorm_bwd_gelu_ndhwc_bf16_det", _chk(x, BF16, "x"), _chk(dy, BF16, "dy"), _chk(dx, BF16, "dx"),
+              _chk(gamma, F32, "gamma"), _chk(stats, F32, "stats"), _chk(dgamma, F32, "dgamma"), _chk(dbeta, F32, "dbeta"),
+              DHW, C, groups, float(eps), None if z is None else _chk(z, BF16, "z"), None if db is None else _chk(db, F32, "db"),
+              W2, sp, sn, _stream())
+
+
+def groupnorm_bwd_gelu(x, dy, dz, gamma, stats, dgamma, dbeta, groups: int, eps: float, z, db, unshuffle: bool, det=None) -> None:
     """GroupNorm backward fused with the GELU backward of the layer that produced x = gelu(z): dz = d(z), db += its column sums;
     ``unshuffle``: x is [D, H2, W2, C] and dz is written as [D, H2/2, W2/2, 4C] (sub-pixel-major channels)."""
     C = x.shape[-1]
     W2 = x.shape[2] if unshuffle else 0
+    if det is not None:
+        _groupnorm_bwd_det(x, dy, dz, gamma, stats, dgamma, dbeta, groups, eps, z, db, W2, det)
+        return
     _lib.call("cvit_groupnorm_bwd_gelu_ndhwc_bf16", _chk(x, BF16, "x"), _chk(dy, BF16, "dy"), _chk(dz, BF16, "dz"),
               _chk(gamma, F32, "gamma"), _chk(stats, F32, "stats"), _chk(dgamma, F32, "dgamma"), _chk(dbeta, F32, "dbeta"),
               x.numel() // C, C, groups, float(eps), _chk(z, BF16, "z"), _chk(db, F32, "db"), W2, _stream())
@@ -122,7 +156,7 @@ def to_cfirst_padded_x3(x, outs, pd: int, ph: int, pw: int) -> None:
               _chk(outs[2], BF16, "out"), D, H, W, C, pd, ph, pw, Wp, pitch, _stream())
 
 
-def wgrad_mn(a, b, out, dil: int = 1, shift_a: bool = False) -> None:
+def wgrad_mn(a, b, out, dil: int = 1, shift_a: bool = False, det=None) -> None:
     """out[t, m, n] += sum_v a[v + off_a(t), m] * b[v + off_b(t), n] from channels-last bf16 volumes [D,H,W,C] (27 taps) or
     [rows, C] matrices (one tap); see cvit_wgrad_mn_ndhwc."""
     ntaps = out.shape[0]
@@ -130,11 +164,16 @@ def wgrad_mn(a, b, out, dil: int = 1, shift_a: bool = False) -> None:
         D, H, W = 1, 1, a.shape[0]
     else:
         D, H, W = a.shape[:3]
+    if det is not None:
+        sp, sn = det_scratch(det, "scratch", _lib.load().cvit_wgrad_mn_ndhwc_det_partials(D, H, W, a.shape[-1], b.shape[-1], ntaps))
+        _lib.call("cvit_wgrad_mn_ndhwc_det", _chk(a, BF16, "a"), _chk(b, BF16, "b"), _chk(out, F32, "out"), D, H, W, a.shape[-1],
+                  b.shape[-1], dil, ntaps, int(shift_a), sp, sn, _stream())
+        return
     _lib.call("cvit_wgrad_mn_ndhwc", _chk(a, BF16, "a"), _chk(b, BF16, "b"), _chk(out, F32, "out"), D, H, W, a.shape[-1], b.shape[-1],
               dil, ntaps, int(shift_a), _stream())
 
 
-def rows_weight_gradient(x_rows, dz_rows):
+def rows_weight_gradient(x_rows, dz_rows, det=None):
     """dW[M, N] = dz_rows^T @ x_rows for row-major bf16 [R, N] / [R, M] (1x1x1 and transposed convolutions) without any
     transposed copy, or None when the shapes do not fit the MN-major kernel (then the caller uses the split-K path).
     Operands narrower than 64 channels are widened by viewing f consecutive rows as one row of f x C channels (both
@@ -148,7 +187,7 @@ def rows_weight_gradient(x_rows, dz_rows):
         return None
     a, b = dz_rows.view(R // f, f * M), x_rows.view(R // f, f * N)
     out = torch.zeros(1, f * M, f * N, device=x_rows.device, dtype=F32)
-    wgrad_mn(a, b, out)
+    wgrad_mn(a, b, out, det=det)
     if f == 1:
         return out[0]
     blocks = out[0].view(f, M, f, N)
@@ -158,7 +197,13 @@ def rows_weight_gradient(x_rows, dz_rows):
 _KOFFS: dict = {}
 
 
-def conv_weight_gradient(x, dz, dil: int, pool: dict | None = None) -> torch.Tensor:
+def narrow_wgrad_switches_off() -> list[str]:
+    """The switches set to select the atomic CUDA-core kernel (cvit_wgrad_narrow_ndhwc) for the narrow layers' weight gradients:
+    a path deterministic mode has no variant of."""
+    return [k for k in ("CVIT_WGRAD_TC8", "CVIT_WGRAD_TCN") if os.environ.get(k, "1") == "0"]
+
+
+def conv_weight_gradient(x, dz, dil: int, pool: dict | None = None, det=None) -> torch.Tensor:
     """dW[27, Cout, Cin] (tap = (kd*3+kh)*3+kw, fp32) of a 3x3x3 depth-dilated "same" convolution from its input x and
     output gradient dz (both bf16 [D,H,W,C]): three column-shifted channels-first copies of x, one of dz, three
     9-tap split-K GEMMs. ``pool`` (a dict) recycles the operand buffers between calls."""
@@ -167,12 +212,26 @@ def conv_weight_gradient(x, dz, dil: int, pool: dict | None = None) -> torch.Ten
     if (Cin, Cout) in ((8, 8), (16, 16), (32, 16), (32, 32)):  # narrow layers: reduction over the channels-last volumes
         dwn = torch.zeros(27, Cout, Cin, device=x.device, dtype=F32)
         if Cin == 8 and W % 8 == 0 and os.environ.get("CVIT_WGRAD_TC8", "1") != "0":  # tcgen05, voxels as K (csrc/wgrad_tc.cu)
+            if det is not None:
+                sp, sn = det_scratch(det, "scratch", _lib.load().cvit_wgrad_tc8_ndhwc_det_partials(D, H, W))
+                _lib.call("cvit_wgrad_tc8_ndhwc_det", _chk(x, BF16, "x"), _chk(dz, BF16, "dz"), _chk(dwn, F32, "dw"), D, H, W, dil,
+                          sp, sn, _stream())
+                return dwn
             _lib.call("cvit_wgrad_tc8_ndhwc", _chk(x, BF16, "x"), _chk(dz, BF16, "dz"), _chk(dwn, F32, "dw"), D, H, W, dil, _stream())
             return dwn
         if Cin > 8 and os.environ.get("CVIT_WGRAD_TCN", "1") != "0":
+            if det is not None:
+                sp, sn = det_scratch(det, "scratch", _lib.load().cvit_wgrad_tcn_ndhwc_det_partials(D, H, W, Cin, Cout))
+                _lib.call("cvit_wgrad_tcn_ndhwc_det", _chk(x, BF16, "x"), _chk(dz, BF16, "dz"), _chk(dwn, F32, "dw"), D, H, W, Cin,
+                          Cout, dil, sp, sn, _stream())
+                return dwn
             _lib.call("cvit_wgrad_tcn_ndhwc", _chk(x, BF16, "x"), _chk(dz, BF16, "dz"), _chk(dwn, F32, "dw"), D, H, W, Cin, Cout,
                       dil, _stream())
             return dwn
+        if det is not None:
+            raise _lib.CryovitB200Error(
+                f"deterministic mode: the {Cin} -> {Cout} weight gradient would take the atomic cvit_wgrad_narrow_ndhwc kernel "
+                f"({', '.join(narrow_wgrad_switches_off()) or 'W % 8 != 0'}=0); unset the switch or turn deterministic mode off")
         _lib.call("cvit_wgrad_narrow_ndhwc", _chk(x, BF16, "x"), _chk(dz, BF16, "dz"), _chk(dwn, F32, "dw"), D, H, W, Cin, Cout,
                   dil, _stream())
         return dwn
@@ -183,10 +242,10 @@ def conv_weight_gradient(x, dz, dil: int, pool: dict | None = None) -> torch.Ten
         waste = lambda c: (c + 127) // 128 * 128 / c
         if waste(Cin) <= waste(Cout):
             out = torch.zeros(27, Cin, Cout, device=x.device, dtype=F32)
-            wgrad_mn(x, dz, out, dil, shift_a=True)   # out[t, ci, co] = sum_v x[v + off_t, ci] dz[v, co]
+            wgrad_mn(x, dz, out, dil, shift_a=True, det=det)   # out[t, ci, co] = sum_v x[v + off_t, ci] dz[v, co]
             return out.transpose(1, 2)
         out = torch.zeros(27, Cout, Cin, device=x.device, dtype=F32)
-        wgrad_mn(dz, x, out, dil, shift_a=False)
+        wgrad_mn(dz, x, out, dil, shift_a=False, det=det)
         return out
     # Remaining shapes: channels-first zero-padded operand copies + the K-major split-K GEMM (csrc/wgrad.cu).
     # No depth padding: a depth tap that leaves the volume shifts the K index outside [0, K), where the GEMM's TMA loads
@@ -215,18 +274,23 @@ def conv_weight_gradient(x, dz, dil: int, pool: dict | None = None) -> torch.Ten
         xts = [buf(f"xt{kw}", Cin * pitch)[:Cin * pitch].view(Cin, pitch) for kw in range(3)]
         to_cfirst_padded_x3(x, xts, pd, 1, 1)
         for kw in range(3):
-            wgrad_splitk(dzt, xts[kw], dw[kw], koffs, pitch)
+            wgrad_splitk(dzt, xts[kw], dw[kw], koffs, pitch, det=det)
     else:
         xt = buf("xt0", Cin * pitch)[:Cin * pitch].view(Cin, pitch)
         for kw in range(3):
             to_cfirst_padded(x, xt, pd, 1, 1, kw - 1)
-            wgrad_splitk(dzt, xt, dw[kw], koffs, pitch)
+            wgrad_splitk(dzt, xt, dw[kw], koffs, pitch, det=det)
     return dw.permute(1, 0, 2, 3).reshape(27, Cout, Cin)
 
 
-def wgrad_splitk(at, bt, out, koffs, k: int) -> None:
+def wgrad_splitk(at, bt, out, koffs, k: int, det=None) -> None:
     """out[t, m, n] += sum_k at[m, k] * bt[n, k + koffs[t]]; at [M, pitch], bt [N, pitch] bf16, out fp32 [T, M, N]."""
     T, M, N = out.shape
+    if det is not None:
+        sp, sn = det_scratch(det, "scratch", _lib.load().cvit_wgrad_splitk_det_partials(M, N, k, T))
+        _lib.call("cvit_wgrad_splitk_det", _chk(at, BF16, "at"), _chk(bt, BF16, "bt"), _chk(out, F32, "out"),
+                  _chk(koffs, torch.int32, "koffs"), M, N, k, at.shape[1], bt.shape[1], T, sp, sn, _stream())
+        return
     _lib.call("cvit_wgrad_splitk", _chk(at, BF16, "at"), _chk(bt, BF16, "bt"), _chk(out, F32, "out"),
               _chk(koffs, torch.int32, "koffs"), M, N, k, at.shape[1], bt.shape[1], T, _stream())
 

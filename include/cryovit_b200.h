@@ -492,6 +492,47 @@ int cvit_adamw_f32(float* p, const float* g, float* m, float* v, int64_t n, floa
  * (models/metrics.py:69-93, strict "> 0.5"). probs, labels: fp32 [n]. */
 int cvit_seg_stats(const float* probs, const float* labels, int64_t n, float threshold, double* out8, void* stream);
 
+/* ---------------------------------------------------------------------------------------------------------------------
+ * Deterministic mode of head training (CryoVITHeadTrainerB200(deterministic=True), trainer.deterministic): the variants of
+ * every reduction the training step ends in float atomics. Each is the same kernel body with per-block (per-CTA, per-K-slice)
+ * partial rows stored in a caller-owned scratch buffer and added in a fixed order by one finalize kernel, so the result
+ * depends on the shapes and the SM count only: bit-identical across runs on one GPU. Arguments and results are those of the
+ * default entry point named in each comment; scratch holds at least *_partials(...) elements (fp32; fp64 for seg_stats). A
+ * null or smaller scratch is refused with CVIT_ERR_INVALID before any launch. The _partials functions return an element
+ * count, not an error code (0 for invalid shapes). */
+int64_t cvit_groupnorm_ndhwc_bf16_det_partials(int64_t DHW, int64_t C, int64_t G);
+int cvit_groupnorm_ndhwc_bf16_det(const void* x, void* out, const float* gamma, const float* beta, float* stats, int64_t DHW, int64_t C,
+                                  int64_t G, float eps, float* scratch, int64_t scratch_elems, void* stream);
+/* cvit_seg_stats, except that out8 is OVERWRITTEN (not accumulated into). */
+int64_t cvit_seg_stats_det_partials(int64_t n);
+int cvit_seg_stats_det(const float* probs, const float* labels, int64_t n, float threshold, double* out8, double* scratch,
+                       int64_t scratch_elems, void* stream);
+int64_t cvit_colsum_bf16_det_partials(int64_t R, int64_t C);
+int cvit_colsum_bf16_det(const void* x, float* out, int64_t R, int64_t C, float* scratch, int64_t scratch_elems, void* stream);
+int64_t cvit_gelu_bwd_colsum_bf16_det_partials(int64_t R, int64_t C);
+int cvit_gelu_bwd_colsum_bf16_det(const void* da, const void* z, void* dz, float* db, int64_t R, int64_t C, float* scratch,
+                                  int64_t scratch_elems, void* stream);
+int64_t cvit_gelu_bwd_colsum_unshuffle_bf16_det_partials(int64_t D, int64_t H2, int64_t W2, int64_t C);
+int cvit_gelu_bwd_colsum_unshuffle_bf16_det(const void* da, const void* z, void* dzun, float* db, int64_t D, int64_t H2, int64_t W2,
+                                            int64_t C, float* scratch, int64_t scratch_elems, void* stream);
+/* cvit_groupnorm_bwd_gelu_ndhwc_bf16 (z = null: cvit_groupnorm_bwd_ndhwc_bf16). */
+int64_t cvit_groupnorm_bwd_gelu_ndhwc_bf16_det_partials(int64_t DHW, int64_t C, int64_t G);
+int cvit_groupnorm_bwd_gelu_ndhwc_bf16_det(const void* x, const void* dy, void* dx, const float* gamma, const float* stats, float* dgamma,
+                                           float* dbeta, int64_t DHW, int64_t C, int64_t G, float eps, const void* z, float* db,
+                                           int64_t W2, float* scratch, int64_t scratch_elems, void* stream);
+int64_t cvit_wgrad_tc8_ndhwc_det_partials(int64_t D, int64_t H, int64_t W);
+int cvit_wgrad_tc8_ndhwc_det(const void* x, const void* dz, float* dw, int64_t D, int64_t H, int64_t W, int64_t dil, float* scratch,
+                             int64_t scratch_elems, void* stream);
+int64_t cvit_wgrad_tcn_ndhwc_det_partials(int64_t D, int64_t H, int64_t W, int64_t Cin, int64_t Cout);
+int cvit_wgrad_tcn_ndhwc_det(const void* x, const void* dz, float* dw, int64_t D, int64_t H, int64_t W, int64_t Cin, int64_t Cout,
+                             int64_t dil, float* scratch, int64_t scratch_elems, void* stream);
+int64_t cvit_wgrad_mn_ndhwc_det_partials(int64_t D, int64_t H, int64_t W, int64_t Ca, int64_t Cb, int64_t ntaps);
+int cvit_wgrad_mn_ndhwc_det(const void* a, const void* b, float* out, int64_t D, int64_t H, int64_t W, int64_t Ca, int64_t Cb,
+                            int64_t dil, int64_t ntaps, int shift_a, float* scratch, int64_t scratch_elems, void* stream);
+int64_t cvit_wgrad_splitk_det_partials(int64_t M, int64_t N, int64_t K, int64_t ntaps);
+int cvit_wgrad_splitk_det(const void* At, const void* Bt, float* out, const int* koffs, int64_t M, int64_t N, int64_t K,
+                          int64_t pitch_a, int64_t pitch_b, int64_t ntaps, float* scratch, int64_t scratch_elems, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
