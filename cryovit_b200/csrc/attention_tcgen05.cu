@@ -7,7 +7,8 @@
 // Barrier phases, the K/V ring and the S/P/O buffers run across items: the tile stream never drains at an item end.
 //   warps 0-3   softmax group A, warps 4-7 softmax group B; one thread per query row (TMEM lane = row). The whole
 //               128-wide S row is held in registers: row max (3-input FMNMX), lazy rescale (O and l are only rescaled
-//               when the max grows by more than 2^8), p = exp2(s*c - m*c) with packed f32x2 FMA/ADD -> bf16 pairs
+//               when the max grows by more than 2^16 for bf16 P, 2^8 for fp16 P: FA_RESCALE_LOG2), p = exp2(s*c - m*c)
+//               with packed f32x2 FMA/ADD -> bf16 pairs
 //               -> TMEM. P(j) is published to the MMA warp only after the loads of S(j+1) were issued, so the TMEM
 //               store drain (300-600 cycles when the tensor pipe is busy) is off the critical path.
 //   warps 8-11  epilogue: O_g / l -> bf16 -> global, while the softmax warps already run the next item.
