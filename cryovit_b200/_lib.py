@@ -88,6 +88,7 @@ SIGNATURES: dict[str, list] = {
     "cvit_wgrad_tc8_ndhwc": [P, P, P, I64, I64, I64, I64, P],
     "cvit_wgrad_tcn_ndhwc": [P, P, P, I64, I64, I64, I64, I64, I64, P],
     "cvit_adamw_f32": [P, P, P, P, I64, F32, F32, F32, F32, F32, I64, F32, P],
+    "cvit_accumulate_f32": [P, P, I64, P],
     "cvit_conv3d_wpack8_gelu": [P, P, P, P, I64, I64, I64, I32, P],
     "cvit_conv3d_wpack8_final": [P, P, P, P, P, I64, I64, I64, P],
     "cvit_linear_bias_cfirst_f16_gn": [P, I64, P, P, P, I64, I64, I64, I64, I32, P, I64, P],

@@ -625,4 +625,9 @@ int cvit_adamw_f32(float* p, const float* g, float* m, float* v, int64_t n, floa
   return check_launch("adamw_kernel");
 }
 
+int cvit_accumulate_f32(float* dst, const float* src, int64_t n, void* stream) {
+  if (!dst || !src || n <= 0) { set_error("accumulate_f32: bad arguments"); return CVIT_ERR_INVALID; }
+  return det_finalize(src, 1, n, n, dst, true, (cudaStream_t)stream);
+}
+
 }  // extern "C"

@@ -165,13 +165,18 @@ class TomoDataset:
                 out[k] = got[k]
         return out
 
+    def max_crop_shape(self) -> tuple[int, int, int]:
+        """(depth, rows, cols) of the largest input crop ``_crop_slices`` cuts: at most 128 slices, 32x32 feature patches
+        (512x512 voxels for raw input)."""
+        side = 32 if self.input_key == "dino_features" else 512
+        return 128, side, side
+
     def _crop_slices(self, shape) -> tuple[tuple[slice, ...], tuple[slice, ...]] | None:
         """tomo_dataset.py:148-178: at most 128 slices, 32x32 feature patches (512x512 voxels for raw input); the
         label crop is the x16 image of the feature crop. Draw order (depth, rows, cols) follows the reference. Only
         the SHAPE is needed, so the same draw serves a numpy array from a file and a volume resident in HBM.
         Returns (input slices over the last three axes, label slices) or None when nothing is cropped."""
-        max_depth = 128
-        side = 32 if self.input_key == "dino_features" else 512
+        max_depth, side, _ = self.max_crop_shape()
         d, h, w = shape[-3:]
         x, y, z = min(d, max_depth), side, side
         if (d, h, w) == (x, y, z):

@@ -1,10 +1,12 @@
 """Head training loop with the reference's schedule (run/train_model.py:206-312, configs/trainer/fit.yaml,
-configs/callbacks/stochastic_weight_average.yaml): seed, AdamW(lr, weight_decay) on every step, batch of ONE tomogram
-crop per process (dataloader/default.yaml batch_size 1), ``max_epochs`` passes, stochastic weight averaging of the
+configs/callbacks/stochastic_weight_average.yaml): seed, AdamW(lr, weight_decay) on every step, a batch of ``batch_size``
+tomogram crops per process and step (dataloader/default.yaml batch_size 1) with ONE masked Dice loss over the batch,
+``max_epochs`` passes, stochastic weight averaging of the
 weights from ``swa_epoch_start`` on (constant learning rate ``swa_lrs = lr``, so SWA is a running mean of the weights
 at the epoch starts, as Lightning's callback samples them),
 final ``weights.pt`` = plain state dict with the reference's parameter names (:312). Lightning itself is not used:
-the step is ``CryoVITHeadTrainerB200.train_step`` (native forward / backward / all-reduce / AdamW)."""
+the step is ``CryoVITHeadTrainerB200.train_step`` (one crop) or ``train_batch`` (native forward / backward / all-reduce /
+AdamW). Validation stays one tomogram at a time."""
 from __future__ import annotations
 
 import logging
@@ -21,16 +23,25 @@ from .datasets import ResidentTomoCache, TomoDataset
 from .shard import rank_world, require_process_group
 
 
-def _cache_budget_bytes(cache_gb: float | None) -> int:
+def _cache_budget_bytes(cache_gb: float | None, reserve: int = 0) -> int:
     """HBM the resident training set may take: ``cache_gb`` (``CRYOVIT_B200_FEATURE_CACHE_GB`` when None; 0 disables),
-    by default 60 % of what is free on the device right now (the trainer's own buffers for a full-size crop are ~6 GB)."""
+    by default 60 % of what is free on the device right now (the trainer's own buffers for a full-size crop are ~6 GB)
+    once ``reserve`` bytes (the further crops of a batch) are set aside."""
     if cache_gb is None:
         env = os.environ.get("CRYOVIT_B200_FEATURE_CACHE_GB", "").strip()
         cache_gb = float(env) if env else None
     if cache_gb is not None:
         return int(cache_gb * 1e9)
     free, _total = torch.cuda.mem_get_info()
-    return int(0.6 * free)
+    return int(0.6 * max(free - reserve, 0))
+
+
+def check_batch_size(batch_size) -> int:
+    """``datamodule.dataloader.batch_size``: an int >= 1. None is refused: Lightning would hand ``collate_fn`` a bare
+    item rather than a batch."""
+    if isinstance(batch_size, bool) or not isinstance(batch_size, int) or batch_size < 1:
+        raise ValueError(f"datamodule.dataloader.batch_size={batch_size!r}: training needs an integer >= 1")
+    return batch_size
 
 
 def _append_row(path: Path, row: dict, first: bool) -> None:
@@ -46,7 +57,7 @@ def _append_row(path: Path, row: dict, first: bool) -> None:
 def fit_head(dataset: TomoDataset, in_channels: int = 1536, max_epochs: int = 50, lr: float = 1e-4, weight_decay: float = 1e-3,
              swa_epoch_start: int | None = 40, seed: int = 42, exp_dir: Path | str | None = None, state_dict: dict | None = None,
              log_every: int = 10, cache_gb: float | None = None, epoch_seconds: list | None = None, validator=None,
-             val_history: list | None = None, deterministic: bool | str = False) -> dict[str, torch.Tensor]:
+             val_history: list | None = None, deterministic: bool | str = False, batch_size: int = 1) -> dict[str, torch.Tensor]:
     """Trains on the items of ``dataset`` (``train=True`` gives the reference's random 128 x 32 x 32 feature crops);
     with several ranks (torchrun) every rank walks its own round-robin share of a common shuffled order and the
     gradients are averaged over the ranks each step. Returns the final (SWA-averaged if enabled) state dict.
@@ -64,23 +75,40 @@ def fit_head(dataset: TomoDataset, in_channels: int = 1536, max_epochs: int = 50
     ``deterministic`` (Lightning's ``trainer.deterministic``: False, True or ``"warn"``): the training step runs its fixed-order
     reductions (``CryoVITHeadTrainerB200(deterministic=True)``), so a run with the same seed, data and build on the same GPU
     model and world size gives bit-identical weights, losses and validation metrics. As Lightning does, torch's
-    ``use_deterministic_algorithms`` is set for the duration (warn-only with ``"warn"``) and restored on exit."""
+    ``use_deterministic_algorithms`` is set for the duration (warn-only with ``"warn"``) and restored on exit.
+
+    ``batch_size`` (``datamodule.dataloader.batch_size``): every rank cuts its share of the epoch's order into consecutive
+    batches of that many crops, the last one shorter when the share does not divide (``drop_last=False``), and takes one
+    optimizer step per batch (``CryoVITHeadTrainerB200.train_batch``: depth padded to the batch's deepest crop, ONE Dice
+    loss over the batch). The crops of a batch must share their feature plane, as ``collate_fn`` requires. Every rank's
+    share has the same length, so every rank takes the same number of steps. SWA, validation and ``log_every`` count
+    optimizer steps."""
     if deterministic not in (False, True, "warn"):
         raise ValueError(f"deterministic={deterministic!r}: expected False, True or 'warn'")
+    batch_size = check_batch_size(batch_size)
     if not deterministic:
         return _fit_head(dataset, in_channels, max_epochs, lr, weight_decay, swa_epoch_start, seed, exp_dir, state_dict, log_every,
-                         cache_gb, epoch_seconds, validator, val_history, False)
+                         cache_gb, epoch_seconds, validator, val_history, False, batch_size)
     prev = (torch.are_deterministic_algorithms_enabled(), torch.is_deterministic_algorithms_warn_only_enabled())
     torch.use_deterministic_algorithms(True, warn_only=deterministic == "warn")
     try:
         return _fit_head(dataset, in_channels, max_epochs, lr, weight_decay, swa_epoch_start, seed, exp_dir, state_dict, log_every,
-                         cache_gb, epoch_seconds, validator, val_history, True)
+                         cache_gb, epoch_seconds, validator, val_history, True, batch_size)
     finally:
         torch.use_deterministic_algorithms(prev[0], warn_only=prev[1])
 
 
+def _check_planes(items) -> None:
+    """collate_fn stacks the crops of a batch: every one needs the first one's channels and feature plane."""
+    a = items[0]
+    for b in items[1:]:
+        if b.data.shape[0] != a.data.shape[0] or b.data.shape[-2:] != a.data.shape[-2:]:
+            raise ValueError(f"batch of crops with different feature planes: {a.sample}/{a.tomo_name} {tuple(a.data.shape)} and "
+                             f"{b.sample}/{b.tomo_name} {tuple(b.data.shape)}; collate_fn needs one (h, w) per batch")
+
+
 def _fit_head(dataset, in_channels, max_epochs, lr, weight_decay, swa_epoch_start, seed, exp_dir, state_dict, log_every, cache_gb,
-              epoch_seconds, validator, val_history, deterministic: bool) -> dict[str, torch.Tensor]:
+              epoch_seconds, validator, val_history, deterministic: bool, batch_size: int) -> dict[str, torch.Tensor]:
     rank, world = rank_world()
     require_process_group("fit_head")  # the data is sharded by rank below: the gradients must really be exchanged
     torch.manual_seed(seed)
@@ -98,7 +126,9 @@ def _fit_head(dataset, in_channels, max_epochs, lr, weight_decay, swa_epoch_star
     step = 0
     cache = None
     cacheable = hasattr(dataset, "_crop_slices") and hasattr(dataset, "_load_tomogram")
-    budget = _cache_budget_bytes(cache_gb) if cacheable or validator is not None else 0
+    # room for the kept activations of a batch's further crops, at the largest crop the dataset cuts
+    reserve = (batch_size - 1) * trainer.sample_bytes(*dataset.max_crop_shape()) if batch_size > 1 and cacheable else 0
+    budget = _cache_budget_bytes(cache_gb, reserve) if cacheable or validator is not None else 0
     if cacheable:
         if budget > 0:
             cache = ResidentTomoCache(dataset, trainer.device, budget)  # where the trainer lives
@@ -121,11 +151,19 @@ def _fit_head(dataset, in_channels, max_epochs, lr, weight_decay, swa_epoch_star
             losses = []
             mine = [int(i) for i in order[:usable][rank::world]]
             nxt = pool.submit(fetch, mine[0]) if mine else None
-            for k in range(len(mine)):
-                item = cache.finish(nxt.result()) if cache is not None else nxt.result()
-                nxt = pool.submit(fetch, mine[k + 1]) if k + 1 < len(mine) else None
+            for b0 in range(0, len(mine), batch_size):
+                items = []
+                for k in range(b0, min(b0 + batch_size, len(mine))):
+                    items.append(cache.finish(nxt.result()) if cache is not None else nxt.result())
+                    nxt = pool.submit(fetch, mine[k + 1]) if k + 1 < len(mine) else None
                 dev = trainer.device
-                loss = trainer.train_step(item.data.to(dev, non_blocking=True), item.label.to(dev, non_blocking=True))
+                if batch_size == 1:
+                    item = items[0]
+                    loss = trainer.train_step(item.data.to(dev, non_blocking=True), item.label.to(dev, non_blocking=True))
+                else:
+                    _check_planes(items)
+                    loss = trainer.train_batch([(it.data.to(dev, non_blocking=True), it.label.to(dev, non_blocking=True))
+                                                for it in items])
                 step += 1
                 if step % log_every == 0 or len(losses) == 0:
                     losses.append(float(loss))
@@ -135,8 +173,8 @@ def _fit_head(dataset, in_channels, max_epochs, lr, weight_decay, swa_epoch_star
                 if epoch_seconds is not None:
                     epoch_seconds.append(time.perf_counter() - t_epoch)
             if rank == 0:
-                logging.info("epoch %d: %d steps/rank, DiceLoss %.4f, %.2f s", epoch, usable // world,
-                             float(np.mean(losses)) if losses else float("nan"), time.perf_counter() - t_epoch)
+                logging.info("epoch %d: %d steps/rank (batches of %d), DiceLoss %.4f, %.2f s", epoch, -(-(usable // world) // batch_size),
+                             batch_size, float(np.mean(losses)) if losses else float("nan"), time.perf_counter() - t_epoch)
             if validator is not None and validator.scheduled(epoch):
                 row = validator.run(trainer, epoch, cache_budget=budget - (cache.used if cache is not None else 0))
                 if val_history is not None:

@@ -12,7 +12,7 @@ import torch
 
 from .._lib import CryovitB200Error
 from .config import instantiate
-from .fit import fit_head
+from .fit import check_batch_size, fit_head
 from .shard import process_group
 from .validate import Validator
 
@@ -75,6 +75,13 @@ def deterministic_setting(cfg) -> bool | str:
     raise ValueError(f"trainer.deterministic={v!r}: expected true, false or 'warn'")
 
 
+def batch_size_setting(cfg) -> int:
+    """``datamodule.dataloader.batch_size`` (the reference's DataLoader batch: crops per process and optimizer step), an
+    int >= 1. ``build_datamodule`` drops the dataloader node, so it is read here."""
+    dl = cfg.datamodule.get("dataloader") or {}
+    return check_batch_size(dl.get("batch_size", 1))
+
+
 def run_trainer(cfg) -> Path:
     """train_model.py:206-312. Returns the path of the saved ``weights.pt``. Under torchrun every rank binds its own
     GPU and joins one NCCL group for the gradient all-reduce (Lightning's DDP strategy in the reference)."""
@@ -112,10 +119,11 @@ def _run_trainer(cfg) -> Path:
             raise ValueError(f"Unsupported checkpoint format: {Path(ckpt).suffix}. Use .pt or .model files.")
     in_channels = int(cfg.model.get("in_channels", 1536))
     deterministic = deterministic_setting(cfg)
+    batch_size = batch_size_setting(cfg)
     validator = build_validator(cfg, datamodule, in_channels)
-    logging.info("Starting training.")
+    logging.info("Starting training: batch size %d (crops per process and optimizer step, one Dice loss per batch).", batch_size)
     fit_head(dataset, in_channels=in_channels, max_epochs=max_epochs, lr=float(cfg.model.lr),
              weight_decay=float(cfg.model.get("weight_decay", 1e-3)), swa_epoch_start=swa_start, seed=int(cfg.random_seed),
-             exp_dir=cfg.paths.exp_dir, state_dict=state, validator=validator, deterministic=deterministic)
+             exp_dir=cfg.paths.exp_dir, state_dict=state, validator=validator, deterministic=deterministic, batch_size=batch_size)
     logging.info("Saving model.")
     return cfg.paths.exp_dir / "weights.pt"

@@ -1,9 +1,12 @@
 """CryoVIT head TRAINING on B200 (BASELINE config 5; reference models/cryovit.py:10-83, models/base_model.py:58-63,
-91-164, models/losses.py:17-32, configs/trainer/fit.yaml: AdamW lr 1e-4 / wd 1e-3, masked DiceLoss, batch of one
-tomogram crop per GPU, 16-mixed precision).
+91-164, models/losses.py:17-32, configs/trainer/fit.yaml: AdamW lr 1e-4 / wd 1e-3, masked DiceLoss, a batch of
+``datamodule.dataloader.batch_size`` tomogram crops per GPU (default one), 16-mixed precision).
 
 One training step = forward with kept pre-activations -> masked Dice loss -> backward -> (data parallel) all-reduce of
-ONE flat fp32 gradient bucket over NCCL -> fused AdamW on fp32 master weights. All arithmetic of the step runs in the
+ONE flat fp32 gradient bucket over NCCL -> fused AdamW on fp32 master weights. A batch of B crops (``train_batch``) is
+padded in depth as the reference's ``collate_fn`` pads it, runs the forward sample by sample, takes ONE Dice loss over
+the whole batch and sums the samples' gradients in the bucket (``cvit_accumulate_f32``): one all-reduce and one AdamW
+step per batch. All arithmetic of the step runs in the
 sm_100a kernels behind the C ABI:
 
   forward    the inference convolution kernels with act = 0 (they store the pre-activation z) + cvit_gelu_fwd
@@ -164,7 +167,8 @@ class _KeepAlivePool(dict):
 
 
 class CryoVITHeadTrainerB200:
-    """Data-parallel trainer of the CryoVIT head: one process per GPU, one tomogram crop per process and step."""
+    """Data-parallel trainer of the CryoVIT head: one process per GPU, one tomogram crop (``train_step``) or one batch of
+    crops with one Dice loss (``train_batch``) per process and step."""
 
     def __init__(self, in_channels: int = 1536, lr: float = 1e-4, weight_decay: float = 1e-3, betas=(0.9, 0.999),
                  eps: float = 1e-8, state_dict: dict | None = None, device=None, seed: int = 0, deterministic: bool = False):
@@ -233,6 +237,8 @@ class CryoVITHeadTrainerB200:
         self._det = self._det_scratch if self.deterministic else None
         self._graphs: dict = {}
         self._graph_broken = False
+        self._gdst = self.g  # where the backward writes the gradients (a batch's samples after the first: _sample_gradients)
+        self._flat_g_sample, self._g_sample = None, None
 
     # ------------------------------------------------------------------ bf16 operand images of the updated weights
     def _pk(self, name: str, key: str, fn) -> torch.Tensor:
@@ -260,6 +266,21 @@ class CryoVITHeadTrainerB200:
         return self._flat_store, dict(self._offsets), {k: tuple(v.shape) for k, v in self.p.items()}
 
     # ------------------------------------------------------------------ helpers
+    def sample_bytes(self, D: int, h: int, w: int) -> int:
+        """Device memory one more crop (C, D, h, w) of a batch step takes (``forward_backward`` of a batch): its staged
+        features (fp16) and labels (at most fp32), the activations the backward keeps of it (bf16: projection, GroupNorm
+        outputs, every z and gelu(z) of the four blocks and output_layer.0), its logits, probabilities and fp32 labels,
+        and its slot of the Dice gradient (bf16 x 8). The backward's scratch is shared by the samples and not counted."""
+        vox, full = D * h * w, D * 256 * h * w
+        bf16 = 2 * 1024 * vox
+        H, W = h, w
+        for c1, c2, c3, _, _ in BLOCKS:
+            v = D * H * W
+            bf16 += v * (c1 + 4 * c2) + 4 * v * 2 * c3
+            H, W = 2 * H, 2 * W
+        bf16 += full * (2 * 8 + 8)
+        return 2 * self.in_channels * vox + 4 * full + 2 * bf16 + 3 * 4 * full
+
     def state_dict(self) -> dict[str, torch.Tensor]:
         return {k: v.detach().clone().cpu() for k, v in self.p.items()}
 
@@ -282,7 +303,7 @@ class CryoVITHeadTrainerB200:
         """dz = da * gelu'(z) and the layer's bias gradient (the column sums of dz) in the same pass."""
         db = torch.zeros(z.shape[-1], device=self.device, dtype=F32)
         T.gelu_bwd(da, z, dz, db, det=self._det)
-        self.g[key_b].copy_(db)
+        self._gdst[key_b].copy_(db)
 
     def _dgrad_gelu(self, conv, dz, z_below, dz_out, key_b, tmp_name):
         """dz_out = conv^T(dz) * gelu'(z_below) (the gradient of the pre-activation below ``conv``) and that layer's bias
@@ -290,7 +311,7 @@ class CryoVITHeadTrainerB200:
         if self.fuse_dgrad_gelu and conv.fuses_gelu_grad(dz):
             db = torch.zeros(z_below.shape[-1], device=self.device, dtype=F32)
             conv.input_gradient(dz, dz_out, z_below=z_below, db=db)
-            self.g[key_b].copy_(db)
+            self._gdst[key_b].copy_(db)
         else:
             da = self._buf(tmp_name, tuple(dz_out.shape))
             conv.input_gradient(dz, da)
@@ -300,14 +321,14 @@ class CryoVITHeadTrainerB200:
         """The bias gradient alone (column sums of dz), for layers whose gelu' was applied by the producing epilogue."""
         db = torch.zeros(dz.shape[-1], device=self.device, dtype=F32)
         T.colsum(dz, db, det=self._det)
-        self.g[key_b].copy_(db)
+        self._gdst[key_b].copy_(db)
 
     def _wgrad_conv(self, x, dz, dil, key_w):
         """Accumulates the weight gradient of a 3x3x3 convolution into the flat bucket (the bias gradient comes out of
         ``_gelu_bwd_bias``, which produced dz)."""
         cin, cout = x.shape[-1], dz.shape[-1]
         dw = T.conv_weight_gradient(x, dz, dil, self._bufs.setdefault("wgrad_pool", {}), det=self._det)  # [27, cout, cin]
-        self.g[key_w].copy_(dw.reshape(3, 3, 3, cout, cin).permute(3, 4, 0, 1, 2))
+        self._gdst[key_w].copy_(dw.reshape(3, 3, 3, cout, cin).permute(3, 4, 0, 1, 2))
         self.launches += 7
 
     def _wgrad_rows(self, x_rows, dz_rows, xt=None):
@@ -336,19 +357,76 @@ class CryoVITHeadTrainerB200:
     # ------------------------------------------------------------------ one step
     def forward_backward(self, features: torch.Tensor, labels: torch.Tensor, grad_scale: float = 1.0) -> torch.Tensor:
         """features (C, D, h, w) fp16|fp32, labels (D, 16h, 16w) with -1 = ignore. Fills the gradient bucket and
-        returns the Dice loss (0-dim tensor on the device)."""
-        p, g, dev = self.p, self.g, self.device
+        returns the Dice loss (0-dim tensor on the device).
+
+        A batch: features (B, C, Dmax, h, w) and labels (B, Dmax, 16h, 16w), every crop's depth padded to Dmax with zero
+        features and -1 labels (``collate_fn``'s padding), as ``train_batch`` stages them. Each sample runs the forward of
+        one crop at Dmax into its own slot of the activations the backward keeps; logits, probabilities and labels lie
+        batch-contiguous, so ONE masked Dice loss over the whole batch (the reference's ``DiceLoss`` of the batch) and ONE
+        Dice backward give every voxel's gradient. The backward then runs sample after sample through shared scratch:
+        sample 0 fills the gradient bucket, every later sample a second bucket that ``cvit_accumulate_f32`` adds into
+        the first, so the bucket holds the sum of the samples' gradients, added in sample order."""
+        if features.dim() == 5:
+            return self._forward_backward_batch(features, labels, grad_scale)
         C, D, h, w = features.shape
         if C != self.in_channels or tuple(labels.shape) != (D, 16 * h, 16 * w):
             raise CryovitB200Error(f"features {tuple(features.shape)} / labels {tuple(labels.shape)} do not match")
+        self._pk_refresh()
+        st = self._forward(features, "")
+        logits, probs, (D, H, W) = st["logits"], st["probs"], st["logits"].shape
+        lab = self._buf("labels", (D, H, W), F32)
+        lab.copy_(labels.to(self.device))
+        stats8 = ops.seg_stats(probs, lab, det=self._det)
+        loss = 1.0 - 2.0 * stats8[2] / (stats8[1] + stats8[0] + 1e-3)
+        self.launches += 4
+        dl8 = self._buf("dlogit8", (D, H, W, 8))
+        T.dice_bwd(logits, probs, lab, stats8, dl8, grad_scale)
+        self._backward(st, dl8, self.g)
+        return loss
+
+    def _forward_backward_batch(self, features: torch.Tensor, labels: torch.Tensor, grad_scale: float) -> torch.Tensor:
+        """forward_backward of a staged batch (see there)."""
+        B, C, D, h, w = features.shape
+        if C != self.in_channels or tuple(labels.shape) != (B, D, 16 * h, 16 * w):
+            raise CryovitB200Error(f"batch features {tuple(features.shape)} / labels {tuple(labels.shape)} do not match")
+        H, W = 16 * h, 16 * w
+        self._pk_refresh()
+        logits, probs = self._buf("logits_b", (B, D, H, W), F32), self._buf("probs_b", (B, D, H, W), F32)
+        states = [self._forward(features[s], "" if s == 0 else f"@{s}", (logits[s], probs[s])) for s in range(B)]
+        lab = self._buf("labels_b", (B, D, H, W), F32)
+        lab.copy_(labels.to(self.device))
+        stats8 = ops.seg_stats(probs, lab, det=self._det)
+        loss = 1.0 - 2.0 * stats8[2] / (stats8[1] + stats8[0] + 1e-3)
+        self.launches += 4
+        dl8 = self._buf("dlogit8_b", (B, D, H, W, 8))
+        T.dice_bwd(logits, probs, lab, stats8, dl8, grad_scale)
+        for s in range(B):
+            self._backward(states[s], dl8[s], self.g if s == 0 else self._sample_gradients())
+            if s > 0:
+                T.accumulate(self.flat_g, self._flat_g_sample)
+                self.launches += 1
+        return loss
+
+    def _sample_gradients(self) -> dict[str, torch.Tensor]:
+        """Views of the second gradient bucket a batch's samples after the first write into, per parameter."""
+        if self._g_sample is None:
+            self._flat_g_sample = torch.zeros_like(self.flat_g)
+            self._g_sample = {k: self._flat_g_sample[o:o + self.g[k].numel()].view(self.g[k].shape) for k, o in self._offsets.items()}
+        return self._g_sample
+
+    def _forward(self, features: torch.Tensor, slot: str, out=None) -> dict:
+        """The forward of one crop (C, D, h, w), keeping what the backward needs in the buffers named with ``slot`` (a
+        batch's samples after the first keep theirs apart); ``out``: (logits, probs) views to write, else the trainer's
+        own. Returns the state ``_backward`` takes."""
+        p, dev = self.p, self.device
+        C, D, h, w = features.shape
         vox = D * h * w
         # CVIT_TRAIN_FUSE_ACT=0: GELU forward / backward as separate element-wise kernels (the A/B arm; default: fused
         # into the epilogues of the convolutions that produce z / the input gradients)
         fuse = self.fuse_activations
-        fuse_sb, fuse_bwd = fuse and self.fuse_store_bound, fuse and self.fuse_backward
-        self._pk_refresh()
+        fuse_sb = fuse and self.fuse_store_bound
         # ---------------- forward, keeping what the backward needs
-        z_proj, a_proj = self._buf("z_proj", (vox, 1024)), self._buf("a_proj", (D, h, w, 1024))
+        z_proj, a_proj = self._buf("z_proj" + slot, (vox, 1024)), self._buf("a_proj" + slot, (D, h, w, 1024))
         feats = features.to(dev).contiguous()
         # fp16 feature volumes whose row pitch TMA accepts: the (C, vox) layout is the projection's A operand as it lies
         # (MN-major) and, cast to bf16, already the channels-first operand of its weight gradient -- no transposes
@@ -359,7 +437,7 @@ class CryoVITHeadTrainerB200:
             ops.linear_bias_cfirst(feats.view(C, vox), w16, p["layers.0.bias"], z_proj, gelu=2 if fuse else 0,
                                    aux=a_proj.view(vox, 1024) if fuse else None)
         else:
-            x0 = self._buf("x0", (D, h, w, C))
+            x0 = self._buf("x0" + slot, (D, h, w, C))
             ops.features_to_ndhwc(feats, x0)
             ops.linear_bias(x0.view(vox, C), self._pk("proj/f", "layers.0.weight", lambda w_: w_.reshape(1024, C)), p["layers.0.bias"],
                             z_proj, gelu=False)
@@ -371,23 +449,23 @@ class CryoVITHeadTrainerB200:
         for bi, (c1, c2, c3, d1, d2) in enumerate(BLOCKS):
             pre = f"layers.{bi + 2}.layers."
             G = max(8, c1 // 8)
-            n_out = self._buf(f"gn{bi}", (D, H, W, c1))
-            stats = self._buf(f"gn{bi}_stats", (2 * G,), F32)
+            n_out = self._buf(f"gn{bi}{slot}", (D, H, W, c1))
+            stats = self._buf(f"gn{bi}_stats{slot}", (2 * G,), F32)
             ops.groupnorm_ndhwc(cur, n_out, p[pre + "0.weight"], p[pre + "0.bias"], stats, G, 1e-3, det=self._det)
             ca, cb = _Conv(self, pre + "1.weight", c1, c2, d1), _Conv(self, pre + "3.weight", c2, c2, d2)
-            za, aa = self._buf(f"za{bi}", (D, H, W, c2)), self._buf(f"aa{bi}", (D, H, W, c2))
+            za, aa = self._buf(f"za{bi}{slot}", (D, H, W, c2)), self._buf(f"aa{bi}{slot}", (D, H, W, c2))
             if fuse:
                 ca.forward(n_out, p[pre + "1.bias"], za, aa)
             else:
                 ca.forward(n_out, p[pre + "1.bias"], za)
                 T.gelu_fwd(za, aa)
-            zb, ab = self._buf(f"zb{bi}", (D, H, W, c2)), self._buf(f"ab{bi}", (D, H, W, c2))
+            zb, ab = self._buf(f"zb{bi}{slot}", (D, H, W, c2)), self._buf(f"ab{bi}{slot}", (D, H, W, c2))
             if fuse:
                 cb.forward(aa, p[pre + "3.bias"], zb, ab)
             else:
                 cb.forward(aa, p[pre + "3.bias"], zb)
                 T.gelu_fwd(zb, ab)
-            zt, at = self._buf(f"zt{bi}", (D, 2 * H, 2 * W, c3)), self._buf(f"at{bi}", (D, 2 * H, 2 * W, c3))
+            zt, at = self._buf(f"zt{bi}{slot}", (D, 2 * H, 2 * W, c3)), self._buf(f"at{bi}{slot}", (D, 2 * H, 2 * W, c3))
             # ConvTranspose weight [c2, c3, 1, 2, 2] -> rows (i*2+j)*c3 + co of the sub-pixel GEMM
             T.convT_act(ab, self._pk(pre + "5/f", pre + "5.weight",
                                      lambda wT, c2_=c2, c3_=c3: wT[:, :, 0].permute(2, 3, 1, 0).reshape(4 * c3_, c2_)),
@@ -398,13 +476,13 @@ class CryoVITHeadTrainerB200:
             saved.append((cur, n_out, stats, G, ca, za, aa, cb, zb, ab, zt, at, H, W))
             cur, H, W = at, 2 * H, 2 * W
         co = _Conv(self, "output_layer.0.weight", 8, 8, 1)
-        z1, a1 = self._buf("z_o0", (D, H, W, 8)), self._buf("a_o0", (D, H, W, 8))
+        z1, a1 = self._buf("z_o0" + slot, (D, H, W, 8)), self._buf("a_o0" + slot, (D, H, W, 8))
         if fuse:
             co.forward(cur, p["output_layer.0.bias"], z1, a1)
         else:
             co.forward(cur, p["output_layer.0.bias"], z1)
             T.gelu_fwd(z1, a1)
-        logits, probs = self._buf("logits", (D, H, W), F32), self._buf("probs", (D, H, W), F32)
+        logits, probs = out if out is not None else (self._buf("logits", (D, H, W), F32), self._buf("probs", (D, H, W), F32))
         if W % 8 == 0 and self.rows8:
             ops.conv3d_rows8_final(a1, self._pk("out2/f/rows8", "output_layer.2.weight", rows8_weight_image),
                                    p["output_layer.2.bias"], logits, probs)
@@ -414,14 +492,19 @@ class CryoVITHeadTrainerB200:
         else:
             ops.head_out_conv(a1, p["output_layer.2.weight"].permute(2, 3, 4, 0, 1).reshape(27, 8).contiguous(),
                               p["output_layer.2.bias"], logits, probs)
-        lab = self._buf("labels", (D, H, W), F32)
-        lab.copy_(labels.to(dev))
-        stats8 = ops.seg_stats(probs, lab, det=self._det)
-        loss = 1.0 - 2.0 * stats8[2] / (stats8[1] + stats8[0] + 1e-3)
-        self.launches += 4
+        return dict(feats=feats, cfirst=cfirst, x0=x0, z_proj=z_proj, saved=saved, cur=cur, co=co, z1=z1, a1=a1, logits=logits,
+                    probs=probs)
+
+    def _backward(self, st: dict, dl8: torch.Tensor, g: dict) -> None:
+        """The backward of one crop from its state and the Dice gradient dl8 (D, H, W, 8) of its logits; every parameter's
+        gradient is written (not added) into the views ``g``."""
+        p, dev = self.p, self.device
+        self._gdst = g
+        feats, cfirst, x0, z_proj, saved, cur, co, z1, a1 = (st[k] for k in ("feats", "cfirst", "x0", "z_proj", "saved", "cur", "co", "z1", "a1"))
+        C, D, H, W = feats.shape[0], *dl8.shape[:3]
+        vox = feats[0].numel()
+        fuse_bwd = self.fuse_activations and self.fuse_backward
         # ---------------- backward
-        dl8 = self._buf("dlogit8", (D, H, W, 8))
-        T.dice_bwd(logits, probs, lab, stats8, dl8, grad_scale)
         # output_layer.2 (8 -> 1): operate on the 8-channel padded gradient (channel 0 live)
         dw2 = T.conv_weight_gradient(a1, dl8, 1, self._bufs.setdefault("wgrad_pool", {}), det=self._det)  # [27, 8 (co, only 0 live), 8 (ci)]
         g["output_layer.2.weight"].copy_(dw2[:, 0].view(3, 3, 3, 8).permute(3, 0, 1, 2)[None])
@@ -527,7 +610,6 @@ class CryoVITHeadTrainerB200:
             dw0 = self._wgrad_rows(x0.view(vox, C), dzp)
         g["layers.0.weight"].copy_(dw0.view(1024, C, 1, 1, 1))
         self.launches += 2
-        return loss
 
     def optimizer_step(self) -> None:
         """Data-parallel: sum the flat gradient bucket over the ranks (one NCCL all-reduce; the 1/world factor was
@@ -548,49 +630,124 @@ class CryoVITHeadTrainerB200:
             self.optimizer_step()
         return loss
 
+    def train_batch(self, crops) -> torch.Tensor:
+        """One optimizer step on a batch of crops ``[(features (C, D_i, h, w), labels (D_i, 16h, 16w)), ...]``: the
+        reference's DataLoader batch of ``batch_size`` items through ``collate_fn``, with depths padded to the deepest crop,
+        ONE masked Dice loss over the whole batch, one backward (``forward_backward`` of the batch), one all-reduce and one
+        AdamW step. Every crop needs the same feature plane (h, w). The crops are copied on the device into static buffers
+        (B, C, Dmax, h, w) / (B, Dmax, 16h, 16w), padded with 0 / -1, and the step is captured as one CUDA graph per
+        (B, Dmax, h, w, dtypes): crops of different depths with the same Dmax replay the same graph."""
+        import torch.distributed as dist
+
+        crops = [(f, l) for f, l in crops]
+        if not crops:
+            raise CryovitB200Error("train_batch: an empty batch")
+        f0, l0 = crops[0]
+        for f, l in crops:
+            if f.dim() != 4 or f.shape[0] != f0.shape[0] or f.shape[2:] != f0.shape[2:]:
+                raise CryovitB200Error(f"train_batch: the crops of a batch need the same channels and feature plane (collate_fn), got "
+                                       f"features {tuple(f0.shape)} and {tuple(f.shape)}")
+            if tuple(l.shape) != (f.shape[1], 16 * f.shape[2], 16 * f.shape[3]):
+                raise CryovitB200Error(f"train_batch: features {tuple(f.shape)} / labels {tuple(l.shape)} do not match")
+        C, _, h, w = f0.shape
+        fshape = (len(crops), C, max(f.shape[1] for f, _ in crops), h, w)
+        world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
+        with nvtx.span("head.train.forward_backward"):
+            loss = self._batch_graphed(crops, fshape, f0.dtype, l0.dtype, 1.0 / world)
+        with nvtx.span("head.train.optimizer"):
+            self.optimizer_step()
+        return loss
+
+    @staticmethod
+    def _stage(crops, fb: torch.Tensor, lb: torch.Tensor) -> None:
+        """Each crop into its slot of the batch buffers, on the device, depth padded with 0 (features) and -1 (labels)."""
+        for s, (f, l) in enumerate(crops):
+            d = f.shape[1]
+            fb[s, :, :d].copy_(f, non_blocking=True)
+            lb[s, :d].copy_(l, non_blocking=True)
+            if d < fb.shape[2]:
+                fb[s, :, d:].zero_()
+                lb[s, d:].fill_(-1)
+
     # ----------------------------------------------------------------------------- CUDA graph of forward + backward
-    def _forward_backward_graphed(self, features: torch.Tensor, labels: torch.Tensor, grad_scale: float) -> torch.Tensor:
-        """forward_backward is ~200 kernels of ours plus the small torch kernels that re-pack the updated weights:
-        launch-bound for a fifth of the step. The first two steps of a given crop shape run eagerly (first-use
-        allocations, attribute settings, lookup tables); the third is captured into a CUDA graph over static input
-        buffers and every later step replays it. The all-reduce and AdamW (whose bias correction takes the step number
-        by value) stay outside the graph. CVIT_TRAIN_GRAPH=0 or a failed capture falls back to eager launches."""
+    def _capture(self, ent: dict, grad_scale: float) -> bool:
+        """Captures forward_backward over the static inputs ``ent["f"]`` / ``ent["l"]`` into ``ent["graph"]``. A failed
+        capture turns graphs off for this trainer (False)."""
+        try:
+            torch.cuda.synchronize()
+            l0 = self.launches
+            graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(graph):
+                ent["loss"] = self.forward_backward(ent["f"], ent["l"], grad_scale)
+            ent["launches"] = self.launches - l0
+            self.launches = l0
+            ent["graph"] = graph
+            return True
+        except Exception as e:  # noqa: BLE001  (capture is an optimisation: never fatal)
+            import logging
+
+            logging.warning("CUDA-graph capture of the training step failed (%s: %s); running eagerly", type(e).__name__, e)
+            self._graph_broken = True
+            torch.cuda.synchronize()
+            return False
+
+    def _graph_entry(self, key) -> dict | None:
+        """The graph table's entry of a step shape once its first two steps have run eagerly (first-use allocations,
+        attribute settings, lookup tables), else None. Every graph keeps its own pool of temporaries: only the first two
+        shapes get one. CVIT_TRAIN_GRAPH=0 or a failed capture: always None."""
         import os
 
         if os.environ.get("CVIT_TRAIN_GRAPH", "1") == "0" or self._graph_broken:
-            return self.forward_backward(features, labels, grad_scale)
-        key = (tuple(features.shape), features.dtype, tuple(labels.shape), labels.dtype, float(grad_scale))
+            return None
         ent = self._graphs.get(key)
         if ent is None:
-            if len(self._graphs) >= 2:  # every graph keeps its own pool of temporaries: only the two commonest crop shapes
-                return self.forward_backward(features, labels, grad_scale)
+            if len(self._graphs) >= 2:
+                return None
             ent = self._graphs[key] = {"seen": 0}
         if "graph" not in ent:
             ent["seen"] += 1
             if ent["seen"] <= 2:
-                return self.forward_backward(features, labels, grad_scale)
-            try:
-                ent["f"] = torch.empty(features.shape, device=self.device, dtype=features.dtype)
-                ent["l"] = torch.empty(labels.shape, device=self.device, dtype=labels.dtype)
-                ent["f"].copy_(features, non_blocking=True)
-                ent["l"].copy_(labels, non_blocking=True)
-                torch.cuda.synchronize()
-                l0 = self.launches
-                graph = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(graph):
-                    ent["loss"] = self.forward_backward(ent["f"], ent["l"], grad_scale)
-                ent["launches"] = self.launches - l0
-                self.launches = l0
-                ent["graph"] = graph
-            except Exception as e:  # noqa: BLE001  (capture is an optimisation: never fatal)
-                import logging
+                return None
+        return ent
 
-                logging.warning("CUDA-graph capture of the training step failed (%s: %s); running eagerly", type(e).__name__, e)
-                self._graph_broken = True
-                torch.cuda.synchronize()
+    def _forward_backward_graphed(self, features: torch.Tensor, labels: torch.Tensor, grad_scale: float) -> torch.Tensor:
+        """forward_backward is ~200 kernels of ours plus the small torch kernels that re-pack the updated weights:
+        launch-bound for a fifth of the step. The first two steps of a given crop shape run eagerly; the third is
+        captured into a CUDA graph over static input buffers and every later step replays it (``_graph_entry``). The
+        all-reduce and AdamW (whose bias correction takes the step number by value) stay outside the graph."""
+        ent = self._graph_entry((tuple(features.shape), features.dtype, tuple(labels.shape), labels.dtype, float(grad_scale)))
+        if ent is None:
+            return self.forward_backward(features, labels, grad_scale)
+        if "graph" not in ent:
+            ent["f"] = torch.empty(features.shape, device=self.device, dtype=features.dtype)
+            ent["l"] = torch.empty(labels.shape, device=self.device, dtype=labels.dtype)
+            ent["f"].copy_(features, non_blocking=True)
+            ent["l"].copy_(labels, non_blocking=True)
+            if not self._capture(ent, grad_scale):
                 return self.forward_backward(features, labels, grad_scale)
         ent["f"].copy_(features, non_blocking=True)
         ent["l"].copy_(labels, non_blocking=True)
+        ent["graph"].replay()
+        self.launches += ent["launches"]
+        return ent["loss"]
+
+    def _batch_graphed(self, crops, fshape: tuple, fdtype, ldtype, grad_scale: float) -> torch.Tensor:
+        """A batch step, eager or from its graph (keyed on (B, C, Dmax, h, w), the dtypes and grad_scale): the crops are
+        staged into the graph's own static buffers, so padding is data and a replay needs no other copy."""
+        B, C, D, h, w = fshape
+        lshape = (B, D, 16 * h, 16 * w)
+        ent = self._graph_entry(("batch", fshape, fdtype, ldtype, float(grad_scale)))
+        if ent is None or "graph" not in ent:
+            if ent is not None:
+                ent["f"] = torch.empty(fshape, device=self.device, dtype=fdtype)
+                ent["l"] = torch.empty(lshape, device=self.device, dtype=ldtype)
+                if self._capture(ent, grad_scale):
+                    return self._batch_graphed(crops, fshape, fdtype, ldtype, grad_scale)
+            fb = torch.empty(fshape, device=self.device, dtype=fdtype)
+            lb = torch.empty(lshape, device=self.device, dtype=ldtype)
+            self._stage(crops, fb, lb)
+            return self.forward_backward(fb, lb, grad_scale)
+        self._stage(crops, ent["f"], ent["l"])
         ent["graph"].replay()
         self.launches += ent["launches"]
         return ent["loss"]

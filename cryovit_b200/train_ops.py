@@ -298,3 +298,10 @@ def wgrad_splitk(at, bt, out, koffs, k: int, det=None) -> None:
 def adamw(p, g, m, v, lr: float, beta1: float, beta2: float, eps: float, weight_decay: float, step: int, grad_scale: float = 1.0) -> None:
     _lib.call("cvit_adamw_f32", _chk(p, F32, "p"), _chk(g, F32, "g"), _chk(m, F32, "m"), _chk(v, F32, "v"), p.numel(),
               float(lr), float(beta1), float(beta2), float(eps), float(weight_decay), int(step), float(grad_scale), _stream())
+
+
+def accumulate(dst, src) -> None:
+    """dst += src over two fp32 tensors of the same size (a batch step's per-sample gradient bucket into the step's)."""
+    if src.numel() != dst.numel():
+        raise _lib.CryovitB200Error(f"accumulate: {src.numel()} elements into {dst.numel()}")
+    _lib.call("cvit_accumulate_f32", _chk(dst, F32, "dst"), _chk(src, F32, "src"), dst.numel(), _stream())

@@ -485,6 +485,11 @@ int cvit_wgrad_tcn_ndhwc(const void* x, const void* dz, float* dw, int64_t D, in
 int cvit_adamw_f32(float* p, const float* g, float* m, float* v, int64_t n, float lr, float beta1, float beta2, float eps,
                    float weight_decay, int64_t step, float grad_scale, void* stream);
 
+/* dst[i] += src[i] for i < n (fp32; each sum rounded once): a batch step's per-sample gradient bucket added into the step's
+ * bucket, one sample after the other, so the batch's gradient is the sum over its samples in sample order. The finalize
+ * kernel of the deterministic mode (csrc/det_reduce.cuh) in its add form over a single row. */
+int cvit_accumulate_f32(float* dst, const float* src, int64_t n, void* stream);
+
 /* Masked segmentation statistics, one pass: over voxels with label > -1 (BaseModel._masked_predict,
  * models/base_model.py:91-112) accumulates out8 (fp64, caller zeroes) = {sum p, sum y, sum p*y | sum y*[p>=thr],
  * sum [p>=thr] | sum y*[p>.5], sum (1-y)*[p>.5], sum y*(1-[p>.5])}: the reductions behind DiceLoss
